@@ -2,7 +2,7 @@
 """Headline benchmark: exact top-100 angular kNN queries/s over 50,000 samples x 3000
 features, 4096-query batches (BASELINE.json configs[2]) on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one batch of 4096 queries answered exactly (ids + distances) against the
 HBM-resident sample matrix.  N > 1 (torchrun, one rank per GPU): every rank holds the
@@ -35,6 +35,23 @@ sys.path.insert(0, ROOT)
 N_SAMPLES, DIM, N_QUERIES, K = 50000, 3000, 4096, 100
 N_SHARDED = 1000000
 METRIC = "exact kNN queries/s (50k samples x 3000 feats, k=100)"
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: array bytes in all, below 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, ids, dists):
+    """--dump-outputs: one step's results as out_dir/ids.npy and out_dir/distances.npy, float64 (the int32 ids are exact
+    in it), one row per query.  Above DUMP_BYTES in all, the same seeded sample of queries is written on every run, with
+    its row numbers as out_dir/query_rows.npy."""
+    arrays = {"ids": np.asarray(ids, dtype=np.float64), "distances": np.asarray(dists, dtype=np.float64)}
+    nq = arrays["ids"].shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) if nq else 0
+    if nq * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=DUMP_BYTES // (row_bytes + 8), replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["query_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -85,18 +102,18 @@ class ClockSampler(threading.Thread):
 # ---------------------------------------------------------------------------------------------- CPU baselines
 def cpu_baseline_run(n_samples, dim, k, n_queries, threads, seed=1234):
     """Times the C port of exact_search_nn (oracle/oracle.c) on `n_queries` queries of the
-    same workload, queries split over `threads` host threads.  Returns queries/s."""
+    same workload, queries split over `threads` host threads.  Returns (queries/s, seconds, (ids, distances)).
+    The C oracle is the one build() compiled: nothing is compiled here, the tree may be read-only."""
     from oracle import c_oracle
-    c_oracle.build()
     rng = np.random.default_rng(seed)
     S = rng.standard_normal((n_samples, dim), dtype=np.float32)
     rows = rng.permutation(n_samples)[:n_queries]
     Q = S[rows].astype(np.float64)
     t0 = time.perf_counter()
-    ids, _ = c_oracle.exact_search_batch(S, Q, k, n_threads=threads)
+    ids, dists = c_oracle.exact_search_batch(S, Q, k, n_threads=threads)
     dt = time.perf_counter() - t0
     assert np.array_equal(ids[:, 0], rows.astype(np.int32))      # each query finds itself first
-    return n_queries / dt, dt
+    return n_queries / dt, dt, (ids, dists)
 
 
 def literal_reference_qps(dim, n_samples, rows=300, seed=1):
@@ -158,9 +175,11 @@ def run_reference(args, rank, world):
         cpu_baseline_run(N_SAMPLES, DIM, K, min(per_step, cores), cores)
     t_total, q_total = 0.0, 0
     for _ in range(args.steps):
-        _, dt = cpu_baseline_run(N_SAMPLES, DIM, K, per_step, cores)
+        _, dt, last = cpu_baseline_run(N_SAMPLES, DIM, K, per_step, cores)
         t_total += dt
         q_total += per_step
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
     value = q_total / t_total
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "queries/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t_total / args.steps,
@@ -206,7 +225,11 @@ def main():
     ap.add_argument("--index-pairs", type=float, default=500e6, help="pairs of the index-build section (0 = skip it)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only-headline", action="store_true", help="skip every extra section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the ids and distances of the last timed step (rank 0's "
+                                                          "batch) to DIR as float64 .npy files, to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -275,10 +298,12 @@ def main():
     launches0 = _lib.launch_count()
     barrier()
     wall0 = time.perf_counter()
-    ms_step, (last_ids, _last_d) = pipeline_ms(torch, srch, [queries64] * args.steps, K)
+    ms_step, (last_ids, last_d) = pipeline_ms(torch, srch, [queries64] * args.steps, K)
     barrier()
     wall1 = time.perf_counter()
     assert int(last_ids[0, 0]) == int(rows[0])
+    # copied now: the pipeline hands out views of its pinned buffers, which the sections below overwrite
+    last_outputs = (last_ids.copy(), last_d.copy()) if args.dump_outputs and rank == 0 else None
     launches = _lib.launch_count() - launches0
     clocks = sampler.window(wall0, wall1)
     ms_step = max_over_ranks(ms_step)
@@ -361,7 +386,7 @@ def main():
         if not args.no_cpu_baseline:
             cores = os.cpu_count() or 1
             nq_cpu = min(N_QUERIES, 96 * cores)          # ~10 s of work on all host cores
-            v, dt = cpu_baseline_run(N_SAMPLES, DIM, K, nq_cpu, cores)
+            v, dt, _ = cpu_baseline_run(N_SAMPLES, DIM, K, nq_cpu, cores)
             sv, sdt, _ = strong_cpu_qps(N_SAMPLES, DIM, K, 1024)
             cpu = {"value": v, "unit": "queries/s", "cores": cores, "kind": "port",
                    "sample": "%d of the 4096 queries, C port of exact_search_nn (morna.py:681-712), %d threads, %.1f s"
@@ -388,6 +413,8 @@ def main():
                 "cpu_baseline": cpu, "peaks": peaks["source"]}
         line.update(extras)
         line["index_build"] = index
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, *last_outputs)
         print(json.dumps(line))
     if world > 1:
         td.destroy_process_group()

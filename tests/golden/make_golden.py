@@ -4,7 +4,10 @@ The reference itself cannot run here (Python 2 + mmh3 + annoy, none installed),
 so these are ORACLE outputs on the reference's fixture tests/tiny_intropolis.tsv,
 not reference outputs.  The oracle is pinned separately against the reference's
 own embedded unit-test vectors (reference_unittest_vectors.json).
-Run:  python tests/golden/make_golden.py
+It also writes murmur3_sklearn_vectors.json: random keys and the hashes
+sklearn.utils.murmurhash3_32 gives them (the reference hashes with mmh3, which
+agrees with sklearn), so the hash check runs without scikit-learn installed.
+Run:  python tests/golden/make_golden.py   (needs scikit-learn)
 """
 import hashlib
 import json
@@ -54,6 +57,21 @@ def main():
     with open(os.path.join(HERE, "tiny_expected.json"), "w") as fh:
         json.dump(out, fh, indent=1)
     print("wrote tiny_expected.json; n_kept", out["n_kept"], "sha", out["matrix_f32_sha256"])
+    write_murmur3_vectors()
+
+
+def write_murmur3_vectors():
+    from sklearn.utils import murmurhash3_32
+    rng = np.random.default_rng(5)
+    keys = []
+    for _ in range(300):
+        n = int(rng.integers(0, 40))
+        keys.append(bytes(rng.integers(32, 127, size=n, dtype=np.uint8)).decode("ascii"))
+    out = {"source": "sklearn.utils.murmurhash3_32(key, seed=0, positive=False) on the ASCII bytes of key",
+           "cases": [[key, int(murmurhash3_32(key.encode("ascii"), seed=0, positive=False))] for key in keys]}
+    with open(os.path.join(HERE, "murmur3_sklearn_vectors.json"), "w") as fh:
+        json.dump(out, fh, indent=0)
+    print("wrote murmur3_sklearn_vectors.json;", len(keys), "keys")
 
 
 if __name__ == "__main__":
