@@ -1586,7 +1586,8 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
     for (int64_t b0 = w.n0; b0 < n;) {
         int64_t b1 = b0 == w.n0 ? (int64_t)(g_first_block > 0 ? g_first_block : g_block_rows) : b0 + step;
         if (b0 != w.n0 && g_block_growth > 1) step *= g_block_growth;
-        if (b1 > n || b1 <= b0) b1 = n;
+        if (b1 <= b0) b1 = b0 + step;      // key 11 (or key 9) at or below the pilot rows: the first block is `step` rows, not the rest
+        if (b1 > n) b1 = n;
         rc = launch_gemm((int32_t)b0, (int32_t)b1, 1);
         if (rc != MORNA_OK) return rc;
         b0 = b1;
@@ -1634,7 +1635,8 @@ static int list_swaps(int64_t n, const BatchWs &w) {
     for (int64_t b0 = w.n0; b0 < n;) {
         int64_t b1 = b0 == w.n0 ? (int64_t)(g_first_block > 0 ? g_first_block : g_block_rows) : b0 + step;
         if (b0 != w.n0 && g_block_growth > 1) step *= g_block_growth;
-        if (b1 > n || b1 <= b0) b1 = n;
+        if (b1 <= b0) b1 = b0 + step;
+        if (b1 > n) b1 = n;
         b0 = b1;
         if (b0 < n) ++swaps;
     }

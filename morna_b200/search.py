@@ -803,13 +803,26 @@ class BatchPipeline(object):
                 sl.host_d.copy_(d, non_blocking=True)
             sl.done.record(sl.stream)
 
+    def _check_resident_ids(self, q):
+        """Internal ids given as queries must name rows of this shard: outside [row_lo, row_hi) the row index would be
+        negative (torch wraps it: a silently wrong query row) or past the block."""
+        s = self.search
+        if q.numel() == 0:
+            return
+        lo, hi = (int(v) for v in (torch.aminmax(q) if q.is_cuda else (q.min(), q.max())))    # (one reduction on the device)
+        if lo < s.row_lo or hi >= s.row_hi:
+            raise ValueError("internal ids %d..%d are not all resident on this shard (rows %d..%d)"
+                             % (lo, hi, s.row_lo, s.row_hi - 1))
+
     def submit(self, queries):
         s, k = self.search, self.k
         sl = self.slots[self.head % self.depth]
         assert self.head - self.tail < self.depth, "collect() before submitting more than `depth` batches"
-        self.head += 1
         q = torch.from_numpy(np.ascontiguousarray(queries)) if isinstance(queries, np.ndarray) else queries
         by_id = q.dim() == 1 and q.dtype in (torch.int32, torch.int64)      # stored rows as queries (search -q): only ids cross PCIe
+        if by_id:
+            self._check_resident_ids(q)      # before the slot is taken: the pipeline stays usable after the error
+        self.head += 1
         if by_id:
             self._size(sl, q.shape[0], torch.float64, staging=False)
             with torch.cuda.stream(sl.stream):
