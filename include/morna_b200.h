@@ -137,6 +137,39 @@ int morna_index_accumulate(const int64_t *row_off, const uint8_t *pass, const in
                            int32_t dim, double *acc, int64_t acc_ld,
                            void *workspace, size_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------ query vectors from a junction file */
+
+/* Device hash table of an index's junction keys (the keys of basename.freq.mor), so that the rows of a query file are
+ * joined against them on the device instead of one `key in sample_frequencies` test per row (morna.py:1456-1473).
+ * Open addressing over a power of two of int32 slots (at least twice the key count), linear probing; a slot holds a
+ * key index or -1.  Slot placement may differ between builds; lookups do not.
+ *   keys/key_off [dev] the n_keys keys, packed as for morna_hash_junctions; keys must be distinct
+ *   raw          [dev] int32[n_keys] their morna_hash_junctions raw hashes (any dim)
+ *   table        [dev] out, morna_junction_table_bytes(n_keys) bytes */
+size_t morna_junction_table_bytes(int64_t n_keys);
+int morna_junction_table_build(const uint8_t *keys, const int32_t *key_off, const int32_t *raw, int64_t n_keys,
+                               void *table, size_t table_bytes, void *stream);
+
+/* Join of n_rows query rows against the table.  Replaces the per-junction `key in sample_frequencies` test and the
+ * idf of finalize_query (morna.py:609-629) for every row of a query file.
+ *   table_keys/table_key_off/table_raw [dev] what the table was built from;  key_idf [dev] double[n_keys], the idf
+ *                of each key (morna_idf_host: the device computes no log)
+ *   keys/key_off/raw [dev] the query rows' keys and raw hashes;  row_off [dev] int64[n_rows+1], sample [dev] int32[nnz]
+ *   match  [dev] int32[n_rows] out: index of the key equal to row j's key (same length and bytes), or -1
+ *   pass   [dev] uint8[n_rows] out: match >= 0
+ *   idf    [dev] double[n_rows] out: key_idf[match], 0 without a match
+ *   flags  [dev] uint8[n_rows] out, 0 for unmatched rows: bit 0 = another row matched the same key, bit 1 = the row's
+ *               sample ids are not strictly ascending (a sample may repeat).  morna_index_accumulate adds such
+ *               rows' pairs one by one, where the reference sums the coverages of a repeated (key, sample) first.
+ *   n_flagged [dev] int32[1] out: number of rows with flags != 0 (the only value a caller need read in the common case)
+ * Workspace: morna_junction_lookup_workspace_bytes(n_keys). */
+size_t morna_junction_lookup_workspace_bytes(int64_t n_keys);
+int morna_junction_lookup(const void *table, size_t table_bytes, const uint8_t *table_keys, const int32_t *table_key_off,
+                          const int32_t *table_raw, const double *key_idf, int64_t n_keys, const uint8_t *keys,
+                          const int32_t *key_off, const int32_t *raw, const int64_t *row_off, const int32_t *sample,
+                          int64_t n_rows, int32_t *match, uint8_t *pass, double *idf, uint8_t *flags, int32_t *n_flagged,
+                          void *workspace, size_t workspace_bytes, void *stream);
+
 /* Round the double accumulator to the float32 sample matrix, row = internal id.
  * Replaces Annoy add_item's float cast at morna.py:405-407 / 422-424.
  *   vectors [dev] float32[n_ids * ld], pad columns zero-filled by this call */

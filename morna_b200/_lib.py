@@ -49,6 +49,11 @@ _SIGNATURES = {
     "morna_index_accumulate_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32]),
     "morna_index_accumulate": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_i64,
                                               _c_vp, _c_i32, _c_i32, _c_i32, _c_i32, _c_vp, _c_i64, _c_vp, _c_sz, _c_vp]),
+    "morna_junction_table_bytes": (_c_sz, [_c_i64]),
+    "morna_junction_table_build": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_sz, _c_vp]),
+    "morna_junction_lookup_workspace_bytes": (_c_sz, [_c_i64]),
+    "morna_junction_lookup": (ctypes.c_int, [_c_vp, _c_sz, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp,
+                                             _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_round_store": (ctypes.c_int, [_c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_vp]),
     "morna_row_norms": (ctypes.c_int, [_c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_vp]),
     "morna_angular_distances": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_i64, _c_i64,

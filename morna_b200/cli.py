@@ -40,13 +40,21 @@ def results_output(results, out=None):
         out.write("\n")
 
 
+class _StoreGiven(argparse._StoreAction):
+    """A store action that also records that the flag was given (its default cannot tell)."""
+
+    def __call__(self, parser, namespace, values, option_string=None):
+        super().__call__(parser, namespace, values, option_string)
+        namespace.given = getattr(namespace, "given", frozenset()) | {self.dest}
+
+
 def add_search_parameters(sub):
     sub.add_argument("-x", "--basename", metavar="<idx>", type=str, required=True,
                      help="path to junction index basename for search")
     sub.add_argument("-v", "--verbose", action="store_const", const=True, default=False, help="be talkative")
     sub.add_argument("--search-k", metavar="<int>", type=int, required=False, default=100,
                      help="accepted for compatibility; the exact search ignores it")
-    sub.add_argument("-f", "--format", metavar="<choice>", type=str, required=False, default="sam",
+    sub.add_argument("-f", "--format", metavar="<choice>", type=str, required=False, default="sam", action=_StoreGiven,
                      help="one of {sam, bed, raw}")
     sub.add_argument("-d", "--distances", action="store_const", const=True, default=False,
                      help="include distances to nearest neighbors")
@@ -93,6 +101,12 @@ def build_parser():
     index_parser.add_argument("--no-junction-shards", action="store_const", const=True, default=False,
                               help="do not write the <basename>.shXX.junc.mor shards (only `junctions` reads them)")
     add_search_parameters(search_parser)
+    search_parser.add_argument("--query-intropolis", metavar="<file>", type=str, required=False, default=None,
+                               help="(gzipped) intropolis-format file: search for every sample it lists, one line per "
+                                    "result prefixed by the sample id and a tab")
+    search_parser.add_argument("--all-samples", action="store_const", const=True, default=False,
+                               help="search for every indexed sample (as -q for each sample id), one line per result "
+                                    "prefixed by the sample id and a tab")
     junctions_parser = subs.add_parser("junctions", help="extracts the junctions of a query's nearest neighbors")
     add_search_parameters(junctions_parser)                      # morna.py:1023-1054
     junctions_parser.add_argument("-i", "--index", metavar="<idx>", type=str, required=True,
@@ -128,6 +142,8 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     if args.convergence_backoff:
         stderr.write("convergence back-off is not supported (see README of the reference: non-functional)\n")
         return 2
+    if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
+        return batch_search(args, stdout, stderr)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
@@ -167,6 +183,28 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
         from .junctions import go_junctions
         go_junctions(args, searcher, results, stdout, stderr)
         opened.close()
+    return 0
+
+
+def batch_search(args, stdout, stderr):
+    """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches."""
+    from . import batch_query
+    from .search import MornaSearch
+    named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
+                                   ("--all-samples", args.all_samples), ("-q", args.query_id is not None),
+                                   ("-rl", args.rawlist), ("-f", "format" in getattr(args, "given", ()))) if on]
+    if len(named) > 1:
+        stderr.write("%s cannot be combined with %s\n" % (named[0], ", ".join(named[1:])))
+        return 2
+    searcher = MornaSearch(basename=args.basename)
+    inverse = batch_query.inverse_map(searcher)
+    if args.all_samples:                       # the stored rows as queries: exact, as -q is
+        results = batch_query.search_all_samples(searcher, args.results, inverse)
+    else:
+        results = batch_query.search_query_file(searcher, args.query_intropolis, args.results, exact=args.exact)
+    meta = args.basename if args.metadata else None
+    for sample_ids, ids, dists in results:
+        batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse)
     return 0
 
 

@@ -4,6 +4,7 @@ store, keeps the float32 sample matrix resident in HBM, and answers exact angula
 top-k queries under the reference's order (distance ascending, ties id-descending).
 """
 import ctypes
+import gc
 import math
 import os
 from collections import defaultdict
@@ -754,15 +755,24 @@ class BatchPipeline(object):
             if self.use_graphs and seen == key and sl.ws is not None:
                 # capture_begin / capture_end directly: the torch.cuda.graph context would synchronise the device, run the
                 # garbage collector and empty the allocator cache first -- a stall of several batch times.  Nothing is
-                # allocated between the two calls (every buffer of the step already exists).
+                # allocated between the two calls (every buffer of the step already exists).  The cyclic garbage collector
+                # is off while capturing: a MornaSearch and its pipelines form a reference cycle, so a dropped search can
+                # be collected at any allocation, and destroying its graphs, events and pinned buffers makes CUDA calls
+                # (event queries among them) that invalidate a capture running on this thread.
                 graph = torch.cuda.CUDAGraph()
                 launches0 = _lib.launch_count()
-                graph.capture_begin(capture_error_mode="thread_local")
+                gc_on = gc.isenabled()
+                gc.disable()
                 try:
-                    self._score(sl, None)
-                    self._rerank_kernels(sl, resume=False)
+                    graph.capture_begin(capture_error_mode="thread_local")
+                    try:
+                        self._score(sl, None)
+                        self._rerank_kernels(sl, resume=False)
+                    finally:
+                        graph.capture_end()
                 finally:
-                    graph.capture_end()
+                    if gc_on:
+                        gc.enable()
                 sl.graph, sl.graph_key = graph, key
                 sl.graph_launches = _lib.launch_count() - launches0      # counted once while capturing: stands for the replay below
                 graph.replay()
