@@ -358,6 +358,45 @@ int morna_knn_batched_approx(const void *hs, int64_t ld_h, const float *rho_max,
                              int32_t *out_ids, double *out_dist, uint8_t *overflow, int32_t *stats,
                              void *workspace, size_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------ range search
+ * Every row within an angular distance R of a query: the rows i with d(q, i) <= R, d the exact FP64 distance of
+ * morna_knn_exact (bit for bit), ids global (id_base + row), each list ordered under the reference order (distance
+ * ascending, equal distances id descending).  R is a finite double >= 0.  Results are CSR: the caller reads the counts,
+ * builds offsets[nq + 1] (int64, offsets[0] = 0) and gives them to the second call, which writes query j's list to
+ * out_ids / out_dist [offsets[j], offsets[j + 1]).  No call synchronises.
+ *
+ * Tensor-core route (nq <= 4096, n <= 2^24): the queries are prepared as for morna_knn_batched, one filter GEMM over
+ * all n rows keeps every row whose fp16 score reaches thr[q] = rd_float((1 - R^2/2) - eps[q] - 2^-30) (a superset of
+ * the rows in range, see DESIGN.md section 4), and each survivor's exact distance is checked against R.
+ *   counts   [dev] int32[nq]  out: rows in range per query; 0 for an overflowed query
+ *   overflow [dev] uint8[nq]  out: 1 where more than 4096 rows passed the filter or a query value is >= 2^127 in
+ *                             magnitude; those queries must be answered by the FP64 route
+ *   stats    [dev] int64[4]   out: {overflowed queries, first-pass survivors (all queries, uncapped),
+ *                              rows in range of the other queries, max rows in range of one query}
+ * morna_range_batched_emit writes the sorted lists of the queries that did not overflow (at most 4096 each; a query's
+ * list is cut to its offsets' length) from the state the first call left in the same workspace. */
+size_t morna_range_batched_workspace_bytes(int64_t n, int64_t nq, int32_t dim);
+int morna_range_batched(const float *vectors, const double *pp, const void *hs, int64_t ld_h, const float *rho_max,
+                        int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
+                        int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
+                        void *workspace, size_t workspace_bytes, void *stream);
+int morna_range_batched_emit(int64_t n, int64_t nq, int32_t dim, const int64_t *offsets, const uint8_t *overflow,
+                             int32_t *out_ids, double *out_dist, const void *workspace, size_t workspace_bytes,
+                             void *stream);
+
+/* FP64 route (any n, nq, query values): the distance scan of morna_knn_exact in query tiles of bounded scratch.  The
+ * count call writes counts [dev] int32[nq]; the fill call scans again, compacts each query's matches in descending
+ * row order and sorts every list by distance with a stable segmented radix sort (so equal distances stay id
+ * descending).  total = offsets[nq] (< 2^31 per call); workspace_bytes(n, nq, 0) suffices for the count call. */
+size_t morna_range_exact_workspace_bytes(int64_t n, int64_t nq, int64_t total);
+int morna_range_exact_count(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                            const double *queries, int64_t nq, int64_t q_ld, double max_distance, int32_t *counts,
+                            void *workspace, size_t workspace_bytes, void *stream);
+int morna_range_exact_fill(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                           const double *queries, int64_t nq, int64_t q_ld, double max_distance, const int64_t *offsets,
+                           int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
+                           void *stream);
+
 /* Test hook: raw fp16 tensor-core scores [nq x n] (n <= 8192) and the per-query bound eps. */
 int morna_debug_tensor_scores(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
                               const double *queries, int64_t nq, int64_t q_ld, float *scores,

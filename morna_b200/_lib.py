@@ -89,6 +89,15 @@ _SIGNATURES = {
     "morna_knn_batched_finalize": (ctypes.c_int, [_c_i64, _c_i64, _c_i32, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_knn_batched_rerank": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_i32,
                                                 _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_i32, _c_vp]),
+    "morna_range_batched_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32]),
+    "morna_range_batched": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64,
+                                           _c_i64, ctypes.c_double, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_batched_emit": (ctypes.c_int, [_c_i64, _c_i64, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_exact_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i64]),
+    "morna_range_exact_count": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_i64, _c_i64, ctypes.c_double,
+                                               _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_exact_fill": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, ctypes.c_double,
+                                              _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_tensor_scores": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_vp,
                                                  _c_i64, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_set_tuning": (ctypes.c_int, [_c_i32, _c_i32]),

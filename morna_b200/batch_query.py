@@ -245,16 +245,62 @@ def search_all_samples(search, k, inverse):
         yield inverse[b:b + ids.shape[0]], ids.copy(), d.copy()
 
 
-def write_results(out, sample_ids, ids, dists, include_distances, meta_basename, inverse):
+def search_query_file_range(search, path, max_distance, cap=None, result_cap=None):
+    """Range variant of search_query_file (always exact): every indexed sample within `max_distance` of each query.
+    Yields (sample ids [b], offsets int64 [b+1], ids, dists) numpy CSR batches in query order; query j's list is
+    ids/dists[offsets[j]:offsets[j+1]].  The lists of a 4096-query batch are counted first, and a batch whose lists
+    would take more than `result_cap` bytes (SLICE_BYTES_CAP by default) comes in smaller groups of queries."""
+    qf = QueryFile(search, path)
+    result_cap = SLICE_BYTES_CAP if result_cap is None else result_cap
+    for lo, hi in qf.slices(cap):
+        vecs = qf.query_vectors(lo, hi)
+        for b in range(0, hi - lo, BATCH_QUERIES):
+            for g0, g1, off, ids, d in search.range_search_groups(vecs[b:b + BATCH_QUERIES], max_distance, result_cap):
+                yield qf.sample_ids[lo + b + g0:lo + b + g1], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
+
+
+def search_all_samples_range(search, max_distance, inverse, result_cap=None):
+    """Range variant of search_all_samples: the stored rows as queries, built on the device from their ids.  Yields
+    (sample ids, offsets, ids, dists) numpy CSR batches as search_query_file_range does."""
+    n = search.index_size
+    result_cap = SLICE_BYTES_CAP if result_cap is None else result_cap
+    for b in range(0, n, BATCH_QUERIES):
+        rows = torch.arange(b, min(n, b + BATCH_QUERIES), device=search.device) - search.row_lo
+        q = search.vectors[rows, :search.dim].to(torch.float64).contiguous()
+        for g0, g1, off, ids, d in search.range_search_groups(q, max_distance, result_cap):
+            yield inverse[b + g0:b + g1], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
+
+
+def cut_lists(offsets, ids, dists, limit):
+    """CSR lists cut to their first `limit` entries (numpy; None: unchanged)."""
+    if limit is None:
+        return offsets, ids, dists
+    lens = np.diff(offsets)
+    keep_len = np.minimum(lens, max(int(limit), 0))
+    rank = np.arange(len(ids)) - np.repeat(offsets[:-1], lens)
+    keep = rank < np.repeat(keep_len, lens)
+    out = np.zeros_like(offsets)
+    np.cumsum(keep_len, out=out[1:])
+    return out, ids[keep], dists[keep]
+
+
+def write_results(out, sample_ids, ids, dists, include_distances, meta_basename, inverse, offsets=None, limit=None):
     """One batch of results.  Each line: the query's sample id, a tab, then exactly the line cli.results_output prints for
-    that query (rank, internal id, distance with -d, metadata tuple with -m)."""
+    that query (rank, internal id, distance with -d, metadata tuple with -m).  With `offsets`, the batch is CSR (query j's
+    list is ids/dists[offsets[j]:offsets[j+1]]) and each list is cut to its first `limit` entries."""
     from .cli import py2_str
+    if offsets is None:
+        kept = ids[ids >= 0]
+        queries = zip(sample_ids.tolist(), ids.tolist(), dists.tolist())
+    else:
+        offsets, ids, dists = cut_lists(offsets, ids, dists, limit)
+        kept, o, il, dl = ids, offsets.tolist(), ids.tolist(), dists.tolist()
+        queries = ((sid, il[o[j]:o[j + 1]], dl[o[j]:o[j + 1]]) for j, sid in enumerate(sample_ids.tolist()))
     meta = None
     if meta_basename is not None:
-        keep = ids >= 0
-        meta = iter(files.read_meta(meta_basename, inverse[ids[keep]].tolist()))
+        meta = iter(files.read_meta(meta_basename, inverse[kept].tolist()))
     lines = []
-    for sid, row_ids, row_d in zip(sample_ids.tolist(), ids.tolist(), dists.tolist()):
+    for sid, row_ids, row_d in queries:
         prefix = str(sid) + "\t"
         rank = 0
         for iid, dist in zip(row_ids, row_d):

@@ -6,7 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libmorna_b200.so")
-SOURCES = ["api.cu", "index_build.cu", "search_exact.cu", "search_single.cu", "search_batched.cu", "search_sparse.cu", "query_build.cu",
+SOURCES = ["api.cu", "index_build.cu", "search_exact.cu", "search_single.cu", "search_batched.cu", "search_sparse.cu", "search_range.cu",
+           "query_build.cu",
            "tokenize.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"] + os.environ.get("MORNA_NVCC_EXTRA", "").split()

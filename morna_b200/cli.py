@@ -13,6 +13,7 @@ search with the stored row as the query (the reference ignores -e after -q).
 The `junctions` subcommand and the convergence back-off loop are outside the hot path and exit with a message.
 """
 import argparse
+import math
 import sys
 
 _help_intro = "morna (B200-native hot path): index and exactly search junction feature vectors"
@@ -68,8 +69,9 @@ def add_search_parameters(sub):
                      help="search for nearest neighbors of the indexed sample with this sample id")
     sub.add_argument("-e", "--exact", action="store_const", const=True, default=False,
                      help="exact nearest neighbor search (always on in this implementation)")
-    sub.add_argument("-r", "--results", metavar="<int>", type=int, required=False, default=20,
-                     help="the number of nearest neighbor results to return")
+    sub.add_argument("-r", "--results", metavar="<int>", type=int, required=False, default=20, action=_StoreGiven,
+                     help="the number of nearest neighbor results to return (with --max-distance: given, at most this "
+                          "many per query)")
     sub.add_argument("-rl", "--rawlist", action="store_const", const=True, default=False,
                      help="regurgitate junction list for input sample instead of performing search")
 
@@ -107,6 +109,9 @@ def build_parser():
     search_parser.add_argument("--all-samples", action="store_const", const=True, default=False,
                                help="search for every indexed sample (as -q for each sample id), one line per result "
                                     "prefixed by the sample id and a tab")
+    search_parser.add_argument("--max-distance", metavar="<float>", type=float, required=False, default=None,
+                               help="return every sample within this angular distance of the query (exact; -r N, if "
+                                    "given, keeps the first N per query)")
     junctions_parser = subs.add_parser("junctions", help="extracts the junctions of a query's nearest neighbors")
     add_search_parameters(junctions_parser)                      # morna.py:1023-1054
     junctions_parser.add_argument("-i", "--index", metavar="<idx>", type=str, required=True,
@@ -142,16 +147,30 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     if args.convergence_backoff:
         stderr.write("convergence back-off is not supported (see README of the reference: non-functional)\n")
         return 2
+    max_distance = getattr(args, "max_distance", None)
+    if max_distance is not None:
+        if not (math.isfinite(max_distance) and max_distance >= 0.0):
+            stderr.write("--max-distance must be a finite number >= 0\n")
+            return 2
+        if args.rawlist:
+            stderr.write("-rl cannot be combined with --max-distance\n")
+            return 2
+    # a range search lists everything within the radius; an explicit -r caps each list
+    limit = args.results if max_distance is not None and "results" in getattr(args, "given", ()) else None
     if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
-        return batch_search(args, stdout, stderr)
+        return batch_search(args, stdout, stderr, max_distance, limit)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
         stdin = opened = open(args.pass1_sam)
     searcher = MornaSearch(basename=args.basename)
     if args.query_id is not None:                               # morna.py:1358-1365
-        results = searcher.search_member_n(args.query_id, args.results, args.search_k,
-                                           include_distances=args.distances, meta_db=args.metadata, out=stdout)
+        if max_distance is not None:
+            results = searcher.search_member_n(args.query_id, limit, include_distances=args.distances,
+                                               meta_db=args.metadata, out=stdout, max_distance=max_distance)
+        else:
+            results = searcher.search_member_n(args.query_id, args.results, args.search_k,
+                                               include_distances=args.distances, meta_db=args.metadata, out=stdout)
         results_output(results, stdout)
         return 0
     if args.format == "sam":                                    # :1367-1373
@@ -174,7 +193,10 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     searcher.finalize_query()
     if args.verbose:
         stderr.write("\n")
-    if args.exact:                                              # :1477-1483
+    if max_distance is not None:                                # always exact: -e changes nothing
+        results = searcher.range_search_nn(max_distance, include_distances=args.distances, meta_db=args.metadata,
+                                           num_neighbors=limit)
+    elif args.exact:                                            # :1477-1483
         results = searcher.exact_search_nn(args.results, include_distances=args.distances, meta_db=args.metadata)
     else:
         results = searcher.search_nn(args.results, args.search_k, include_distances=args.distances, meta_db=args.metadata)
@@ -186,8 +208,9 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     return 0
 
 
-def batch_search(args, stdout, stderr):
-    """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches."""
+def batch_search(args, stdout, stderr, max_distance=None, limit=None):
+    """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches.  With
+    `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given."""
     from . import batch_query
     from .search import MornaSearch
     named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
@@ -198,11 +221,19 @@ def batch_search(args, stdout, stderr):
         return 2
     searcher = MornaSearch(basename=args.basename)
     inverse = batch_query.inverse_map(searcher)
+    meta = args.basename if args.metadata else None
+    if max_distance is not None:
+        if args.all_samples:
+            results = batch_query.search_all_samples_range(searcher, max_distance, inverse)
+        else:
+            results = batch_query.search_query_file_range(searcher, args.query_intropolis, max_distance)
+        for sample_ids, offsets, ids, dists in results:
+            batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse, offsets=offsets, limit=limit)
+        return 0
     if args.all_samples:                       # the stored rows as queries: exact, as -q is
         results = batch_query.search_all_samples(searcher, args.results, inverse)
     else:
         results = batch_query.search_query_file(searcher, args.query_intropolis, args.results, exact=args.exact)
-    meta = args.basename if args.metadata else None
     for sample_ids, ids, dists in results:
         batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse)
     return 0

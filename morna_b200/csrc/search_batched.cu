@@ -1953,6 +1953,267 @@ extern "C" int morna_debug_tensor_scores(const void *hs, int64_t ld_h, const flo
     return launch_knn_gemm(tmap_q, tmap_s, gp, s);
 }
 
+// ------------------------------------------------------------------ range search, tensor-core route
+// With the radius known up front there is no pilot, no k-th selection and no refinement between row blocks: the query
+// prep, one filter GEMM over all rows with thresholds fixed before it starts, and an FP64 check of every survivor.
+//
+// Threshold.  Let c be the exact cosine of (q, i) and d_fp the FP64 distance the scan returns.  d_fp <= R implies
+// c >= 1 - R^2/2 - delta_fp, where delta_fp covers the canonical sums' rounding (at most ~dim * 2^-53 relative to
+// |p||q|, 3.3e-12 at dim = 30,000) and that of the division, sqrt and the final subtraction (a few ulps of 2).  The
+// fp16 score s has |s - c| <= eps[q] (prep_queries_kernel).  So every row in range scores
+// s >= (1 - R^2/2) - eps[q] - delta_fp >= (1 - R^2/2) - eps[q] - 2^-30, and thr[q] is that double rounded down to a
+// float: the filter drops no row in range.  A zero query or zero row scores 0 and sits at sqrt(2); it passes whenever
+// R >= sqrt(2), where the bound is <= -eps - 2^-30 < 0.
+namespace morna {
+
+constexpr int kRangeMaxQueries = 4096;
+constexpr int kRangeWarps = 8;
+constexpr int kRangeEmitThreads = 512;
+
+struct RangeWs {
+    size_t hq, qq, eps, thr, cand_score, cand_id, cand_cnt, match_id, match_dist, match_cnt, prep_stats, total;
+    int64_t nq_pad;
+};
+static RangeWs range_ws_layout(int64_t nq, int64_t ld_h) {
+    RangeWs w{};
+    w.nq_pad = (nq + 2 * gemm::BM - 1) / (2 * gemm::BM) * (2 * gemm::BM);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t at = off; off += align_up(bytes, 256); return at; };
+    w.hq = take((size_t)w.nq_pad * ld_h * sizeof(__half));
+    w.qq = take((size_t)nq * sizeof(double));
+    w.eps = take((size_t)nq * sizeof(float));
+    w.thr = take((size_t)nq * sizeof(float));
+    w.cand_score = take((size_t)nq * kCandCap * sizeof(float));
+    w.cand_id = take((size_t)nq * kCandCap * sizeof(int32_t));
+    w.cand_cnt = take((size_t)nq * sizeof(int32_t));
+    w.match_id = take((size_t)nq * kCandCap * sizeof(int32_t));
+    w.match_dist = take((size_t)nq * kCandCap * sizeof(double));
+    w.match_cnt = take((size_t)nq * sizeof(int32_t));
+    w.prep_stats = take(4 * sizeof(int32_t));
+    w.total = off + 1024;
+    return w;
+}
+
+__global__ void range_thr_kernel(const float *__restrict__ eps, const uint8_t *__restrict__ overflow, int32_t nq, double R,
+                                 float *__restrict__ thr) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const double t = (1.0 - 0.5 * R * R) - (double)eps[q] - 0x1p-30;
+    thr[q] = overflow[q] ? INFINITY : __double2float_rd(t);      // a flagged query collects nothing: the FP64 route answers it
+}
+
+struct RangeCheckParams {
+    const float *vectors; const double *pp; int64_t ld; int32_t dim, id_base, nq;
+    const double *queries; int64_t q_ld; const double *qq;
+    const int32_t *cand_id; const int32_t *cand_cnt; const uint8_t *overflow;
+    double R;
+    int32_t *match_id; double *match_dist; int32_t *match_cnt;
+};
+
+// A work item is (32-candidate window, query) of a first-pass list, one warp each: the window's rows go through
+// rerank_rows (canonical sums, query read from global memory, so any dim) 4 at a time, and the rows within R are
+// appended to the query's match list.  Windows past a list's end, and queries that overflowed, are skipped.
+__global__ void __launch_bounds__(kRangeWarps * 32)
+range_check_kernel(const RangeCheckParams p) {
+    constexpr int kRows = 4, kWindows = kCandCap / 32;
+    const int lane = threadIdx.x & 31;
+    const long long total = (long long)p.nq * kWindows;
+    const long long warps = (long long)gridDim.x * kRangeWarps;
+    const bool vec_ok = ((p.q_ld & 1) == 0) && ((reinterpret_cast<uintptr_t>(p.queries) & 15) == 0);
+    const int chunks = (int)(p.ld >> 2);
+    for (long long t = (long long)blockIdx.x * kRangeWarps + (threadIdx.x >> 5); t < total; t += warps) {
+        // window-major: the live items (the first windows of every query) are spread evenly over the warps
+        const int win = (int)(t / p.nq), q = (int)(t - (long long)win * p.nq), i0 = win * 32;
+        const int count = p.cand_cnt[q];
+        if (count > kCandCap || p.overflow[q] || i0 >= count) continue;
+        const int m = min(32, count - i0);
+        const int32_t *ids = p.cand_id + (int64_t)q * kCandCap + i0;
+        const double *qsrc = p.queries + (int64_t)q * p.q_ld;
+        const double qqv = p.qq[q];
+        for (int g = 0; g < m; g += kRows) {
+            const int cnt = min(kRows, m - g);
+            const float4 *src[kRows];
+            int my_id = 0;
+#pragma unroll
+            for (int u = 0; u < kRows; ++u) {
+                const int id = ids[min(g + u, m - 1)];
+                src[u] = reinterpret_cast<const float4 *>(p.vectors + (int64_t)(id - p.id_base) * p.ld);
+                if (lane == u) my_id = id;
+            }
+            double acc[kRows];
+            rerank_rows<kRows, 4, false>(src, cnt, qsrc, p.dim, chunks, vec_ok, lane, acc);
+            double mine = 0.0;
+#pragma unroll
+            for (int u = 0; u < kRows; ++u) {
+                if (u < cnt) {                                           // cnt is warp-uniform
+                    const double s = warp_sum(acc[u]);
+                    if (lane == u) mine = s;
+                }
+            }
+            double d = 0.0;
+            if (lane < cnt) d = angular_from_sums(p.pp[my_id - p.id_base], qqv, mine);
+            const bool keep = lane < cnt && d <= p.R;
+            const unsigned mask = __ballot_sync(kFull, keep);
+            if (mask) {
+                int at = 0;
+                if (lane == 0) at = atomicAdd(p.match_cnt + q, __popc(mask));
+                at = __shfl_sync(kFull, at, 0) + __popc(mask & ((1u << lane) - 1u));
+                if (keep) {                                              // at < kCandCap: matches are a subset of the list
+                    p.match_id[(int64_t)q * kCandCap + at] = my_id;
+                    p.match_dist[(int64_t)q * kCandCap + at] = d;
+                }
+            }
+        }
+    }
+}
+
+__global__ void range_finish_kernel(const int32_t *__restrict__ cand_cnt, const int32_t *__restrict__ match_cnt, int32_t nq,
+                                    uint8_t *__restrict__ overflow, int32_t *__restrict__ counts,
+                                    unsigned long long *__restrict__ stats) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const int c = cand_cnt[q];
+    const bool over = overflow[q] || c > kCandCap;
+    const int m = over ? 0 : match_cnt[q];
+    overflow[q] = over ? 1 : 0;
+    counts[q] = m;
+    if (over) atomicAdd(stats + 0, 1ull);
+    if (c) atomicAdd(stats + 1, (unsigned long long)c);
+    if (m) { atomicAdd(stats + 2, (unsigned long long)m); atomicMax(stats + 3, (unsigned long long)m); }
+}
+
+// One CTA per query: its matches sorted under the reference order (bitonic network in shared memory), written to
+// out[offsets[q], offsets[q+1]).
+__global__ void __launch_bounds__(kRangeEmitThreads)
+range_emit_kernel(const int32_t *__restrict__ match_id, const double *__restrict__ match_dist, const int32_t *__restrict__ match_cnt,
+                  const uint8_t *__restrict__ overflow, const int64_t *__restrict__ offsets, int32_t *__restrict__ out_ids,
+                  double *__restrict__ out_dist) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    double *sd = reinterpret_cast<double *>(smem_raw);                 // [kCandCap]
+    int *si = reinterpret_cast<int *>(sd + kCandCap);                  // [kCandCap]
+    const int tid = threadIdx.x, q = blockIdx.x;
+    const int64_t o = offsets[q];
+    const int64_t room = offsets[q + 1] - o;
+    if (overflow[q] || room <= 0) return;
+    const int count = min(match_cnt[q], kCandCap);
+    int P = 32;
+    while (P < count) P <<= 1;
+    for (int i = tid; i < P; i += kRangeEmitThreads) {
+        const bool have = i < count;
+        sd[i] = have ? match_dist[(int64_t)q * kCandCap + i] : INFINITY;
+        si[i] = have ? match_id[(int64_t)q * kCandCap + i] : -1;
+    }
+    for (int size = 2; size <= P; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            __syncthreads();
+            for (int i = tid; i < (P >> 1); i += kRangeEmitThreads) {
+                const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+                const bool asc = (lo & size) == 0;
+                const double dl = sd[lo], dh = sd[hi];
+                const int il = si[lo], ih = si[hi];
+                if (asc ? before(dh, ih, dl, il) : before(dl, il, dh, ih)) { sd[lo] = dh; sd[hi] = dl; si[lo] = ih; si[hi] = il; }
+            }
+        }
+    }
+    __syncthreads();
+    const int n_out = (int)min((int64_t)count, room);
+    for (int i = tid; i < n_out; i += kRangeEmitThreads) { out_ids[o + i] = si[i]; out_dist[o + i] = sd[i]; }
+}
+
+}  // namespace morna
+
+extern "C" size_t morna_range_batched_workspace_bytes(int64_t n, int64_t nq, int32_t dim) {
+    if (n <= 0 || nq <= 0 || dim <= 0) return 1024;
+    return range_ws_layout(nq, morna_tensor_operand_ld(dim)).total;
+}
+
+extern "C" int morna_range_batched(const float *vectors, const double *pp, const void *hs, int64_t ld_h, const float *rho_max,
+                                   int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
+                                   int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
+                                   void *workspace, size_t workspace_bytes, void *stream) {
+    if (!vectors || !pp || !hs || !rho_max || !queries || !counts || !overflow || !stats || n <= 0 || n > kBatchedMaxRows ||
+        nq <= 0 || nq > kRangeMaxQueries || dim <= 0 || ld < dim || (ld & 3) || q_ld < dim ||
+        ld_h != morna_tensor_operand_ld(dim) || !(max_distance >= 0.0) || isinf(max_distance))
+        return MORNA_ERR_INVALID_ARGUMENT;
+    const RangeWs w = range_ws_layout(nq, ld_h);
+    if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned char *ws = (unsigned char *)workspace;
+    __half *hq = (__half *)(ws + w.hq);
+    double *qq = (double *)(ws + w.qq);
+    float *eps = (float *)(ws + w.eps);
+    float *thr = (float *)(ws + w.thr);
+    int32_t *cand_cnt = (int32_t *)(ws + w.cand_cnt);
+    int32_t *match_cnt = (int32_t *)(ws + w.match_cnt);
+    MORNA_CUDA_TRY(cudaMemsetAsync(overflow, 0, (size_t)nq, s));
+    MORNA_CUDA_TRY(cudaMemsetAsync(stats, 0, 4 * sizeof(int64_t), s));
+    MORNA_CUDA_TRY(cudaMemsetAsync(cand_cnt, 0, (size_t)nq * sizeof(int32_t), s));
+    MORNA_CUDA_TRY(cudaMemsetAsync(match_cnt, 0, (size_t)nq * sizeof(int32_t), s));
+    MORNA_CUDA_TRY(cudaMemsetAsync(ws + w.prep_stats, 0, 4 * sizeof(int32_t), s));
+
+    const float eps_acc = (float)((double)(dim / 16 + 8) * 2.384185791015625e-07 * 1.01);     // as in score_impl
+    {
+        int64_t blocks = (w.nq_pad + 7) / 8;
+        if (blocks > (int64_t)sm_count_b() * 8) blocks = (int64_t)sm_count_b() * 8;
+        prep_queries_kernel<<<(unsigned)blocks, kPrepThreads, 0, s>>>(queries, nq, w.nq_pad, dim, q_ld, hq, ld_h, qq, eps, rho_max,
+                                                                    eps_acc, overflow, (int32_t *)(ws + w.prep_stats));
+        MORNA_LAUNCH_CHECK();
+    }
+    range_thr_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(eps, overflow, (int32_t)nq, max_distance, thr);
+    MORNA_LAUNCH_CHECK();
+
+    CUtensorMap tmap_q, tmap_s;
+    int rc = make_tmap(&tmap_q, hq, (uint64_t)w.nq_pad, (uint64_t)ld_h, gemm::BM);
+    if (rc != MORNA_OK) return rc;
+    rc = make_tmap(&tmap_s, hs, (uint64_t)n, (uint64_t)ld_h,
+                   g_gemm_pair == 2 && (w.nq_pad / gemm::BM) % 4 == 0 ? gemm2::BN_HALF / 2 : g_gemm_pair ? gemm2::BN_HALF : gemm::BN);
+    if (rc != MORNA_OK) return rc;
+    GemmParams gp{};
+    gp.debug = g_gemm_debug; gp.relaxed_ns = g_gemm_relaxed_ns; gp.l2_keep = g_gemm_l2_keep;
+    gp.nq = (int32_t)nq; gp.kblocks = (int32_t)(ld_h / gemm::BK); gp.m_blocks = (int32_t)(w.nq_pad / gemm::BM);
+    gp.cap = kCandCap; gp.id_base = id_base; gp.thr = thr;
+    gp.cand_score = (float *)(ws + w.cand_score); gp.cand_id = (int32_t *)(ws + w.cand_id); gp.cand_cnt = cand_cnt;
+    gp.n_begin = 0; gp.n_end = (int32_t)n; gp.mode = 1;
+    gp.n_tiles = (int32_t)((n + gemm::BN - 1) / gemm::BN);
+    if ((rc = launch_knn_gemm(tmap_q, tmap_s, gp, s)) != MORNA_OK) return rc;
+
+    RangeCheckParams cp{};
+    cp.vectors = vectors; cp.pp = pp; cp.ld = ld; cp.dim = dim; cp.id_base = id_base; cp.nq = (int32_t)nq;
+    cp.queries = queries; cp.q_ld = q_ld; cp.qq = qq; cp.cand_id = gp.cand_id; cp.cand_cnt = cand_cnt; cp.overflow = overflow;
+    cp.R = max_distance; cp.match_id = (int32_t *)(ws + w.match_id); cp.match_dist = (double *)(ws + w.match_dist);
+    cp.match_cnt = match_cnt;
+    int per_sm = 0;
+    MORNA_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, range_check_kernel, kRangeWarps * 32, 0));
+    if (per_sm < 1) per_sm = 1;
+    const int64_t items = nq * (kCandCap / 32);
+    int64_t grid = (int64_t)per_sm * sm_count_b();
+    if (grid * kRangeWarps > items) grid = (items + kRangeWarps - 1) / kRangeWarps;
+    range_check_kernel<<<(unsigned)grid, kRangeWarps * 32, 0, s>>>(cp);
+    MORNA_LAUNCH_CHECK();
+    range_finish_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(cand_cnt, match_cnt, (int32_t)nq, overflow, counts,
+                                                                    (unsigned long long *)stats);
+    MORNA_LAUNCH_CHECK();
+    return MORNA_OK;
+}
+
+extern "C" int morna_range_batched_emit(int64_t n, int64_t nq, int32_t dim, const int64_t *offsets, const uint8_t *overflow,
+                                        int32_t *out_ids, double *out_dist, const void *workspace, size_t workspace_bytes,
+                                        void *stream) {
+    if (!offsets || !overflow || !out_ids || !out_dist || n <= 0 || n > kBatchedMaxRows || nq <= 0 || nq > kRangeMaxQueries ||
+        dim <= 0)
+        return MORNA_ERR_INVALID_ARGUMENT;
+    const RangeWs w = range_ws_layout(nq, morna_tensor_operand_ld(dim));
+    if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
+    const unsigned char *ws = (const unsigned char *)workspace;
+    const size_t smem = (size_t)kCandCap * (sizeof(double) + sizeof(int));
+    { int rca = ensure_dynamic_smem((const void *)range_emit_kernel, smem); if (rca != MORNA_OK) return rca; }
+    range_emit_kernel<<<(unsigned)nq, kRangeEmitThreads, smem, (cudaStream_t)stream>>>(
+        (const int32_t *)(ws + w.match_id), (const double *)(ws + w.match_dist), (const int32_t *)(ws + w.match_cnt), overflow,
+        offsets, out_ids, out_dist);
+    MORNA_LAUNCH_CHECK();
+    return MORNA_OK;
+}
+
 /* Experiment knobs, process-wide: key 0 = GEMM variant (1 CTA pairs / 0 single CTA),
  * key 1 = shared-memory pipeline stages of the pair variant (4 or 6). */
 namespace morna { void set_single_tma(int v); void set_acc_pipelined(int v); void set_acc_split(int v); void set_acc_variant(int v); void set_acc_shift(int v); void set_ids_early_exit(int v); void set_single_prefetch(int v); void set_single_prefetch_rows(int v); void set_single_chain(int v); void set_sparse_tile_mb(int v); }

@@ -19,6 +19,30 @@ from .index import round_up
 PHASE_NAMES = ("prep_queries", "gemm_pilot", "kth_pilot", "gemm_filter", "kth_final", "rerank_select")
 
 
+def check_radius(max_distance):
+    """A range search radius as a float: finite and >= 0, else ValueError."""
+    r = float(max_distance)
+    if not (math.isfinite(r) and r >= 0.0):
+        raise ValueError("max_distance must be a finite number >= 0, got %r" % (max_distance,))
+    return r
+
+
+def _range_groups(counts, byte_cap):
+    """[lo, hi) runs of consecutive queries whose lists (12 bytes per match) fit byte_cap; one run without a cap."""
+    nq = len(counts)
+    if byte_cap is None:
+        return [(0, nq)] if nq else []
+    groups, lo, size = [], 0, 0
+    for j, c in enumerate(np.asarray(counts, dtype=np.int64).tolist()):
+        if j > lo and size + 12 * c > byte_cap:
+            groups.append((lo, j))
+            lo, size = j, 0
+        size += 12 * c
+    if nq:
+        groups.append((lo, nq))
+    return groups
+
+
 def make_phase_events():
     """Seven CUDA events for morna_knn_batched's phase boundaries: (events, ctypes array)."""
     import ctypes
@@ -647,9 +671,10 @@ class MornaSearch(object):
         return results
 
     def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
-                        meta_db=False, out=None):
+                        meta_db=False, out=None, max_distance=None):
         """morna.py:733-787 with the stored row as the query (float32 values), run
-        through the exact scan."""
+        through the exact scan.  With ``max_distance``: every sample within it (range_search_nn), the first
+        ``num_neighbors`` of them when that is not None."""
         import sys
         out = out or sys.stdout
         out.write("querying by sample id " + str(query_id) + "\n")
@@ -663,11 +688,175 @@ class MornaSearch(object):
         if not (self.row_lo <= internal_id < self.row_hi):
             raise ValueError("internal id %d is not resident on this shard" % internal_id)
         self.query_sample = self.vectors[internal_id - self.row_lo, :self.dim].to(torch.float64).cpu().tolist()
+        if max_distance is not None:
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors)
         return self.exact_search_nn(num_neighbors, include_distances, meta_db)
 
     def _metadata(self, internal_ids):
         """morna.py:666-676: keywords of every result's sample id from basename.meta.mor."""
         return files.read_meta(self.basename, [self.inverse_lookup(iid) for iid in internal_ids])
+
+    # ------------------------------------------------------------------ range search
+    RANGE_BATCH_QUERIES = 4096        # queries per morna_range_batched call (its candidate lists: 4096 x 4096 entries)
+    RANGE_TENSOR_MIN_QUERIES = 64     # smaller batches go to the FP64 scan, as top-k batches do
+
+    def range_search_device(self, queries, max_distance):
+        """Every row within ``max_distance`` of each query: queries CUDA float64 [nq x dim] -> device CSR (offsets int64
+        [nq+1], ids int32 [total], dists float64 [total]); query j's list is ids/dists[offsets[j]:offsets[j+1]], ordered as
+        the reference orders results (distance ascending, equal distances id descending), ids global.  The distance is
+        exactly exact_search_device's and the comparison inclusive; a query with nothing in range has an empty list.
+        Sets ``last_stats`` = [overflowed queries, first-pass survivors, matches] and ``last_range_route`` ("tensor":
+        the tensor-core filter with an FP64 check, overflowed queries answered by the scan; "exact": the FP64 scan)."""
+        parts = list(self.range_search_groups(queries, max_distance))
+        if not parts:
+            dev = self.device
+            return (torch.zeros(1, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
+                    torch.zeros(0, dtype=torch.float64, device=dev))
+        offsets, base = [parts[0][2][:1]], 0
+        for p in parts:
+            offsets.append(p[2][1:] + base)
+            base += p[3].numel()
+        return torch.cat(offsets), torch.cat([p[3] for p in parts]), torch.cat([p[4] for p in parts])
+
+    def range_search_groups(self, queries, max_distance, byte_cap=None):
+        """Generator over (lo, hi, offsets, ids, dists): the range_search_device CSR of queries [lo, hi), in query order.
+        Batches of RANGE_BATCH_QUERIES are counted first (one small read back); with ``byte_cap``, a batch whose lists
+        would take more than that many bytes (12 per match) is emitted in groups of consecutive queries that fit it (one
+        query per group at least), so no more than that is allocated at once."""
+        r = check_radius(max_distance)
+        assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2 and queries.shape[1] == self.dim
+        queries = queries.contiguous()
+        nq = queries.shape[0]
+        route = self._range_route(nq)
+        stats = [0, 0, 0]
+        self.last_range_route, self.last_stats = route, list(stats)
+        for b0 in range(0, nq, self.RANGE_BATCH_QUERIES):
+            st = self._range_counts(queries[b0:b0 + self.RANGE_BATCH_QUERIES], r, route)
+            stats = [a + b for a, b in zip(stats, st["stats"])]
+            self.last_stats = list(stats)
+            for lo, hi in _range_groups(st["counts"], byte_cap):
+                off, ids, d = self._range_emit(st, lo, hi)
+                yield b0 + lo, b0 + hi, off, ids, d
+
+    def range_search_batch(self, queries, max_distance):
+        """Host entry: queries numpy [nq x dim] -> numpy CSR (offsets, ids, dists) of range_search_device."""
+        queries = np.ascontiguousarray(queries)
+        if queries.dtype != np.float32:
+            queries = queries.astype(np.float64, copy=False)
+        q = torch.from_numpy(queries)
+        if q.numel():
+            q = q.pin_memory()
+        qd = q.to(self.device, non_blocking=True).to(torch.float64)
+        return tuple(t.cpu().numpy() for t in self.range_search_device(qd, max_distance))
+
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None):
+        """Every indexed sample within ``max_distance`` of the current ``query_sample``, as exact_search_nn returns its
+        results; ``num_neighbors``: keep only the first that many."""
+        _, ids, d = self.range_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], max_distance)
+        if num_neighbors is not None:
+            ids, d = ids[:max(int(num_neighbors), 0)], d[:max(int(num_neighbors), 0)]
+        results = (ids.tolist(),)
+        if include_distances:
+            results += (d.tolist(),)
+        if meta_db:
+            results += (self._metadata(results[0]),)
+        return results
+
+    def _range_route(self, nq):
+        n = self.row_hi - self.row_lo
+        sparse_ties = self.csr is not None and self.sparse_exact         # its parallel rows would overflow every list
+        tensor = 0 < n <= self.BATCH_BLOCK_ROWS and nq >= self.RANGE_TENSOR_MIN_QUERIES and not sparse_ties
+        return "tensor" if tensor else "exact"
+
+    def _range_counts(self, queries, r, route):
+        """Matches per query of one batch (host int64) and what _range_emit needs; on the tensor route the counts,
+        overflow flags and stats come back in one copy, and overflowed queries are counted again by the scan."""
+        nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
+        st = {"queries": queries, "r": r, "route": route, "over": np.zeros(0, np.int64), "stats": [0, 0, 0],
+              "counts": np.zeros(nq, np.int64)}
+        if n == 0 or nq == 0:
+            return st
+        with torch.cuda.device(dev):
+            if route == "exact":
+                st["counts"] = self._range_exact_counts(queries, r)
+            else:
+                self.enable_tensor_path()
+                counts = torch.empty(nq, dtype=torch.int32, device=dev)
+                overflow = torch.empty(nq, dtype=torch.uint8, device=dev)
+                stats = torch.empty(4, dtype=torch.int64, device=dev)
+                ws = self._workspace(self.lib.morna_range_batched_workspace_bytes(n, nq, self.dim), "range")
+                _lib.check(self.lib.morna_range_batched(
+                    _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), _lib.dev_ptr(self.hs), self.ld_h, _lib.dev_ptr(self.rho_max),
+                    n, self.dim, self.ld, self.row_lo, _lib.ptr(queries), nq, self.dim, r, _lib.dev_ptr(counts),
+                    _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()),
+                    "morna_range_batched")
+                host = torch.cat([counts.to(torch.int64), overflow.to(torch.int64), stats]).cpu().numpy()
+                c, over = host[:nq].copy(), np.nonzero(host[nq:2 * nq])[0]
+                if len(over):
+                    c[over] = self._range_exact_counts(queries[torch.from_numpy(over).to(dev)], r)
+                st.update(counts=c, over=over, ws=ws, overflow=overflow)
+                st["stats"] = [int(host[2 * nq]), int(host[2 * nq + 1]), 0]
+        st["stats"][2] = int(st["counts"].sum())
+        return st
+
+    def _range_exact_counts(self, queries, r):
+        nq, n = queries.shape[0], self.row_hi - self.row_lo
+        counts = torch.empty(nq, dtype=torch.int32, device=self.device)
+        ws = self._workspace(self.lib.morna_range_exact_workspace_bytes(n, nq, 0), "range_exact")
+        _lib.check(self.lib.morna_range_exact_count(
+            _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.ptr(queries), nq, self.dim, r,
+            _lib.dev_ptr(counts), _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_range_exact_count")
+        return counts.cpu().numpy().astype(np.int64)
+
+    def _range_exact_fill(self, queries, r, counts):
+        """FP64 route's lists of `queries` given their counts: device (offsets, ids, dists)."""
+        nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
+        off = np.zeros(nq + 1, dtype=np.int64)
+        np.cumsum(counts, out=off[1:])
+        total = int(off[-1])
+        offsets = torch.from_numpy(off).to(dev)
+        ids = torch.empty(total, dtype=torch.int32, device=dev)
+        d = torch.empty(total, dtype=torch.float64, device=dev)
+        if total:
+            ws = self._workspace(self.lib.morna_range_exact_workspace_bytes(n, nq, total), "range_exact")
+            _lib.check(self.lib.morna_range_exact_fill(
+                _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, self.row_lo, _lib.ptr(queries), nq,
+                self.dim, r, _lib.dev_ptr(offsets), total, _lib.dev_ptr(ids), _lib.dev_ptr(d), _lib.dev_ptr(ws), ws.numel(),
+                _lib.stream_ptr()), "morna_range_exact_fill")
+        return offsets, ids, d
+
+    def _range_emit(self, st, lo, hi):
+        """Device CSR of queries [lo, hi) of a counted batch."""
+        dev, n = self.device, self.row_hi - self.row_lo
+        with torch.cuda.device(dev):
+            if st["route"] == "exact" or n == 0:
+                return self._range_exact_fill(st["queries"][lo:hi], st["r"], st["counts"][lo:hi])
+            nq = st["queries"].shape[0]
+            counts = st["counts"]
+            full = np.zeros(nq + 1, dtype=np.int64)              # queries outside [lo, hi) get empty ranges
+            np.cumsum(counts[lo:hi], out=full[lo + 1:hi + 1])
+            full[hi + 1:] = full[hi]
+            total = int(full[hi])
+            offsets = torch.from_numpy(full).to(dev)
+            ids = torch.empty(total, dtype=torch.int32, device=dev)
+            d = torch.empty(total, dtype=torch.float64, device=dev)
+            if total:
+                ws = st["ws"]
+                _lib.check(self.lib.morna_range_batched_emit(
+                    n, nq, self.dim, _lib.dev_ptr(offsets), _lib.dev_ptr(st["overflow"]), _lib.dev_ptr(ids), _lib.dev_ptr(d),
+                    _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_range_batched_emit")
+            over = st["over"][(st["over"] >= lo) & (st["over"] < hi)]
+            if len(over):                                        # the scan's lists spliced into their places
+                sub_off, sub_ids, sub_d = self._range_exact_fill(st["queries"][torch.from_numpy(over).to(dev)], st["r"],
+                                                                 counts[over])
+                sub_total = sub_ids.numel()
+                if sub_total:
+                    lens = torch.from_numpy(counts[over]).to(dev)
+                    shift = offsets[torch.from_numpy(over).to(dev)] - sub_off[:-1]
+                    dst = torch.repeat_interleave(shift, lens, output_size=sub_total) + torch.arange(sub_total, device=dev)
+                    ids[dst] = sub_ids
+                    d[dst] = sub_d
+            return offsets[lo:hi + 1], ids, d
 
 
 class _PipeSlot(object):
