@@ -397,6 +397,21 @@ int morna_range_exact_fill(const float *vectors, const double *pp, int64_t n, in
                            int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
                            void *stream);
 
+/* Merge of per-rank range lists (the rows-sharded range search, after one all-gather of packed per-rank buffers).
+ *   gathered     [dev] n_lists buffers back to back, 8-byte aligned; buffer g is cap doubles (distances) followed by cap
+ *                int32 (ids), cap even (so every buffer stays 8-byte aligned), the same cap for every rank
+ *   rank_offsets [dev] int64[n_lists * (nq + 1)]: rank g's CSR offsets (rank_offsets[g * (nq + 1)] = 0); query j's list
+ *                of rank g is entries [off[j], off[j + 1]) of buffer g, off[nq] <= cap, slots past off[nq] are padding
+ *   out_offsets  [dev] int64[nq + 1]: out_offsets[j] = sum over ranks of query j's earlier lists (out_offsets[0] = 0);
+ *                total = out_offsets[nq]
+ *   out_ids / out_dist [dev] [total]: query j's merged list at [out_offsets[j], out_offsets[j + 1])
+ * Preconditions: each rank's list for a query is ordered under the reference order (distance ascending, equal distances
+ * id descending), and no id occurs on two ranks.  The merge is a permutation (ids and distance bits copied unchanged),
+ * by rank counting: an entry's place is its index in its own list plus, per other rank, the entries of that rank's list
+ * for the same query that come before it.  Any list length; nq == 0 or total == 0 does nothing. */
+int morna_merge_sorted_csr(const void *gathered, int32_t n_lists, int64_t nq, int64_t cap, const int64_t *rank_offsets,
+                           const int64_t *out_offsets, int64_t total, int32_t *out_ids, double *out_dist, void *stream);
+
 /* Test hook: raw fp16 tensor-core scores [nq x n] (n <= 8192) and the per-query bound eps. */
 int morna_debug_tensor_scores(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
                               const double *queries, int64_t nq, int64_t q_ld, float *scores,

@@ -98,6 +98,7 @@ _SIGNATURES = {
                                                _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_range_exact_fill": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, ctypes.c_double,
                                               _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_merge_sorted_csr": (ctypes.c_int, [_c_vp, _c_i32, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp]),
     "morna_debug_tensor_scores": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_vp,
                                                  _c_i64, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_set_tuning": (ctypes.c_int, [_c_i32, _c_i32]),

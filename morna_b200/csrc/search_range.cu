@@ -8,6 +8,8 @@
 // rather than keep n distances per query between the calls.  Each query tile writes n doubles per query to the
 // scratch and reads them back once per call; the fill then sorts 12 bytes per match (segmented radix sort over the
 // 64 key bits, about 2x the list in extra scratch).
+//
+// morna_merge_sorted_csr, at the end, merges the per-rank lists of the rows-sharded range search (morna_b200/dist.py).
 #include <math.h>
 
 #include <cub/block/block_scan.cuh>
@@ -100,6 +102,51 @@ static bool range_args_ok(const float *vectors, const double *pp, int64_t n, int
            R >= 0.0 && !isinf(R);
 }
 
+// Merge of the rows-sharded range search: one thread per slot of the all-gathered buffer.  A slot past its rank's last
+// entry is padding.  The entry finds its query by binary search in its rank's offsets, then its output position as its
+// index in its own list plus, for every other rank, how many of that rank's entries for the query come before it
+// (binary search in global memory).  Lists of any length: nothing is staged in shared memory.
+constexpr int kMergeCsrThreads = 256;
+
+__global__ void __launch_bounds__(kMergeCsrThreads)
+merge_sorted_csr_kernel(const unsigned char *__restrict__ gathered, int32_t n_lists, int64_t nq, int64_t cap,
+                        const int64_t *__restrict__ rank_offsets, const int64_t *__restrict__ out_offsets,
+                        int32_t *__restrict__ out_ids, double *__restrict__ out_dist) {
+    const int64_t t = (int64_t)blockIdx.x * kMergeCsrThreads + threadIdx.x;
+    if (t >= (int64_t)n_lists * cap) return;
+    const int g = (int)(t / cap);
+    const int64_t e = t - (int64_t)g * cap;
+    const int64_t *off = rank_offsets + (int64_t)g * (nq + 1);
+    if (e >= off[nq]) return;
+    int64_t lo = 0, hi = nq;                                   // the query j with off[j] <= e < off[j + 1]
+    while (hi - lo > 1) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (off[mid] <= e) lo = mid; else hi = mid;
+    }
+    const int64_t j = lo;
+    const size_t rank_bytes = (size_t)cap * 12;
+    const double *dg = reinterpret_cast<const double *>(gathered + (size_t)g * rank_bytes);
+    const int32_t *ig = reinterpret_cast<const int32_t *>(gathered + (size_t)g * rank_bytes + (size_t)cap * 8);
+    const double d = dg[e];
+    const int32_t id = ig[e];
+    int64_t pos = out_offsets[j] + (e - off[j]);
+    for (int h = 0; h < n_lists; ++h) {
+        if (h == g) continue;
+        const int64_t *oh = rank_offsets + (int64_t)h * (nq + 1);
+        const double *dh = reinterpret_cast<const double *>(gathered + (size_t)h * rank_bytes);
+        const int32_t *ih = reinterpret_cast<const int32_t *>(gathered + (size_t)h * rank_bytes + (size_t)cap * 8);
+        int64_t a = oh[j], b = oh[j + 1];                      // first entry of rank h's list that does NOT come before
+        const int64_t start = a;
+        while (a < b) {
+            const int64_t mid = (a + b) >> 1;
+            if (before(dh[mid], ih[mid], d, id)) a = mid + 1; else b = mid;
+        }
+        pos += a - start;
+    }
+    out_ids[pos] = id;
+    out_dist[pos] = d;
+}
+
 }  // namespace morna
 
 using namespace morna;
@@ -159,5 +206,22 @@ extern "C" int morna_range_exact_fill(const float *vectors, const double *pp, in
         MORNA_CUDA_TRY(cudaMemcpyAsync(out_dist, kb.Current(), (size_t)total * sizeof(double), cudaMemcpyDeviceToDevice, s));
         MORNA_CUDA_TRY(cudaMemcpyAsync(out_ids, vb.Current(), (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
     }
+    return MORNA_OK;
+}
+
+extern "C" int morna_merge_sorted_csr(const void *gathered, int32_t n_lists, int64_t nq, int64_t cap, const int64_t *rank_offsets,
+                                      const int64_t *out_offsets, int64_t total, int32_t *out_ids, double *out_dist,
+                                      void *stream) {
+    if (n_lists <= 0 || nq < 0 || cap < 0 || (cap & 1) || total < 0 || total > (int64_t)n_lists * cap)
+        return MORNA_ERR_INVALID_ARGUMENT;
+    if (nq == 0 || total == 0) return MORNA_OK;
+    if (!gathered || ((uintptr_t)gathered & 7) || !rank_offsets || !out_offsets || !out_ids || !out_dist)
+        return MORNA_ERR_INVALID_ARGUMENT;
+    const int64_t slots = (int64_t)n_lists * cap;
+    const int64_t blocks = (slots + kMergeCsrThreads - 1) / kMergeCsrThreads;
+    if (blocks > INT32_MAX) return MORNA_ERR_INVALID_ARGUMENT;
+    merge_sorted_csr_kernel<<<(unsigned)blocks, kMergeCsrThreads, 0, (cudaStream_t)stream>>>(
+        (const unsigned char *)gathered, n_lists, nq, cap, rank_offsets, out_offsets, out_ids, out_dist);
+    MORNA_LAUNCH_CHECK();
     return MORNA_OK;
 }

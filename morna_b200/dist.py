@@ -4,10 +4,16 @@ on its block, the per-rank top-k lists are all-gathered (NCCL over NVLink; gloo 
 CPU tests) and merged under the reference order.  The union of per-shard exact
 top-k lists contains the global top-k, so the result equals one process scanning
 all rows (morna.py:697-712).  This is the only exchange step on the path.
+
+Range search (every row within a distance) runs over the same row blocks: sharded_range_search_groups below.
 """
+import struct
+
+import numpy as np
 import torch
 
 from . import _lib
+from .search import _range_groups, check_radius, concat_range_groups
 
 
 def shard_bounds(n_rows, rank, world):
@@ -153,3 +159,119 @@ def gather_merge_packed(ids, dists, k, group=None, packed=None):
         _lib.check(lib.morna_merge_packed_topk(_lib.dev_ptr(every), world, nq, k_in, k, _lib.dev_ptr(out_i), _lib.dev_ptr(out_d),
                                                _lib.stream_ptr()), "morna_merge_packed_topk")
     return out_i, out_d
+
+
+# ------------------------------------------------------------------ range search over a rows-sharded index
+# A range list has no fixed length, so the ranks first agree on sizes: every size of a later collective (the query
+# groups, each group's buffer) is computed from all-gathered counts, never from one rank's own counts.
+
+def _world_size(group):
+    import torch.distributed as td
+    return td.get_world_size(group) if (td.is_available() and td.is_initialized()) else 1
+
+
+def pack_range_lists(ids, dists, cap):
+    """One rank's send buffer of the list all-gather: `cap` doubles (distances), then `cap` int32 (ids), as uint8
+    [12 * cap] on the lists' device; slots past the lists are padding.  cap is even so every rank's buffer in the
+    gathered tensor stays 8-byte aligned."""
+    assert cap % 2 == 0 and ids.numel() == dists.numel() <= cap
+    buf = torch.empty(cap * 12, dtype=torch.uint8, device=ids.device)
+    m = ids.numel()
+    buf[:cap * 8].view(torch.float64)[:m].copy_(dists)
+    buf[cap * 8:].view(torch.int32)[:m].copy_(ids)
+    return buf
+
+
+def merge_sorted_csr(gathered, n_lists, nq, cap, rank_offsets, out_offsets, total, stream=None):
+    """morna_merge_sorted_csr: the merged (ids, dists) [total] of n_lists packed buffers (pack_range_lists) back to back
+    in `gathered`; rank_offsets int64 [n_lists * (nq + 1)] and out_offsets int64 [nq + 1] on the GPU."""
+    lib = _lib.load()
+    dev = gathered.device
+    out_i = torch.empty(total, dtype=torch.int32, device=dev)
+    out_d = torch.empty(total, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.morna_merge_sorted_csr(_lib.dev_ptr(gathered), n_lists, nq, cap, _lib.dev_ptr(rank_offsets),
+                                              _lib.dev_ptr(out_offsets), total, _lib.dev_ptr(out_i), _lib.dev_ptr(out_d),
+                                              _lib.stream_ptr(stream)), "morna_merge_sorted_csr")
+    return out_i, out_d
+
+
+def merge_gathered_csr(gathered, counts, cap, merge=None):
+    """The step after the list all-gather: `gathered` (flat uint8, world buffers of pack_range_lists(.., cap)) and
+    `counts` (host int64 [world x nq], every rank's matches per query of the group) -> the merged device CSR
+    (offsets [nq + 1], ids, dists).  `merge` replaces morna_merge_sorted_csr (same arguments as merge_sorted_csr)."""
+    counts = np.asarray(counts, dtype=np.int64)
+    world, nq = counts.shape
+    rank_off = np.zeros((world, nq + 1), dtype=np.int64)
+    np.cumsum(counts, axis=1, out=rank_off[:, 1:])
+    out_off = np.zeros(nq + 1, dtype=np.int64)
+    np.cumsum(counts.sum(axis=0), out=out_off[1:])
+    dev = gathered.device
+    rank_off_t = torch.from_numpy(rank_off.reshape(-1)).to(dev)
+    out_off_t = torch.from_numpy(out_off).to(dev)
+    ids, dists = (merge or merge_sorted_csr)(gathered, world, nq, cap, rank_off_t, out_off_t, int(out_off[-1]))
+    return out_off_t, ids, dists
+
+
+def _range_group_exchange(search, st, lo, hi, counts, group, merge):
+    """Queries [lo, hi) of a counted batch: this rank's lists, one all-gather, the merge.  counts: host [world x (hi-lo)]."""
+    import torch.distributed as td
+    dev = st["queries"].device
+    cap = int(counts.sum(axis=1).max())
+    cap += cap & 1
+    if cap == 0:                                      # no rank has a match: every rank skips the list collective
+        return (torch.zeros(hi - lo + 1, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
+                torch.zeros(0, dtype=torch.float64, device=dev))
+    _, ids, dists = search.range_emit(st, lo, hi)
+    mine = pack_range_lists(ids, dists, cap)
+    every = torch.empty(counts.shape[0] * mine.numel(), dtype=torch.uint8, device=dev)
+    td.all_gather_into_tensor(every, mine, group=group)
+    return merge_gathered_csr(every, counts, cap, merge)
+
+
+def sharded_range_search_groups(search, queries, max_distance, group=None, byte_cap=None, merge=None):
+    """Range search over a rows-sharded index, one process per GPU: generator over (lo, hi, offsets, ids, dists), the
+    device CSR of queries [lo, hi) in query order, as MornaSearch.range_search_groups.  `search` holds this rank's row
+    block (MornaSearch(..., shard=(rank, world))); `queries` (CUDA float64 [nq x dim]) and every argument are the same
+    on every rank.  Every rank yields the same groups and lists, equal bit for bit to one process holding all rows.
+
+      1. one all-gather of a header (nq, dim, radius bits, byte cap): ValueError on every rank if they differ;
+      2. per batch of RANGE_BATCH_QUERIES queries every rank counts its matches (its own route, overflow handling and
+         last_stats) and the counts are all-gathered; the query groups follow from the global counts alone, so the
+         gathered lists plus the merged ones stay under byte_cap (one query per group at least);
+      3. per group every rank writes its lists, ONE all-gather of the packed lists (skipped when no rank has a
+         match), and morna_merge_sorted_csr (or `merge`) puts every entry in its place.
+    Collectives use flat 1-D tensors on the queries' device (NCCL with CUDA tensors, gloo with CPU tensors)."""
+    import torch.distributed as td
+    world = _world_size(group)
+    if world == 1:
+        yield from search.range_search_groups(queries, max_distance, byte_cap)
+        return
+    dev = queries.device
+    nq = int(queries.shape[0])
+    r = float(max_distance)
+    head = torch.tensor([nq, int(queries.shape[1]), struct.unpack("<q", struct.pack("<d", r))[0],
+                         -1 if byte_cap is None else int(byte_cap)], dtype=torch.int64, device=dev)
+    every = torch.empty(world * head.numel(), dtype=torch.int64, device=dev)
+    td.all_gather_into_tensor(every, head, group=group)
+    rows = every.view(world, -1).cpu()
+    if not bool((rows == rows[0]).all()):
+        raise ValueError("sharded range search: the ranks' (queries, dim, radius bits, byte cap) differ: %s" % rows.tolist())
+    if nq == 0:
+        check_radius(r)
+        return
+    for b0, st in search.range_count_batches(queries, r):
+        counts = torch.from_numpy(np.ascontiguousarray(st["counts"], dtype=np.int64)).to(dev)
+        every = torch.empty(world * counts.numel(), dtype=torch.int64, device=dev)
+        td.all_gather_into_tensor(every, counts, group=group)
+        rank_counts = every.cpu().numpy().reshape(world, -1)
+        for lo, hi in _range_groups(rank_counts.sum(axis=0) * (world + 1), byte_cap):
+            yield (b0 + lo, b0 + hi) + tuple(_range_group_exchange(search, st, lo, hi, rank_counts[:, lo:hi], group, merge))
+
+
+def sharded_range_search(search, queries, max_distance, group=None, merge=None):
+    """The whole device CSR (offsets, ids, dists) of sharded_range_search_groups, as MornaSearch.range_search_device."""
+    if _world_size(group) == 1:
+        return search.range_search_device(queries, max_distance)
+    return concat_range_groups(list(sharded_range_search_groups(search, queries, max_distance, group, merge=merge)),
+                               queries.device)

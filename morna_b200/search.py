@@ -43,6 +43,18 @@ def _range_groups(counts, byte_cap):
     return groups
 
 
+def concat_range_groups(parts, device):
+    """One CSR (offsets, ids, dists) from consecutive (lo, hi, offsets, ids, dists) groups of a range search."""
+    if not parts:
+        return (torch.zeros(1, dtype=torch.int64, device=device), torch.zeros(0, dtype=torch.int32, device=device),
+                torch.zeros(0, dtype=torch.float64, device=device))
+    offsets, base = [parts[0][2][:1]], 0
+    for p in parts:
+        offsets.append(p[2][1:] + base)
+        base += p[3].numel()
+    return torch.cat(offsets), torch.cat([p[3] for p in parts]), torch.cat([p[4] for p in parts])
+
+
 def make_phase_events():
     """Seven CUDA events for morna_knn_batched's phase boundaries: (events, ctypes array)."""
     import ctypes
@@ -707,22 +719,22 @@ class MornaSearch(object):
         exactly exact_search_device's and the comparison inclusive; a query with nothing in range has an empty list.
         Sets ``last_stats`` = [overflowed queries, first-pass survivors, matches] and ``last_range_route`` ("tensor":
         the tensor-core filter with an FP64 check, overflowed queries answered by the scan; "exact": the FP64 scan)."""
-        parts = list(self.range_search_groups(queries, max_distance))
-        if not parts:
-            dev = self.device
-            return (torch.zeros(1, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
-                    torch.zeros(0, dtype=torch.float64, device=dev))
-        offsets, base = [parts[0][2][:1]], 0
-        for p in parts:
-            offsets.append(p[2][1:] + base)
-            base += p[3].numel()
-        return torch.cat(offsets), torch.cat([p[3] for p in parts]), torch.cat([p[4] for p in parts])
+        return concat_range_groups(list(self.range_search_groups(queries, max_distance)), self.device)
 
     def range_search_groups(self, queries, max_distance, byte_cap=None):
         """Generator over (lo, hi, offsets, ids, dists): the range_search_device CSR of queries [lo, hi), in query order.
         Batches of RANGE_BATCH_QUERIES are counted first (one small read back); with ``byte_cap``, a batch whose lists
         would take more than that many bytes (12 per match) is emitted in groups of consecutive queries that fit it (one
         query per group at least), so no more than that is allocated at once."""
+        for b0, st in self.range_count_batches(queries, max_distance):
+            for lo, hi in _range_groups(st["counts"], byte_cap):
+                off, ids, d = self.range_emit(st, lo, hi)
+                yield b0 + lo, b0 + hi, off, ids, d
+
+    def range_count_batches(self, queries, max_distance):
+        """The counting half of range_search_groups: generator over (b0, st), one per batch of RANGE_BATCH_QUERIES
+        queries starting at query b0, where st["counts"] (host int64) holds the batch's matches per query and st is what
+        range_emit needs to write any run of its lists.  Updates last_range_route and last_stats as the batches go."""
         r = check_radius(max_distance)
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2 and queries.shape[1] == self.dim
         queries = queries.contiguous()
@@ -734,9 +746,7 @@ class MornaSearch(object):
             st = self._range_counts(queries[b0:b0 + self.RANGE_BATCH_QUERIES], r, route)
             stats = [a + b for a, b in zip(stats, st["stats"])]
             self.last_stats = list(stats)
-            for lo, hi in _range_groups(st["counts"], byte_cap):
-                off, ids, d = self._range_emit(st, lo, hi)
-                yield b0 + lo, b0 + hi, off, ids, d
+            yield b0, st
 
     def range_search_batch(self, queries, max_distance):
         """Host entry: queries numpy [nq x dim] -> numpy CSR (offsets, ids, dists) of range_search_device."""
@@ -769,7 +779,7 @@ class MornaSearch(object):
         return "tensor" if tensor else "exact"
 
     def _range_counts(self, queries, r, route):
-        """Matches per query of one batch (host int64) and what _range_emit needs; on the tensor route the counts,
+        """Matches per query of one batch (host int64) and what range_emit needs; on the tensor route the counts,
         overflow flags and stats come back in one copy, and overflowed queries are counted again by the scan."""
         nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
         st = {"queries": queries, "r": r, "route": route, "over": np.zeros(0, np.int64), "stats": [0, 0, 0],
@@ -825,8 +835,9 @@ class MornaSearch(object):
                 _lib.stream_ptr()), "morna_range_exact_fill")
         return offsets, ids, d
 
-    def _range_emit(self, st, lo, hi):
-        """Device CSR of queries [lo, hi) of a counted batch."""
+    def range_emit(self, st, lo, hi):
+        """Device CSR (offsets [hi - lo + 1] from 0, ids, dists) of queries [lo, hi) of a batch range_count_batches
+        counted."""
         dev, n = self.device, self.row_hi - self.row_lo
         with torch.cuda.device(dev):
             if st["route"] == "exact" or n == 0:
