@@ -14,6 +14,7 @@ import torch
 from . import _lib, files, parse
 from .index import round_up
 from .parse import RowBatch
+from .search import FilteredSearch
 
 # Above this many bytes of query vectors in flight (nq * dim * 16: the bucket-major accumulator and its transpose), the
 # vectors are built and searched in slices of query ids.
@@ -235,14 +236,22 @@ def search_query_file(search, path, k, exact=True, cap=None):
             yield qf.sample_ids[lo + b:lo + b + ids.shape[0]], ids.copy(), d.copy()
 
 
+def all_sample_ids(search):
+    """Internal ids of the samples --all-samples queries: every indexed sample, or every sample of a FilteredSearch's
+    subset (its k-NN or range graph)."""
+    if isinstance(search, FilteredSearch):
+        return search.member_ids
+    return np.arange(search.index_size, dtype=np.int64)
+
+
 def search_all_samples(search, k, inverse):
     """Every indexed sample by internal id (the stored rows as queries, as `search -q`), exactly; only ids cross PCIe.
     Yields (sample ids, ids, dists) numpy arrays as search_query_file does."""
-    n = search.index_size
-    starts = range(0, n, BATCH_QUERIES)
-    batches = (np.arange(b, min(n, b + BATCH_QUERIES), dtype=np.int64) for b in starts)
+    members = all_sample_ids(search)
+    starts = range(0, len(members), BATCH_QUERIES)
+    batches = (members[b:b + BATCH_QUERIES] for b in starts)
     for b, (ids, d) in zip(starts, search.search_batches(batches, k)):
-        yield inverse[b:b + ids.shape[0]], ids.copy(), d.copy()
+        yield inverse[members[b:b + ids.shape[0]]], ids.copy(), d.copy()
 
 
 def search_query_file_range(search, path, max_distance, cap=None, result_cap=None):
@@ -262,13 +271,17 @@ def search_query_file_range(search, path, max_distance, cap=None, result_cap=Non
 def search_all_samples_range(search, max_distance, inverse, result_cap=None):
     """Range variant of search_all_samples: the stored rows as queries, built on the device from their ids.  Yields
     (sample ids, offsets, ids, dists) numpy CSR batches as search_query_file_range does."""
-    n = search.index_size
+    members = all_sample_ids(search)
     result_cap = SLICE_BYTES_CAP if result_cap is None else result_cap
-    for b in range(0, n, BATCH_QUERIES):
-        rows = torch.arange(b, min(n, b + BATCH_QUERIES), device=search.device) - search.row_lo
-        q = search.vectors[rows, :search.dim].to(torch.float64).contiguous()
+    for b in range(0, len(members), BATCH_QUERIES):
+        batch = members[b:b + BATCH_QUERIES]
+        if isinstance(search, FilteredSearch):
+            q = search.stored_queries(batch)
+        else:
+            rows = torch.arange(b, b + len(batch), device=search.device) - search.row_lo
+            q = search.vectors[rows, :search.dim].to(torch.float64).contiguous()
         for g0, g1, off, ids, d in search.range_search_groups(q, max_distance, result_cap):
-            yield inverse[b + g0:b + g1], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
+            yield inverse[batch[g0:g1]], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
 
 
 def cut_lists(offsets, ids, dists, limit):

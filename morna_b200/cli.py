@@ -108,7 +108,12 @@ def build_parser():
                                     "result prefixed by the sample id and a tab")
     search_parser.add_argument("--all-samples", action="store_const", const=True, default=False,
                                help="search for every indexed sample (as -q for each sample id), one line per result "
-                                    "prefixed by the sample id and a tab")
+                                    "prefixed by the sample id and a tab; with --samples / --exclude-samples, for every "
+                                    "sample of the subset (the k-NN or range graph of the subset)")
+    search_parser.add_argument("--samples", metavar="<file>", type=str, required=False, default=None,
+                               help="search only among these indexed samples: a file with one sample id per line")
+    search_parser.add_argument("--exclude-samples", metavar="<file>", type=str, required=False, default=None,
+                               help="search among every indexed sample except these: a file with one sample id per line")
     search_parser.add_argument("--max-distance", metavar="<float>", type=float, required=False, default=None,
                                help="return every sample within this angular distance of the query (exact; -r N, if "
                                     "given, keeps the first N per query)")
@@ -128,6 +133,51 @@ def build_parser():
     return parser
 
 
+def sample_filter(args):
+    """--samples / --exclude-samples: the internal ids of the samples to search among (numpy int64, ascending), or None
+    without either flag.  Raises ValueError with the message for the user when the flags or the file are not usable."""
+    given = [(flag, path) for flag, path in (("--samples", getattr(args, "samples", None)),
+                                             ("--exclude-samples", getattr(args, "exclude_samples", None))) if path is not None]
+    if not given:
+        return None
+    if len(given) > 1:
+        raise ValueError("--samples cannot be combined with --exclude-samples")
+    flag, path = given[0]
+    try:
+        with open(path) as fh:
+            lines = fh.read().splitlines()
+    except (OSError, UnicodeDecodeError) as exc:
+        raise ValueError("%s: cannot read %s: %s" % (flag, path, exc))
+    listed = {}
+    for number, line in enumerate(lines, 1):
+        text = line.strip()
+        if not text:
+            continue
+        try:
+            listed.setdefault(int(text), number)
+        except ValueError:
+            raise ValueError("%s: line %d of %s is not an integer sample id: %r" % (flag, number, path, text))
+    import numpy as np
+    from . import files
+    id_map = files.read_map(args.basename)
+    for sample_id, number in listed.items():
+        if sample_id not in id_map:
+            raise ValueError("%s: sample id %d (line %d of %s) is not in the index: no internal id is mapped to that "
+                             "sample id" % (flag, sample_id, number, path))
+    keep = flag == "--samples"
+    ids = np.array(sorted(iid for sid, iid in id_map.items() if (sid in listed) == keep), dtype=np.int64)
+    if ids.size == 0:
+        raise ValueError("%s: no sample is left to search among" % flag)
+    return ids
+
+
+def open_search(basename, keep, keep_parent_rows):
+    """The index's MornaSearch, or with `keep` (sample_filter's ids) a FilteredSearch over those samples."""
+    from .search import MornaSearch
+    searcher = MornaSearch(basename=basename)
+    return searcher if keep is None else searcher.subset(keep, keep_parent_rows)
+
+
 def main(argv=None, stdin=None, stdout=None, stderr=None):
     stdin, stdout, stderr = stdin or sys.stdin, stdout or sys.stdout, stderr or sys.stderr
     parser = build_parser()
@@ -143,7 +193,6 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
         return 0
 
     from . import parse
-    from .search import MornaSearch
     if args.convergence_backoff:
         stderr.write("convergence back-off is not supported (see README of the reference: non-functional)\n")
         return 2
@@ -157,13 +206,19 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
             return 2
     # a range search lists everything within the radius; an explicit -r caps each list
     limit = args.results if max_distance is not None and "results" in getattr(args, "given", ()) else None
+    try:
+        keep = sample_filter(args)
+    except ValueError as exc:
+        stderr.write(str(exc) + "\n")
+        return 2
     if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
-        return batch_search(args, stdout, stderr, max_distance, limit)
+        return batch_search(args, stdout, stderr, max_distance, limit, keep)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
         stdin = opened = open(args.pass1_sam)
-    searcher = MornaSearch(basename=args.basename)
+    # (a filter keeps the whole index's rows only for -q, whose sample may lie outside the subset)
+    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None)
     if args.query_id is not None:                               # morna.py:1358-1365
         if max_distance is not None:
             results = searcher.search_member_n(args.query_id, limit, include_distances=args.distances,
@@ -208,18 +263,18 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     return 0
 
 
-def batch_search(args, stdout, stderr, max_distance=None, limit=None):
+def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None):
     """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches.  With
-    `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given."""
+    `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given.  With
+    `keep` (sample_filter's ids), the search runs over those samples only."""
     from . import batch_query
-    from .search import MornaSearch
     named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
                                    ("--all-samples", args.all_samples), ("-q", args.query_id is not None),
                                    ("-rl", args.rawlist), ("-f", "format" in getattr(args, "given", ()))) if on]
     if len(named) > 1:
         stderr.write("%s cannot be combined with %s\n" % (named[0], ", ".join(named[1:])))
         return 2
-    searcher = MornaSearch(basename=args.basename)
+    searcher = open_search(args.basename, keep, keep_parent_rows=False)
     inverse = batch_query.inverse_map(searcher)
     meta = args.basename if args.metadata else None
     if max_distance is not None:

@@ -55,6 +55,21 @@ def concat_range_groups(parts, device):
     return torch.cat(offsets), torch.cat([p[3] for p in parts]), torch.cat([p[4] for p in parts])
 
 
+def _member_internal_id(internal_id_map, query_id, out=None):
+    """search -q: the internal id of sample `query_id`, with the two progress lines the reference prints (morna.py:733-745)."""
+    import sys
+    out = out or sys.stdout
+    out.write("querying by sample id " + str(query_id) + "\n")
+    try:
+        internal_id = internal_id_map[query_id]
+    except KeyError:
+        raise ValueError("Querying sample id " + str(query_id) + " is not possible because no internal "
+                         "id is mapped to that sample id. Likely no sample with that id was included "
+                         "in the index.")
+    out.write("this is internal id " + str(internal_id) + "\n")
+    return internal_id
+
+
 def make_phase_events():
     """Seven CUDA events for morna_knn_batched's phase boundaries: (events, ctypes array)."""
     import ctypes
@@ -687,16 +702,7 @@ class MornaSearch(object):
         """morna.py:733-787 with the stored row as the query (float32 values), run
         through the exact scan.  With ``max_distance``: every sample within it (range_search_nn), the first
         ``num_neighbors`` of them when that is not None."""
-        import sys
-        out = out or sys.stdout
-        out.write("querying by sample id " + str(query_id) + "\n")
-        try:
-            internal_id = self.internal_id_map[query_id]
-        except KeyError:
-            raise ValueError("Querying sample id " + str(query_id) + " is not possible because no internal "
-                             "id is mapped to that sample id. Likely no sample with that id was included "
-                             "in the index.")
-        out.write("this is internal id " + str(internal_id) + "\n")
+        internal_id = _member_internal_id(self.internal_id_map, query_id, out)
         if not (self.row_lo <= internal_id < self.row_hi):
             raise ValueError("internal id %d is not resident on this shard" % internal_id)
         self.query_sample = self.vectors[internal_id - self.row_lo, :self.dim].to(torch.float64).cpu().tolist()
@@ -707,6 +713,13 @@ class MornaSearch(object):
     def _metadata(self, internal_ids):
         """morna.py:666-676: keywords of every result's sample id from basename.meta.mor."""
         return files.read_meta(self.basename, [self.inverse_lookup(iid) for iid in internal_ids])
+
+    def subset(self, internal_ids, keep_parent_rows=True):
+        """A search over only the rows of these internal ids (any order, repeats allowed; resident on this object): a
+        FilteredSearch whose results carry this object's internal ids.  ``keep_parent_rows=False``: the result does not
+        hold this object's device rows, so dropping this object frees them; queries by internal id must then name rows of
+        the subset."""
+        return FilteredSearch(self, internal_ids, keep_parent_rows)
 
     # ------------------------------------------------------------------ range search
     RANGE_BATCH_QUERIES = 4096        # queries per morna_range_batched call (its candidate lists: 4096 x 4096 entries)
@@ -868,6 +881,179 @@ class MornaSearch(object):
                     ids[dst] = sub_ids
                     d[dst] = sub_d
             return offsets[lo:hi + 1], ids, d
+
+
+class FilteredSearch(object):
+    """The searches of a MornaSearch over a chosen subset of its rows (MornaSearch.subset), with results under the
+    parent's internal ids.
+
+    The subset is a compacted index of its own, ``inner``: a MornaSearch over the chosen rows gathered on the device in
+    ascending id order, with their norms copied; it builds its CSR form and tensor-core operand from them as any index
+    does.  Every route runs unchanged on ``inner``, which only ever sees its own row numbers; each entry point below maps
+    the ids back once, where the results leave.  The results are those of a brute-force search over the subset rows, bit
+    for bit: a row's distance is the same canonical FP64 sum wherever the row sits, and local row -> parent id is strictly
+    increasing, so the reference order (distance ascending, equal distances id descending) survives the map.
+
+    ``member_ids``: the subset's parent internal ids (numpy int64, ascending).  ``index_size``, ``sample_count``,
+    ``internal_id_map``, ``sample_frequencies`` and ``basename`` are the parent's, so query vectors and metadata are
+    built exactly as on the whole index."""
+
+    def __init__(self, parent, internal_ids, keep_parent_rows=True):
+        ids = np.unique(np.asarray(internal_ids, dtype=np.int64).reshape(-1))
+        if ids.size == 0:
+            raise ValueError("a filtered search needs at least one row")
+        if ids[0] < parent.row_lo or ids[-1] >= parent.row_hi:
+            raise ValueError("internal ids %d..%d are not all resident (rows %d..%d)"
+                             % (ids[0], ids[-1], parent.row_lo, parent.row_hi - 1))
+        dev = parent.device
+        self.lib, self.device, self.dim, self.basename = parent.lib, dev, parent.dim, parent.basename
+        self.sample_count, self.index_size = parent.sample_count, parent.index_size
+        self.sample_frequencies, self.internal_id_map = parent.sample_frequencies, parent.internal_id_map
+        self.row_lo, self.row_hi = parent.row_lo, parent.row_hi
+        self.member_ids = ids
+        self._ids32 = ids.astype(np.int32)
+        m = int(ids.size)
+        with torch.cuda.device(dev):
+            rows = torch.from_numpy(ids - parent.row_lo).to(dev)
+            self._ids_dev = torch.from_numpy(self._ids32).to(dev)
+            self._local = torch.full((parent.row_hi - parent.row_lo,), -1, dtype=torch.int64, device=dev)
+            self._local[rows] = torch.arange(m, device=dev)
+            inner = MornaSearch.__new__(MornaSearch)
+            inner.lib, inner.device, inner.basename = parent.lib, dev, parent.basename
+            inner.sample_count, inner.index_size, inner.dim, inner.ld = parent.sample_count, m, parent.dim, parent.ld
+            # (the parent's map: inner._metadata is only ever given parent ids)
+            inner.sample_frequencies, inner.internal_id_map = parent.sample_frequencies, parent.internal_id_map
+            inner.row_lo, inner.row_hi = 0, m
+            inner.vectors = parent.vectors.index_select(0, rows)
+            inner.pp = parent.pp.index_select(0, rows)
+            inner._build_csr()
+            inner.query, inner.query_sample = defaultdict(int), [0.0] * parent.dim
+        self.inner = inner
+        self._parent_rows = parent.vectors if keep_parent_rows else None
+
+    def _to_parent(self, ids):
+        """Result ids of `inner` (torch on the current stream, or numpy) -> parent internal ids (int32); -1 padding stays."""
+        top = self.member_ids.size - 1
+        if isinstance(ids, torch.Tensor):
+            return torch.where(ids >= 0, self._ids_dev[ids.long().clamp(0, top)], ids)
+        ids = np.asarray(ids)
+        return np.where(ids >= 0, self._ids32[np.clip(ids, 0, top)], ids).astype(np.int32)
+
+    def _nn(self, results, meta_db):
+        ids = self.member_ids[np.asarray(results[0], dtype=np.int64)].tolist()
+        out = (ids,) + tuple(results[1:])
+        if meta_db:
+            out += (self.inner._metadata(ids),)
+        return out
+
+    @property
+    def last_stats(self):
+        return self.inner.last_stats
+
+    @property
+    def last_range_route(self):
+        return self.inner.last_range_route
+
+    @property
+    def query_sample(self):
+        return self.inner.query_sample
+
+    @query_sample.setter
+    def query_sample(self, value):
+        self.inner.query_sample = value
+
+    def update_query(self, junction):
+        self.inner.update_query(junction)
+
+    def finalize_query(self):
+        self.inner.finalize_query()
+
+    def stored_queries(self, internal_ids):
+        """The stored rows of these parent internal ids as float64 device queries [len x dim], as ``search -q`` uses them.
+        Rows outside the subset are legal queries (they cannot return themselves) when the parent's rows were kept;
+        otherwise every id must be in the subset.  (The subset's rows are bit copies of the parent's: either source gives
+        the same queries.)"""
+        ids = torch.as_tensor(internal_ids).to(torch.int64).reshape(-1)
+        if ids.numel():
+            lo, hi = (int(v) for v in torch.aminmax(ids))
+            if lo < self.row_lo or hi >= self.row_hi:
+                raise ValueError("internal ids %d..%d are not all resident (rows %d..%d)" % (lo, hi, self.row_lo, self.row_hi - 1))
+        rows = ids.to(self.device) - self.row_lo
+        if self._parent_rows is not None:
+            return self._parent_rows[rows, :self.dim].to(torch.float64).contiguous()
+        local = self._local[rows]
+        if ids.numel() and bool((local < 0).any()):
+            raise ValueError("internal ids outside the subset are queries only with keep_parent_rows=True")
+        return self.inner.vectors[local, :self.dim].to(torch.float64).contiguous()
+
+    # ------------------------------------------------------------------ top-k (MornaSearch's entry points, ids mapped)
+    def exact_search_device(self, queries, k, stream=None, allow_single=True):
+        ids, d = self.inner.exact_search_device(queries, k, stream, allow_single)
+        with torch.cuda.stream(stream):
+            return self._to_parent(ids), d
+
+    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None):
+        ids, d = self.inner.batched_search_device(queries, k, stream, check_overflow, phase_events)
+        with torch.cuda.stream(stream):
+            return self._to_parent(ids), d
+
+    def single_search_device(self, query, k, stream=None):
+        ids, d = self.inner.single_search_device(query, k, stream)
+        with torch.cuda.stream(stream):
+            return self._to_parent(ids), d
+
+    def single_search_stream(self, queries, k):
+        ids, d = self.inner.single_search_stream(queries, k)
+        return self._to_parent(ids), d
+
+    def approx_search_device(self, queries, k):
+        ids, d = self.inner.approx_search_device(queries, k)
+        return self._to_parent(ids), d
+
+    def exact_search_batch(self, queries, k, tensor_cores=None):
+        ids, d = self.inner.exact_search_batch(queries, k, tensor_cores)
+        return self._to_parent(ids), d
+
+    def search_batches(self, batches, k, depth=2, side_job=False):
+        """MornaSearch.search_batches over the subset; a batch of internal ids becomes the stored rows of those ids
+        (stored_queries) on the device.  The distances are views of pinned buffers, as there."""
+        def queries():
+            for q in batches:
+                t = torch.from_numpy(np.ascontiguousarray(q)) if isinstance(q, np.ndarray) else q
+                yield self.stored_queries(t) if t.dim() == 1 and t.dtype in (torch.int32, torch.int64) else t
+        for ids, d in self.inner.search_batches(queries(), k, depth, side_job):
+            yield self._to_parent(ids), d
+
+    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False):
+        return self._nn(self.inner.exact_search_nn(num_neighbors, include_distances), meta_db)
+
+    def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False):
+        return self._nn(self.inner.search_nn(num_neighbors, search_k, include_distances), meta_db)
+
+    def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
+                        meta_db=False, out=None, max_distance=None):
+        """MornaSearch.search_member_n over the subset; the queried sample may lie outside it."""
+        internal_id = _member_internal_id(self.internal_id_map, query_id, out)
+        self.query_sample = self.stored_queries([internal_id])[0].cpu().tolist()
+        if max_distance is not None:
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors)
+        return self.exact_search_nn(num_neighbors, include_distances, meta_db)
+
+    # ------------------------------------------------------------------ range search
+    def range_search_device(self, queries, max_distance):
+        offsets, ids, d = self.inner.range_search_device(queries, max_distance)
+        return offsets, self._to_parent(ids), d
+
+    def range_search_groups(self, queries, max_distance, byte_cap=None):
+        for lo, hi, offsets, ids, d in self.inner.range_search_groups(queries, max_distance, byte_cap):
+            yield lo, hi, offsets, self._to_parent(ids), d
+
+    def range_search_batch(self, queries, max_distance):
+        offsets, ids, d = self.inner.range_search_batch(queries, max_distance)
+        return offsets, self._to_parent(ids), d
+
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None):
+        return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors), meta_db)
 
 
 class _PipeSlot(object):
