@@ -227,6 +227,18 @@ int morna_knn_exact(const float *vectors, const double *pp, int64_t n, int32_t d
                     int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
                     int32_t *out_ids, double *out_dist,
                     void *workspace, size_t workspace_bytes, void *stream);
+/* Per-query exclusion ("which OTHER samples resemble this one"): every *_excl entry point below takes the arguments of
+ * its plain form plus
+ *   row_group   [dev] int32[n]   label of each row of the call (row i = id id_base + i)
+ *   query_group [dev] int32[nq]  label of each query
+ * and treats row i as absent for query q iff query_group[q] >= 0 && row_group[i] == query_group[q].  Both NULL (the
+ * plain form) or both set.  Results equal the plain call's over the rows that are not excluded, bit for bit; a query
+ * left with fewer than k rows gets a shorter list padded with id -1 / +inf.  Here the FP64 distances of excluded pairs
+ * are set to +inf before the selection, and the selected +inf entries are turned into padding. */
+int morna_knn_exact_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                         int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
+                         int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
+                         const int32_t *row_group, const int32_t *query_group, void *stream);
 
 /* exact_search_nn for ONE query, HBM-bound, one kernel: every warp streams its share of the rows once
  * (4*n*ld bytes) and computes each row's exact distance with the FP64 sums of morna_knn_exact; the
@@ -273,6 +285,12 @@ int morna_knn_exact_sparse(const int64_t *row_off, const int32_t *cols, const fl
                            const double *pp, int64_t n, int32_t dim, int32_t id_base, const double *queries, int64_t nq,
                            int64_t q_ld, int32_t k, int32_t *out_ids, double *out_dist, void *workspace,
                            size_t workspace_bytes, void *stream);
+/* The same with a per-query exclusion (see morna_knn_exact_excl): excluded pairs are masked between the distance
+ * kernel and the selection. */
+int morna_knn_exact_sparse_excl(const int64_t *row_off, const int32_t *cols, const float *vals, const int32_t *plan,
+                                const double *pp, int64_t n, int32_t dim, int32_t id_base, const double *queries, int64_t nq,
+                                int64_t q_ld, int32_t k, int32_t *out_ids, double *out_dist, void *workspace,
+                                size_t workspace_bytes, const int32_t *row_group, const int32_t *query_group, void *stream);
 
 /* ------------------------------------------------------------------ batched search (tensor cores) */
 
@@ -330,6 +348,17 @@ int morna_knn_batched_score(const void *hs, int64_t ld_h, const float *rho_max, 
                             uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes,
                             void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound,
                             void *stream);
+/* The scoring half with a per-query exclusion (see morna_knn_exact_excl; row_group covers this call's n rows): an
+ * excluded entry is absent from every selection pass (pilot threshold, refinement between row blocks, final lists), so
+ * the final lists hold only allowed rows and morna_knn_batched_rerank then orders them as usual.  Excluded rows can
+ * still take first-pass list slots (the filter GEMM does not look at labels); a query whose list overflows is flagged
+ * as usual and must be answered by morna_knn_exact_excl.  kth_bound must be NULL (rows-sharded search has no
+ * exclusion). */
+int morna_knn_batched_score_excl(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
+                                 int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
+                                 uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes,
+                                 void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound,
+                                 const int32_t *row_group, const int32_t *query_group, void *stream);
 /* Rows-sharded search (one process per GPU, each holding a block of rows): give the scoring call a
  * kth_bound [dev] float[nq * k]; instead of the final candidate lists it then writes, per query, lower bounds of the
  * true cosines of its k best rows (score minus this rank's error bound; -inf pads a shorter list or an overflowed
@@ -380,6 +409,13 @@ int morna_range_batched(const float *vectors, const double *pp, const void *hs, 
                         int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
                         int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
                         void *workspace, size_t workspace_bytes, void *stream);
+/* The tensor-core route with a per-query exclusion (see morna_knn_exact_excl): excluded survivors of the filter are
+ * dropped before the d <= R check, so counts, lists and stats cover allowed rows only. */
+int morna_range_batched_excl(const float *vectors, const double *pp, const void *hs, int64_t ld_h, const float *rho_max,
+                             int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
+                             int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
+                             void *workspace, size_t workspace_bytes, const int32_t *row_group, const int32_t *query_group,
+                             void *stream);
 int morna_range_batched_emit(int64_t n, int64_t nq, int32_t dim, const int64_t *offsets, const uint8_t *overflow,
                              int32_t *out_ids, double *out_dist, const void *workspace, size_t workspace_bytes,
                              void *stream);
@@ -396,6 +432,16 @@ int morna_range_exact_fill(const float *vectors, const double *pp, int64_t n, in
                            const double *queries, int64_t nq, int64_t q_ld, double max_distance, const int64_t *offsets,
                            int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
                            void *stream);
+/* The FP64 route with a per-query exclusion (see morna_knn_exact_excl): each tile's distances are masked before both the
+ * count and the fill pass, so an excluded pair sits at +inf > R in both and counts and lists agree. */
+int morna_range_exact_count_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                                 const double *queries, int64_t nq, int64_t q_ld, double max_distance, int32_t *counts,
+                                 void *workspace, size_t workspace_bytes, const int32_t *row_group,
+                                 const int32_t *query_group, void *stream);
+int morna_range_exact_fill_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                                const double *queries, int64_t nq, int64_t q_ld, double max_distance, const int64_t *offsets,
+                                int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
+                                const int32_t *row_group, const int32_t *query_group, void *stream);
 
 /* Merge of per-rank range lists (the rows-sharded range search, after one all-gather of packed per-rank buffers).
  *   gathered     [dev] n_lists buffers back to back, 8-byte aligned; buffer g is cap doubles (distances) followed by cap

@@ -66,10 +66,14 @@ _SIGNATURES = {
     "morna_knn_exact_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32]),
     "morna_knn_exact": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64,
                                        _c_i32, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_knn_exact_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64,
+                                            _c_i32, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_sparse_max_nnz": (_c_i32, []),
     "morna_knn_exact_sparse_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32]),
     "morna_knn_exact_sparse": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_i64, _c_i32,
                                               _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_knn_exact_sparse_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_i64,
+                                                   _c_i32, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_knn_single_workspace_bytes": (_c_sz, [_c_i64]),
     "morna_knn_single_workspace_init": (ctypes.c_int, [_c_vp, _c_sz, _c_vp]),
     "morna_knn_single": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i32, _c_vp, _c_vp,
@@ -83,6 +87,9 @@ _SIGNATURES = {
                                          _c_vp, _c_i64, _c_i64, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp]),
     "morna_knn_batched_score": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_i64, _c_i32,
                                                _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, ctypes.POINTER(RerankJob), _c_vp, _c_vp]),
+    "morna_knn_batched_score_excl": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_i64, _c_i32,
+                                                    _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, ctypes.POINTER(RerankJob), _c_vp, _c_vp, _c_vp,
+                                                    _c_vp]),
     "morna_knn_batched_approx": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i32, _c_vp, _c_i64, _c_i64, _c_i32,
                                                 _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_union_kth_bound": (ctypes.c_int, [_c_vp, _c_i32, _c_i64, _c_i32, _c_vp, _c_vp]),
@@ -92,12 +99,18 @@ _SIGNATURES = {
     "morna_range_batched_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32]),
     "morna_range_batched": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64,
                                            _c_i64, ctypes.c_double, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_batched_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64,
+                                                _c_i64, ctypes.c_double, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_range_batched_emit": (ctypes.c_int, [_c_i64, _c_i64, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_range_exact_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i64]),
     "morna_range_exact_count": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_i64, _c_i64, ctypes.c_double,
                                                _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_exact_count_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_i64, _c_i64, ctypes.c_double,
+                                                    _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_range_exact_fill": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, ctypes.c_double,
                                               _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_range_exact_fill_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64,
+                                                   ctypes.c_double, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_merge_sorted_csr": (ctypes.c_int, [_c_vp, _c_i32, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp]),
     "morna_debug_tensor_scores": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_vp,
                                                  _c_i64, _c_vp, _c_vp, _c_sz, _c_vp]),

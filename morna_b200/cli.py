@@ -16,6 +16,8 @@ import argparse
 import math
 import sys
 
+import numpy as np
+
 _help_intro = "morna (B200-native hot path): index and exactly search junction feature vectors"
 
 
@@ -114,6 +116,13 @@ def build_parser():
                                help="search only among these indexed samples: a file with one sample id per line")
     search_parser.add_argument("--exclude-samples", metavar="<file>", type=str, required=False, default=None,
                                help="search among every indexed sample except these: a file with one sample id per line")
+    search_parser.add_argument("--exclude-self", action="store_const", const=True, default=False,
+                               help="leave each query's own sample out of its results (-q, --all-samples, "
+                                    "--query-intropolis -e): the most similar OTHER samples")
+    search_parser.add_argument("--exclude-group", metavar="<file>", type=str, required=False, default=None,
+                               help="a file of 'sample_id<TAB>group' lines (a group is any string, e.g. a study "
+                                    "accession): leave each query's own sample and every sample of its group out of its "
+                                    "results (-q, --all-samples, --query-intropolis -e)")
     search_parser.add_argument("--max-distance", metavar="<float>", type=float, required=False, default=None,
                                help="return every sample within this angular distance of the query (exact; -r N, if "
                                     "given, keeps the first N per query)")
@@ -171,10 +180,85 @@ def sample_filter(args):
     return ids
 
 
-def open_search(basename, keep, keep_parent_rows):
-    """The index's MornaSearch, or with `keep` (sample_filter's ids) a FilteredSearch over those samples."""
+class Exclusion(object):
+    """--exclude-self / --exclude-group: every indexed sample carries a label, and a query leaves out every sample whose
+    label equals its own.  Listed groups are numbered densely (0 .. n_groups-1, in order of first appearance); a sample
+    not listed is a group of its own, labelled n_groups + its internal id.  So a query's own sample is always left out."""
+
+    def __init__(self, group_of, id_map, index_size):
+        self.group_of, self.id_map = group_of, id_map           # sample id -> group number; sample id -> internal id
+        n_groups = len(set(group_of.values()))
+        self.row_labels = np.arange(n_groups, n_groups + index_size, dtype=np.int64)
+        for sample_id, g in group_of.items():
+            iid = id_map.get(sample_id)
+            if iid is not None:
+                self.row_labels[iid] = g
+        if self.row_labels.size and self.row_labels.max() > np.iinfo(np.int32).max:
+            raise ValueError("too many exclusion groups for int32 labels")
+        self.row_labels = self.row_labels.astype(np.int32)
+
+    def labels_of_samples(self, sample_ids):
+        """Labels of queries named by sample id (--query-intropolis): the group of a listed or indexed sample, else -1
+        (nothing left out)."""
+        out = np.full(len(sample_ids), -1, dtype=np.int32)
+        for j, sid in enumerate(np.asarray(sample_ids).tolist()):
+            if sid in self.group_of:
+                out[j] = self.group_of[sid]
+            elif sid in self.id_map:
+                out[j] = self.row_labels[self.id_map[sid]]
+        return out
+
+
+def exclusion(args):
+    """--exclude-self / --exclude-group: an Exclusion, or None without either flag.  Raises ValueError with the message
+    for the user when the flags, the query mode or the file are not usable (before any GPU work)."""
+    self_only, path = getattr(args, "exclude_self", False), getattr(args, "exclude_group", None)
+    if not self_only and path is None:
+        return None
+    flag = "--exclude-self" if self_only else "--exclude-group"
+    if self_only and path is not None:
+        raise ValueError("--exclude-self cannot be combined with --exclude-group")
+    if args.query_id is None and not args.all_samples and args.query_intropolis is None:
+        raise ValueError("%s needs queries that are samples (-q, --all-samples or --query-intropolis): a query read "
+                         "from stdin has no sample id" % flag)
+    if args.query_intropolis is not None and not args.exact:
+        raise ValueError("%s with --query-intropolis needs -e: the approximate mode has no exclusion" % flag)
+    group_of = {}
+    if path is not None:
+        try:
+            with open(path) as fh:
+                lines = fh.read().splitlines()
+        except (OSError, UnicodeDecodeError) as exc:
+            raise ValueError("%s: cannot read %s: %s" % (flag, path, exc))
+        numbers, first_line = {}, {}
+        for number, line in enumerate(lines, 1):
+            text = line.strip()
+            if not text:
+                continue
+            fields = text.split("\t")
+            if len(fields) != 2 or not fields[1].strip():
+                raise ValueError("%s: line %d of %s is not 'sample_id<TAB>group': %r" % (flag, number, path, text))
+            try:
+                sample_id = int(fields[0].strip())
+            except ValueError:
+                raise ValueError("%s: line %d of %s does not start with an integer sample id: %r" % (flag, number, path, text))
+            g = numbers.setdefault(fields[1].strip(), len(numbers))
+            if group_of.setdefault(sample_id, g) != g:
+                raise ValueError("%s: sample id %d is listed with two different groups (lines %d and %d of %s)"
+                                 % (flag, sample_id, first_line[sample_id], number, path))
+            first_line.setdefault(sample_id, number)
+    from . import files
+    index_size = files.read_stats(args.basename)[1]
+    return Exclusion(group_of, files.read_map(args.basename), index_size)
+
+
+def open_search(basename, keep, keep_parent_rows, excl=None):
+    """The index's MornaSearch, or with `keep` (sample_filter's ids) a FilteredSearch over those samples; with `excl`
+    (an Exclusion) every row carries its label."""
     from .search import MornaSearch
     searcher = MornaSearch(basename=basename)
+    if excl is not None:
+        searcher.set_row_groups(excl.row_labels)
     return searcher if keep is None else searcher.subset(keep, keep_parent_rows)
 
 
@@ -208,24 +292,27 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     limit = args.results if max_distance is not None and "results" in getattr(args, "given", ()) else None
     try:
         keep = sample_filter(args)
+        excl = exclusion(args) if args.subparser_name == "search" else None
     except ValueError as exc:
         stderr.write(str(exc) + "\n")
         return 2
     if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
-        return batch_search(args, stdout, stderr, max_distance, limit, keep)
+        return batch_search(args, stdout, stderr, max_distance, limit, keep, excl)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
         stdin = opened = open(args.pass1_sam)
     # (a filter keeps the whole index's rows only for -q, whose sample may lie outside the subset)
-    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None)
+    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None, excl=excl)
     if args.query_id is not None:                               # morna.py:1358-1365
         if max_distance is not None:
             results = searcher.search_member_n(args.query_id, limit, include_distances=args.distances,
-                                               meta_db=args.metadata, out=stdout, max_distance=max_distance)
+                                               meta_db=args.metadata, out=stdout, max_distance=max_distance,
+                                               exclude=excl is not None)
         else:
             results = searcher.search_member_n(args.query_id, args.results, args.search_k,
-                                               include_distances=args.distances, meta_db=args.metadata, out=stdout)
+                                               include_distances=args.distances, meta_db=args.metadata, out=stdout,
+                                               exclude=excl is not None)
         results_output(results, stdout)
         return 0
     if args.format == "sam":                                    # :1367-1373
@@ -263,10 +350,11 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     return 0
 
 
-def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None):
+def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None, excl=None):
     """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches.  With
     `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given.  With
-    `keep` (sample_filter's ids), the search runs over those samples only."""
+    `keep` (sample_filter's ids), the search runs over those samples only.  With `excl` (an Exclusion), each query
+    leaves out the samples of its group."""
     from . import batch_query
     named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
                                    ("--all-samples", args.all_samples), ("-q", args.query_id is not None),
@@ -274,21 +362,26 @@ def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None)
     if len(named) > 1:
         stderr.write("%s cannot be combined with %s\n" % (named[0], ", ".join(named[1:])))
         return 2
-    searcher = open_search(args.basename, keep, keep_parent_rows=False)
+    # (with an exclusion, --all-samples over a subset takes its labels from the whole index's rows)
+    searcher = open_search(args.basename, keep, keep_parent_rows=False, excl=excl)
     inverse = batch_query.inverse_map(searcher)
     meta = args.basename if args.metadata else None
+    exclude = excl is not None
+    query_labels = excl.labels_of_samples if exclude else None
     if max_distance is not None:
         if args.all_samples:
-            results = batch_query.search_all_samples_range(searcher, max_distance, inverse)
+            results = batch_query.search_all_samples_range(searcher, max_distance, inverse, exclude=exclude)
         else:
-            results = batch_query.search_query_file_range(searcher, args.query_intropolis, max_distance)
+            results = batch_query.search_query_file_range(searcher, args.query_intropolis, max_distance,
+                                                          query_labels=query_labels)
         for sample_ids, offsets, ids, dists in results:
             batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse, offsets=offsets, limit=limit)
         return 0
     if args.all_samples:                       # the stored rows as queries: exact, as -q is
-        results = batch_query.search_all_samples(searcher, args.results, inverse)
+        results = batch_query.search_all_samples(searcher, args.results, inverse, exclude=exclude)
     else:
-        results = batch_query.search_query_file(searcher, args.query_intropolis, args.results, exact=args.exact)
+        results = batch_query.search_query_file(searcher, args.query_intropolis, args.results, exact=args.exact,
+                                                query_labels=query_labels)
     for sample_ids, ids, dists in results:
         batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse)
     return 0

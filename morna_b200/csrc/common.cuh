@@ -87,4 +87,12 @@ __device__ __forceinline__ bool before(double da, int ia, double db, int ib) {
     return da < db || (da == db && ia > ib);
 }
 
+// Per-query exclusion on the FP64 routes (search_exact.cu).  Row i is excluded for query q iff
+// query_group[q] >= 0 && row_group[i] == query_group[q]; the mask writes +inf into the distance scratch
+// [nq x dist_ld] of every excluded pair, so a selection after it never prefers an excluded row to a real
+// distance (<= 2).  The padding pass turns the selected +inf entries into id -1 (the padding of short lists).
+int launch_mask_excluded(double *dist, int64_t n, int64_t dist_ld, int64_t nq, const int32_t *row_group,
+                         const int32_t *query_group, cudaStream_t s);
+int launch_pad_masked(int32_t *ids, const double *dist, int64_t total, cudaStream_t s);
+
 }  // namespace morna

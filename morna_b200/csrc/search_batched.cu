@@ -1007,6 +1007,9 @@ struct KthParams {
     int32_t *fin_id; int32_t *fin_cnt;
     uint8_t *overflow; int32_t *stats;
     float *kth_bound;                             // modes 3 / 4: per-query lower bound of the k-th best true cosine
+    // modes 0-2, per-query exclusion (nullptr = off): the row behind entry idx (pilot: row n_begin + idx; lists:
+    // cand_id[idx] - id_base) is absent for query q iff query_group[q] >= 0 && row_group[row] == query_group[q]
+    const int32_t *row_group; const int32_t *query_group;
 };
 
 // key of the kk-th largest of the keys one warp holds in registers (kItems per lane; 0 = padding)
@@ -1051,6 +1054,10 @@ constexpr int kKwSmem = kKwWarps * 32 * kKwSlots * (int)(sizeof(uint32_t) + size
 //   kMode 3 (bound) : input = candidate list      -> kth_bound[q] = (k-th largest score) - eps, nothing emitted.  Rows-sharded
 //                     search: the maximum of this bound over the ranks is a lower bound of the GLOBAL k-th best cosine
 //   kMode 4 (emit)  : input = candidate list      -> final candidate list = everything >= kth_bound[q] - eps
+// With an exclusion (modes 0-2) an excluded entry is absent everywhere: it never enters the lane lists, the bisection
+// does not count it and nothing emits it; kk is the number of ALLOWED entries when fewer than k are allowed, and then
+// the threshold stays -inf and every allowed entry is emitted.  Labels are looked up only for entries that pass the
+// pivot (or, without a usable pivot, in the fallback passes).
 template <int kMode>
 __global__ void __launch_bounds__(kKwWarps * 32)
 kth_warp_kernel(KthParams p, int nq) {
@@ -1078,9 +1085,15 @@ kth_warp_kernel(KthParams p, int nq) {
         }
     }
     const float *src = kPilot ? p.pilot + (int64_t)q * p.pilot_ld : p.cand_score + (int64_t)q * p.cap;
-    const int kk = min(p.k, count);
+    int kk = min(p.k, count);
     const int out_cap = (kPilot || kRefine) ? p.cap : p.fcap;
     const float eps = p.eps[q];
+    const int32_t qgroup = (!kBound && !kEmit && p.row_group) ? p.query_group[q] : -1;
+    const bool excl = qgroup >= 0;                              // warp-uniform
+    auto allowed = [&](int idx) -> bool {
+        const int64_t row = kPilot ? (int64_t)p.n_begin + idx : (int64_t)p.cand_id[(int64_t)q * p.cap + idx] - p.id_base;
+        return p.row_group[row] != qgroup;
+    };
 
     uint32_t best = 0;          // key of the kk-th largest entry
     bool lists_ok = false;      // lane lists hold every entry >= pivot
@@ -1143,7 +1156,7 @@ kth_warp_kernel(KthParams p, int nq) {
 #pragma unroll
                         for (int i = 0; i < 2; ++i) s2[i] = (e & 8) ? s4[2 * i + 1] : s4[2 * i];
                         const uint32_t key = float_key((e & 16) ? s2[1] : s2[0]);
-                        if (key >= pivot) {
+                        if (key >= pivot && (!excl || allowed(idx))) {
                             if (mine < kKwSlots) { lkey[mine * 32 + lane] = key; lidx[mine * 32 + lane] = (uint16_t)idx; }
                             else overflowed = true;
                             ++mine;
@@ -1162,7 +1175,7 @@ kth_warp_kernel(KthParams p, int nq) {
                     if (vv[t] >= pivot_f) {
                         const int idx = 4 * g + t;
                         const uint32_t key = float_key(vv[t]);
-                        if (idx < count && key >= pivot) {
+                        if (idx < count && key >= pivot && (!excl || allowed(idx))) {
                             if (mine < kKwSlots) { lkey[mine * 32 + lane] = key; lidx[mine * 32 + lane] = (uint16_t)idx; }
                             else overflowed = true;
                             ++mine;
@@ -1172,17 +1185,24 @@ kth_warp_kernel(KthParams p, int nq) {
             }
         }
         const int m = __reduce_add_sync(kFull, mine);
-        lists_ok = !__any_sync(kFull, overflowed) && m >= kk;
+        const bool any_over = __any_sync(kFull, overflowed);
+        if (excl && pivot == 0u && !any_over) kk = min(kk, m);      // the lists hold every allowed entry
+        lists_ok = !any_over && m >= kk;
         if (lists_ok) {
             uint32_t sk[kKwSlots];
 #pragma unroll
             for (int j = 0; j < kKwSlots; ++j) sk[j] = j < mine ? lkey[j * 32 + lane] : 0u;
             best = warp_kth_largest<kKwSlots>(sk, kk);
-        } else {                                     // streaming bisection over every entry
-            for (int bit = 31; bit >= 0; --bit) {
+        } else {                                     // streaming bisection over every (allowed) entry
+            if (excl) {
+                int ca = 0;
+                for (int i = lane; i < count; i += 32) ca += allowed(i);
+                kk = min(kk, __reduce_add_sync(kFull, ca));
+            }
+            for (int bit = 31; bit >= 0 && kk > 0; --bit) {
                 const uint32_t trial = best | (1u << bit);
                 int c = 0;
-                for (int i = lane; i < count; i += 32) c += float_key(src[i]) >= trial;
+                for (int i = lane; i < count; i += 32) c += float_key(src[i]) >= trial && (!excl || allowed(i));
                 c = __reduce_add_sync(kFull, c);
                 if (c >= kk) best = trial;
             }
@@ -1285,7 +1305,9 @@ kth_warp_kernel(KthParams p, int nq) {
         for (int i0 = 0; i0 < count; i0 += 32) {
             const int i = i0 + lane;
             const float v = i < count ? src[i] : 0.f;
-            emit(i < count && v >= cut, v, i);
+            bool keep = i < count && v >= cut;
+            if (excl && keep) keep = allowed(i);
+            emit(keep, v, i);
         }
     }
     if (lane == 0) {
@@ -1497,9 +1519,10 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
                       int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
                       uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes,
                       void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound, int final_mode,
-                      void *stream) {
+                      const int32_t *row_group, const int32_t *query_group, void *stream) {
     if (!hs || !rho_max || !queries || !overflow || !stats || n <= 0 || n > kBatchedMaxRows || nq <= 0 || dim <= 0 ||
-        q_ld < dim || k <= 0 || k > kFinCap / 2 || ld_h != morna_tensor_operand_ld(dim))
+        q_ld < dim || k <= 0 || k > kFinCap / 2 || ld_h != morna_tensor_operand_ld(dim) || !row_group != !query_group ||
+        (row_group && final_mode == 1))
         return MORNA_ERR_INVALID_ARGUMENT;
     BatchWs w = batch_ws_layout(n, nq, ld_h);
     if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
@@ -1566,7 +1589,7 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
     kp.k = k; kp.n0 = (int32_t)w.n0; kp.n_begin = 0; kp.id_base = id_base; kp.cap = kCandCap; kp.fcap = kFinCap;
     kp.pilot = pilot; kp.pilot_ld = w.pilot_ld; kp.eps = eps; kp.thr = thr; kp.cand_score = cand_score;
     kp.cand_id = cand_id; kp.cand_cnt = cand_cnt; kp.fin_id = fin_id; kp.fin_cnt = fin_cnt; kp.overflow = overflow;
-    kp.stats = stats;
+    kp.stats = stats; kp.row_group = row_group; kp.query_group = query_group;
     if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<1>, kKwSmem)) != MORNA_OK) return rc;
     if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<0>, kKwSmem)) != MORNA_OK) return rc;
     if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<2>, kKwSmem)) != MORNA_OK) return rc;
@@ -1624,7 +1647,16 @@ extern "C" int morna_knn_batched_score(const void *hs, int64_t ld_h, const float
                                        void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound,
                                        void *stream) {
     return score_impl(hs, ld_h, rho_max, n, dim, id_base, queries, nq, q_ld, k, overflow, stats, workspace, workspace_bytes,
-                      phase_events, side_job, kth_bound, kth_bound ? 1 : 0, stream);
+                      phase_events, side_job, kth_bound, kth_bound ? 1 : 0, nullptr, nullptr, stream);
+}
+
+extern "C" int morna_knn_batched_score_excl(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
+                                            int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
+                                            uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes,
+                                            void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound,
+                                            const int32_t *row_group, const int32_t *query_group, void *stream) {
+    return score_impl(hs, ld_h, rho_max, n, dim, id_base, queries, nq, q_ld, k, overflow, stats, workspace, workspace_bytes,
+                      phase_events, side_job, kth_bound, kth_bound ? 1 : 0, row_group, query_group, stream);
 }
 
 namespace morna {
@@ -1701,7 +1733,7 @@ extern "C" int morna_knn_batched_approx(const void *hs, int64_t ld_h, const floa
                                         void *workspace, size_t workspace_bytes, void *stream) {
     if (!out_ids || !out_dist) return MORNA_ERR_INVALID_ARGUMENT;
     int rc = score_impl(hs, ld_h, rho_max, n, dim, id_base, queries, nq, q_ld, k, overflow, stats, workspace, workspace_bytes,
-                        nullptr, nullptr, nullptr, 2, stream);
+                        nullptr, nullptr, nullptr, 2, nullptr, nullptr, stream);
     if (rc != MORNA_OK) return rc;
     BatchWs w = batch_ws_layout(n, nq, ld_h);
     unsigned char *ws = (unsigned char *)workspace;
@@ -2008,6 +2040,7 @@ struct RangeCheckParams {
     const int32_t *cand_id; const int32_t *cand_cnt; const uint8_t *overflow;
     double R;
     int32_t *match_id; double *match_dist; int32_t *match_cnt;
+    const int32_t *row_group; const int32_t *query_group;      // per-query exclusion (nullptr = off), as in KthParams
 };
 
 // A work item is (32-candidate window, query) of a first-pass list, one warp each: the window's rows go through
@@ -2030,6 +2063,7 @@ range_check_kernel(const RangeCheckParams p) {
         const int32_t *ids = p.cand_id + (int64_t)q * kCandCap + i0;
         const double *qsrc = p.queries + (int64_t)q * p.q_ld;
         const double qqv = p.qq[q];
+        const int32_t qgroup = p.row_group ? p.query_group[q] : -1;
         for (int g = 0; g < m; g += kRows) {
             const int cnt = min(kRows, m - g);
             const float4 *src[kRows];
@@ -2052,7 +2086,7 @@ range_check_kernel(const RangeCheckParams p) {
             }
             double d = 0.0;
             if (lane < cnt) d = angular_from_sums(p.pp[my_id - p.id_base], qqv, mine);
-            const bool keep = lane < cnt && d <= p.R;
+            const bool keep = lane < cnt && !(qgroup >= 0 && p.row_group[my_id - p.id_base] == qgroup) && d <= p.R;
             const unsigned mask = __ballot_sync(kFull, keep);
             if (mask) {
                 int at = 0;
@@ -2131,6 +2165,16 @@ extern "C" int morna_range_batched(const float *vectors, const double *pp, const
                                    int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
                                    int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
                                    void *workspace, size_t workspace_bytes, void *stream) {
+    return morna_range_batched_excl(vectors, pp, hs, ld_h, rho_max, n, dim, ld, id_base, queries, nq, q_ld, max_distance, counts,
+                                    overflow, stats, workspace, workspace_bytes, nullptr, nullptr, stream);
+}
+
+extern "C" int morna_range_batched_excl(const float *vectors, const double *pp, const void *hs, int64_t ld_h, const float *rho_max,
+                                        int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
+                                        int64_t q_ld, double max_distance, int32_t *counts, uint8_t *overflow, int64_t *stats,
+                                        void *workspace, size_t workspace_bytes, const int32_t *row_group,
+                                        const int32_t *query_group, void *stream) {
+    if (!row_group != !query_group) return MORNA_ERR_INVALID_ARGUMENT;
     if (!vectors || !pp || !hs || !rho_max || !queries || !counts || !overflow || !stats || n <= 0 || n > kBatchedMaxRows ||
         nq <= 0 || nq > kRangeMaxQueries || dim <= 0 || ld < dim || (ld & 3) || q_ld < dim ||
         ld_h != morna_tensor_operand_ld(dim) || !(max_distance >= 0.0) || isinf(max_distance))
@@ -2181,7 +2225,7 @@ extern "C" int morna_range_batched(const float *vectors, const double *pp, const
     cp.vectors = vectors; cp.pp = pp; cp.ld = ld; cp.dim = dim; cp.id_base = id_base; cp.nq = (int32_t)nq;
     cp.queries = queries; cp.q_ld = q_ld; cp.qq = qq; cp.cand_id = gp.cand_id; cp.cand_cnt = cand_cnt; cp.overflow = overflow;
     cp.R = max_distance; cp.match_id = (int32_t *)(ws + w.match_id); cp.match_dist = (double *)(ws + w.match_dist);
-    cp.match_cnt = match_cnt;
+    cp.match_cnt = match_cnt; cp.row_group = row_group; cp.query_group = query_group;
     int per_sm = 0;
     MORNA_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, range_check_kernel, kRangeWarps * 32, 0));
     if (per_sm < 1) per_sm = 1;

@@ -240,6 +240,44 @@ select_topk_kernel(const double *__restrict__ keys, const int32_t *__restrict__ 
 
 static int sm_count_cached() { return sm_count_current(); }
 
+// grid (row blocks, query): +inf for every row of the query's group (nothing for a query labelled < 0)
+__global__ void __launch_bounds__(256)
+mask_excluded_kernel(double *__restrict__ dist, int64_t n, int64_t dist_ld, const int32_t *__restrict__ row_group,
+                     const int32_t *__restrict__ query_group) {
+    const int64_t q = blockIdx.y;
+    const int32_t g = query_group[q];
+    if (g < 0) return;
+    double *dq = dist + q * dist_ld;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256)
+        if (row_group[i] == g) dq[i] = INFINITY;
+}
+
+__global__ void pad_masked_kernel(int32_t *__restrict__ ids, const double *__restrict__ dist, int64_t total) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i < total && isinf(dist[i])) ids[i] = -1;
+}
+
+int launch_mask_excluded(double *dist, int64_t n, int64_t dist_ld, int64_t nq, const int32_t *row_group,
+                         const int32_t *query_group, cudaStream_t s) {
+    if (n <= 0 || nq <= 0) return MORNA_OK;
+    for (int64_t q0 = 0; q0 < nq; q0 += 65535) {
+        const int64_t cnt = std::min<int64_t>(nq - q0, 65535);
+        int64_t bx = (n + 255) / 256, cap = ((int64_t)sm_count_cached() * 16 + cnt - 1) / cnt;
+        if (bx > cap) bx = cap;
+        mask_excluded_kernel<<<dim3((unsigned)bx, (unsigned)cnt), 256, 0, s>>>(dist + q0 * dist_ld, n, dist_ld, row_group,
+                                                                              query_group + q0);
+        MORNA_LAUNCH_CHECK();
+    }
+    return MORNA_OK;
+}
+
+int launch_pad_masked(int32_t *ids, const double *dist, int64_t total, cudaStream_t s) {
+    if (total <= 0) return MORNA_OK;
+    pad_masked_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(ids, dist, total);
+    MORNA_LAUNCH_CHECK();
+    return MORNA_OK;
+}
+
 static size_t select_level_entries(int64_t n, int32_t k) {
     int64_t chunks = (n + kSelChunk - 1) / kSelChunk;
     return chunks > 1 ? (size_t)chunks * k : 0;
@@ -536,9 +574,17 @@ extern "C" int morna_knn_exact(const float *vectors, const double *pp, int64_t n
                                int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
                                int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
                                void *stream) {
+    return morna_knn_exact_excl(vectors, pp, n, dim, ld, id_base, queries, nq, q_ld, k, out_ids, out_dist, workspace,
+                                workspace_bytes, nullptr, nullptr, stream);
+}
+
+extern "C" int morna_knn_exact_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                                    int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
+                                    int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
+                                    const int32_t *row_group, const int32_t *query_group, void *stream) {
     if (!workspace || workspace_bytes < morna_knn_exact_workspace_bytes(n, nq, k))
         return MORNA_ERR_WORKSPACE_TOO_SMALL;
-    if (n <= 0 || nq < 0 || k <= 0 || k > kSelMaxK) return MORNA_ERR_INVALID_ARGUMENT;
+    if (n <= 0 || nq < 0 || k <= 0 || k > kSelMaxK || !row_group != !query_group) return MORNA_ERR_INVALID_ARGUMENT;
     int64_t tile = knn_query_tile(n, nq);
     double *dist = (double *)workspace;
     size_t dist_bytes = align_up((size_t)tile * (size_t)n * sizeof(double), 256);
@@ -548,9 +594,13 @@ extern "C" int morna_knn_exact(const float *vectors, const double *pp, int64_t n
         int64_t cnt = std::min<int64_t>(tile, nq - q0);
         int rc = morna_angular_distances(vectors, pp, n, dim, ld, queries + q0 * q_ld, cnt, q_ld, dist, n, stream);
         if (rc != MORNA_OK) return rc;
+        if (row_group && (rc = launch_mask_excluded(dist, n, n, cnt, row_group, query_group + q0, (cudaStream_t)stream)) != MORNA_OK)
+            return rc;
         rc = morna_select_topk(dist, nullptr, n, n, id_base, cnt, k, out_ids + q0 * k, out_dist + q0 * k,
                                sel_ws, sel_bytes, stream);
         if (rc != MORNA_OK) return rc;
+        if (row_group && (rc = launch_pad_masked(out_ids + q0 * k, out_dist + q0 * k, cnt * k, (cudaStream_t)stream)) != MORNA_OK)
+            return rc;
     }
     return MORNA_OK;
 }

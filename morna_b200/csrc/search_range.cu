@@ -159,7 +159,17 @@ extern "C" size_t morna_range_exact_workspace_bytes(int64_t n, int64_t nq, int64
 extern "C" int morna_range_exact_count(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
                                        const double *queries, int64_t nq, int64_t q_ld, double max_distance, int32_t *counts,
                                        void *workspace, size_t workspace_bytes, void *stream) {
-    if (!range_args_ok(vectors, pp, n, dim, ld, queries, nq, q_ld, max_distance) || !counts) return MORNA_ERR_INVALID_ARGUMENT;
+    return morna_range_exact_count_excl(vectors, pp, n, dim, ld, queries, nq, q_ld, max_distance, counts, workspace, workspace_bytes,
+                                        nullptr, nullptr, stream);
+}
+
+// The count and fill passes run the same mask on the same distances, so counts and lists agree.
+extern "C" int morna_range_exact_count_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                                            const double *queries, int64_t nq, int64_t q_ld, double max_distance, int32_t *counts,
+                                            void *workspace, size_t workspace_bytes, const int32_t *row_group,
+                                            const int32_t *query_group, void *stream) {
+    if (!range_args_ok(vectors, pp, n, dim, ld, queries, nq, q_ld, max_distance) || !counts || !row_group != !query_group)
+        return MORNA_ERR_INVALID_ARGUMENT;
     if (nq == 0) return MORNA_OK;
     const RangeExactWs w = range_exact_layout(n, nq, 0);
     if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
@@ -169,6 +179,7 @@ extern "C" int morna_range_exact_count(const float *vectors, const double *pp, i
         const int64_t cnt = std::min<int64_t>(w.tile, nq - q0);
         int rc = morna_angular_distances(vectors, pp, n, dim, ld, queries + q0 * q_ld, cnt, q_ld, dist, n, stream);
         if (rc != MORNA_OK) return rc;
+        if (row_group && (rc = launch_mask_excluded(dist, n, n, cnt, row_group, query_group + q0, s)) != MORNA_OK) return rc;
         range_count_kernel<<<(unsigned)cnt, kRangeCountThreads, 0, s>>>(dist, n, max_distance, counts + q0);
         MORNA_LAUNCH_CHECK();
     }
@@ -179,8 +190,16 @@ extern "C" int morna_range_exact_fill(const float *vectors, const double *pp, in
                                       const double *queries, int64_t nq, int64_t q_ld, double max_distance, const int64_t *offsets,
                                       int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
                                       void *stream) {
+    return morna_range_exact_fill_excl(vectors, pp, n, dim, ld, id_base, queries, nq, q_ld, max_distance, offsets, total, out_ids,
+                                       out_dist, workspace, workspace_bytes, nullptr, nullptr, stream);
+}
+
+extern "C" int morna_range_exact_fill_excl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                                           const double *queries, int64_t nq, int64_t q_ld, double max_distance, const int64_t *offsets,
+                                           int64_t total, int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes,
+                                           const int32_t *row_group, const int32_t *query_group, void *stream) {
     if (!range_args_ok(vectors, pp, n, dim, ld, queries, nq, q_ld, max_distance) || !offsets || !out_ids || !out_dist ||
-        total < 0 || total > INT32_MAX || nq > INT32_MAX)
+        total < 0 || total > INT32_MAX || nq > INT32_MAX || !row_group != !query_group)
         return MORNA_ERR_INVALID_ARGUMENT;
     if (nq == 0 || total == 0) return MORNA_OK;
     const RangeExactWs w = range_exact_layout(n, nq, total);
@@ -192,6 +211,7 @@ extern "C" int morna_range_exact_fill(const float *vectors, const double *pp, in
         const int64_t cnt = std::min<int64_t>(w.tile, nq - q0);
         int rc = morna_angular_distances(vectors, pp, n, dim, ld, queries + q0 * q_ld, cnt, q_ld, dist, n, stream);
         if (rc != MORNA_OK) return rc;
+        if (row_group && (rc = launch_mask_excluded(dist, n, n, cnt, row_group, query_group + q0, s)) != MORNA_OK) return rc;
         range_compact_kernel<<<(unsigned)cnt, kRangeCompactThreads, 0, s>>>(dist, n, max_distance, id_base, offsets + q0,
                                                                            out_ids, out_dist);
         MORNA_LAUNCH_CHECK();

@@ -343,7 +343,17 @@ extern "C" int morna_knn_exact_sparse(const int64_t *row_off, const int32_t *col
                                       const double *pp, int64_t n, int32_t dim, int32_t id_base, const double *queries, int64_t nq,
                                       int64_t q_ld, int32_t k, int32_t *out_ids, double *out_dist, void *workspace,
                                       size_t workspace_bytes, void *stream) {
-    if (!row_off || !cols || !vals || !plan || !pp || !queries || !out_ids || !out_dist || n <= 0 || nq < 0 || dim <= 0 || q_ld < dim || k <= 0)
+    return morna_knn_exact_sparse_excl(row_off, cols, vals, plan, pp, n, dim, id_base, queries, nq, q_ld, k, out_ids, out_dist,
+                                       workspace, workspace_bytes, nullptr, nullptr, stream);
+}
+
+extern "C" int morna_knn_exact_sparse_excl(const int64_t *row_off, const int32_t *cols, const float *vals, const int32_t *plan,
+                                           const double *pp, int64_t n, int32_t dim, int32_t id_base, const double *queries,
+                                           int64_t nq, int64_t q_ld, int32_t k, int32_t *out_ids, double *out_dist, void *workspace,
+                                           size_t workspace_bytes, const int32_t *row_group, const int32_t *query_group,
+                                           void *stream) {
+    if (!row_off || !cols || !vals || !plan || !pp || !queries || !out_ids || !out_dist || n <= 0 || nq < 0 || dim <= 0 || q_ld < dim || k <= 0 ||
+        !row_group != !query_group)
         return MORNA_ERR_INVALID_ARGUMENT;
     if (!workspace || workspace_bytes < morna_knn_exact_sparse_workspace_bytes(n, nq, k)) return MORNA_ERR_WORKSPACE_TOO_SMALL;
     if (nq == 0) return MORNA_OK;
@@ -366,16 +376,28 @@ extern "C" int morna_knn_exact_sparse(const int64_t *row_off, const int32_t *col
                                                                    qq + q0, dist, n);
             MORNA_LAUNCH_CHECK();
         }
+        if (row_group) {
+            const int rc = launch_mask_excluded(dist, n, n, cnt, row_group, query_group + q0, s);
+            if (rc != MORNA_OK) return rc;
+        }
         if (k <= kRsMaxK && n <= 0x7fffffff) {
             const size_t smem = (size_t)kRsMaxK * (sizeof(double) + sizeof(int));
             select_radix_kernel<<<(unsigned)cnt, kRsThreads, smem, s>>>(dist, n, n, id_base, k, out_ids + q0 * k, out_dist + q0 * k);
             MORNA_LAUNCH_CHECK();
+            if (row_group) {
+                const int rc = launch_pad_masked(out_ids + q0 * k, out_dist + q0 * k, cnt * k, s);
+                if (rc != MORNA_OK) return rc;
+            }
             continue;
         }
         for (int64_t y0 = 0; y0 < cnt; y0 += 65535) {
             const int64_t ny = cnt - y0 < 65535 ? cnt - y0 : 65535;
             int rc = morna_select_topk(dist + y0 * n, nullptr, n, n, id_base, ny, k, out_ids + (q0 + y0) * k, out_dist + (q0 + y0) * k,
                                        sel_ws, sel_bytes, stream);
+            if (rc != MORNA_OK) return rc;
+        }
+        if (row_group) {
+            const int rc = launch_pad_masked(out_ids + q0 * k, out_dist + q0 * k, cnt * k, s);
             if (rc != MORNA_OK) return rc;
         }
     }

@@ -90,11 +90,18 @@ def all_gather_topk(ids, dists, group=None):
     return torch.cat(gi, dim=1), torch.cat(gd, dim=1)
 
 
-def sharded_exact_search(local_search, queries, k, group=None, merge=None):
+def _no_exclusion(query_groups):
+    if query_groups is not None:
+        raise ValueError("rows-sharded search has no per-query exclusion (query_groups); search one GPU's index instead")
+
+
+def sharded_exact_search(local_search, queries, k, group=None, merge=None, query_groups=None):
     """`local_search(queries, k)` -> this rank's (ids, dists) with GLOBAL internal ids, sorted under the
     reference order.  Returns the merged global (ids, dists), identical on every rank.  On the GPU the
     lists are gathered as [world x nq x k] and merged by rank counting (morna_merge_sorted_topk); a
-    `merge(ids [nq x world*k], dists, k)` callable replaces that (the CPU tests pass their own reference rule)."""
+    `merge(ids [nq x world*k], dists, k)` callable replaces that (the CPU tests pass their own reference rule).
+    ``query_groups`` (per-query exclusion) is not supported here: ValueError."""
+    _no_exclusion(query_groups)
     import torch.distributed as td
     ids, dists = local_search(queries, k)
     if not (td.is_available() and td.is_initialized() and td.get_world_size(group) > 1):
@@ -106,7 +113,7 @@ def sharded_exact_search(local_search, queries, k, group=None, merge=None):
     return (merge or merge_topk)(ids, dists, k)
 
 
-def sharded_batched_search(search, queries, k, group=None, check_overflow=True):
+def sharded_batched_search(search, queries, k, group=None, check_overflow=True, query_groups=None):
     """Rows-sharded exact search of a query batch on the tensor-core path, one process per GPU.  `search` holds this
     rank's row block (MornaSearch(..., shard=(rank, world))), `queries` (CUDA float64 [nq x dim]) are replicated.
 
@@ -118,7 +125,9 @@ def sharded_batched_search(search, queries, k, group=None, check_overflow=True):
       3. every rank re-ranks (exact FP64) and orders its surviving rows; ONE more all-gather moves the [nq x k] lists
          (ids and distances packed in one buffer) and every rank merges them by rank counting.
 
-    Returns (ids, dists), identical on every rank and identical to one process scanning all rows."""
+    Returns (ids, dists), identical on every rank and identical to one process scanning all rows.  ``query_groups``
+    (per-query exclusion) is not supported here: ValueError."""
+    _no_exclusion(query_groups)
     import torch.distributed as td
     world = td.get_world_size(group) if (td.is_available() and td.is_initialized()) else 1
     if world == 1:
@@ -229,7 +238,7 @@ def _range_group_exchange(search, st, lo, hi, counts, group, merge):
     return merge_gathered_csr(every, counts, cap, merge)
 
 
-def sharded_range_search_groups(search, queries, max_distance, group=None, byte_cap=None, merge=None):
+def sharded_range_search_groups(search, queries, max_distance, group=None, byte_cap=None, merge=None, query_groups=None):
     """Range search over a rows-sharded index, one process per GPU: generator over (lo, hi, offsets, ids, dists), the
     device CSR of queries [lo, hi) in query order, as MornaSearch.range_search_groups.  `search` holds this rank's row
     block (MornaSearch(..., shard=(rank, world))); `queries` (CUDA float64 [nq x dim]) and every argument are the same
@@ -241,7 +250,9 @@ def sharded_range_search_groups(search, queries, max_distance, group=None, byte_
          gathered lists plus the merged ones stay under byte_cap (one query per group at least);
       3. per group every rank writes its lists, ONE all-gather of the packed lists (skipped when no rank has a
          match), and morna_merge_sorted_csr (or `merge`) puts every entry in its place.
-    Collectives use flat 1-D tensors on the queries' device (NCCL with CUDA tensors, gloo with CPU tensors)."""
+    Collectives use flat 1-D tensors on the queries' device (NCCL with CUDA tensors, gloo with CPU tensors).
+    ``query_groups`` (per-query exclusion) is not supported here: ValueError."""
+    _no_exclusion(query_groups)
     import torch.distributed as td
     world = _world_size(group)
     if world == 1:
@@ -269,8 +280,9 @@ def sharded_range_search_groups(search, queries, max_distance, group=None, byte_
             yield (b0 + lo, b0 + hi) + tuple(_range_group_exchange(search, st, lo, hi, rank_counts[:, lo:hi], group, merge))
 
 
-def sharded_range_search(search, queries, max_distance, group=None, merge=None):
+def sharded_range_search(search, queries, max_distance, group=None, merge=None, query_groups=None):
     """The whole device CSR (offsets, ids, dists) of sharded_range_search_groups, as MornaSearch.range_search_device."""
+    _no_exclusion(query_groups)
     if _world_size(group) == 1:
         return search.range_search_device(queries, max_distance)
     return concat_range_groups(list(sharded_range_search_groups(search, queries, max_distance, group, merge=merge)),

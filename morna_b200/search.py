@@ -330,19 +330,49 @@ class MornaSearch(object):
                            "morna_knn_single_workspace_init")
         return ws
 
+    row_group = None                 # device int32 [n]: label of every resident row (set_row_groups), or None
+
+    def set_row_groups(self, labels):
+        """Labels for per-query exclusion: int32 [n], one per resident row (None clears them).  A search given
+        ``query_groups`` then leaves out, for query q, every row whose label equals query_groups[q] (a label < 0 excludes
+        nothing): with every row its own label and a query's label its row's, a stored row no longer finds itself."""
+        if labels is None:
+            self.row_group = None
+            return
+        t = torch.as_tensor(labels).to(device=self.device, dtype=torch.int32).contiguous()
+        if t.shape != (self.row_hi - self.row_lo,):
+            raise ValueError("row labels must be one per resident row (%d), got shape %r" % (self.row_hi - self.row_lo, tuple(t.shape)))
+        self.row_group = t
+
+    def _query_groups(self, query_groups, nq):
+        """Query labels as device int32 [nq], or None without an exclusion."""
+        if query_groups is None:
+            return None
+        if self.row_group is None:
+            raise ValueError("query_groups need row labels: call set_row_groups first")
+        qg = torch.as_tensor(query_groups).to(device=self.device, dtype=torch.int32).contiguous()
+        if qg.shape != (nq,):
+            raise ValueError("query_groups must hold one label per query (%d), got shape %r" % (nq, tuple(qg.shape)))
+        return qg
+
+    def _excl_args(self, qg, rows=slice(None)):
+        """The (row_group, query_group) pointers an *_excl entry point takes."""
+        return (_lib.dev_ptr(self.row_group[rows]), _lib.dev_ptr(qg))
+
     MAX_SELECT_K = 2048              # kSelMaxK of morna_select_topk
     sparse_exact = False             # set at load for a sparse index whose tie groups would overflow the tensor path's lists
     TIE_GROUP_FOR_SPARSE_PATH = 512  # (the final candidate lists hold 1024 rows; a query usually sees two or more such groups)
 
-    def exact_search_device(self, queries, k, stream=None, allow_single=True):
+    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None):
         """queries: CUDA float64 [nq x dim].  Returns device (ids int32 [nq x k], dists float64 [nq x k]); ids are
         global internal ids (row_lo + local row); short lists are padded with id -1 / +inf.  Like the reference's
         exact_search_nn (morna.py:681-712) any k is served: k above the number of rows returns every row, k <= 0
-        an empty list."""
+        an empty list.  ``query_groups`` (int32 [nq], see set_row_groups): query q leaves out the rows labelled
+        query_groups[q]; the lists are the brute-force lists of the remaining rows."""
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2
         if stream is not None and stream != torch.cuda.current_stream(self.device):
             with torch.cuda.stream(stream):
-                return self.exact_search_device(queries, k, allow_single=allow_single)
+                return self.exact_search_device(queries, k, allow_single=allow_single, query_groups=query_groups)
         queries = queries.contiguous()
         nq = queries.shape[0]
         q_ld = queries.shape[1]            # (a size-1 leading dimension may report stride 0)
@@ -353,41 +383,43 @@ class MornaSearch(object):
         out_ids = torch.full((nq, k), -1, dtype=torch.int32, device=dev)
         out_d = torch.full((nq, k), float("inf"), dtype=torch.float64, device=dev)
         k_eff = min(k, n)
+        qg = self._query_groups(query_groups, nq)
         if n == 0 or nq == 0 or k_eff == 0:
             return out_ids, out_d
-        if nq == 1 and allow_single and k_eff <= 512 and self.csr is None:
+        if nq == 1 and allow_single and k_eff <= 512 and self.csr is None and qg is None:
             return self.single_search_device(queries[0], k)
+        excl = () if qg is None else self._excl_args(qg)
         with torch.cuda.device(dev):
             if k_eff > self.MAX_SELECT_K:
-                return self._full_sort_search(queries, k, out_ids, out_d)
+                return self._full_sort_search(queries, k, out_ids, out_d, qg)
             ids_k = out_ids if k_eff == k else torch.empty((nq, k_eff), dtype=torch.int32, device=dev)
             d_k = out_d if k_eff == k else torch.empty((nq, k_eff), dtype=torch.float64, device=dev)
             if self.csr is not None and bool(torch.isfinite(queries).all()):
                 row_off, cols, vals, plan = self.csr
                 ws = self._workspace(self.lib.morna_knn_exact_sparse_workspace_bytes(n, nq, k_eff), "sparse")
-                _lib.check(self.lib.morna_knn_exact_sparse(
+                _lib.check((self.lib.morna_knn_exact_sparse_excl if excl else self.lib.morna_knn_exact_sparse)(
                     _lib.dev_ptr(row_off), _lib.dev_ptr(cols), _lib.dev_ptr(vals), _lib.dev_ptr(plan), _lib.dev_ptr(self.pp), n,
                     self.dim, self.row_lo,
                     _lib.ptr(queries), nq, q_ld, k_eff, _lib.dev_ptr(ids_k), _lib.dev_ptr(d_k), _lib.dev_ptr(ws), ws.numel(),
-                    _lib.stream_ptr()), "morna_knn_exact_sparse")
+                    *excl, _lib.stream_ptr()), "morna_knn_exact_sparse")
                 if k_eff != k:
                     out_ids[:, :k_eff] = ids_k
                     out_d[:, :k_eff] = d_k
                 return out_ids, out_d
             ws = self._workspace(self.lib.morna_knn_exact_workspace_bytes(n, nq, k_eff))
-            _lib.check(self.lib.morna_knn_exact(
+            _lib.check((self.lib.morna_knn_exact_excl if excl else self.lib.morna_knn_exact)(
                 _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, self.row_lo,
                 _lib.ptr(queries), nq, q_ld, k_eff, _lib.dev_ptr(ids_k), _lib.dev_ptr(d_k),
-                _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_knn_exact")
+                _lib.dev_ptr(ws), ws.numel(), *excl, _lib.stream_ptr()), "morna_knn_exact")
             if k_eff != k:
                 out_ids[:, :k_eff] = ids_k
                 out_d[:, :k_eff] = d_k
         return out_ids, out_d
 
-    def _full_sort_search(self, queries, k, out_ids, out_d):
+    def _full_sort_search(self, queries, k, out_ids, out_d, qg=None):
         """k beyond the select kernel's list size (2048): all distances (morna_angular_distances, the canonical FP64
         sums) and a full device sort per query under the reference order -- rare (a user asking for thousands of
-        neighbours), so the sort is torch's."""
+        neighbours), so the sort is torch's.  With query labels `qg`, excluded rows sit at +inf and end as padding."""
         n, dev = self.row_hi - self.row_lo, self.device
         k_eff = min(k, n)
         dist = torch.empty(n, dtype=torch.float64, device=dev)
@@ -395,11 +427,14 @@ class MornaSearch(object):
             _lib.check(self.lib.morna_angular_distances(
                 _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.ptr(queries[j]), 1, self.dim,
                 _lib.dev_ptr(dist), n, _lib.stream_ptr()), "morna_angular_distances")
+            if qg is not None:
+                dist.masked_fill_((self.row_group == qg[j]) & (qg[j] >= 0), float("inf"))
             # distance ascending, equal distances id descending: stable sort of the id-reversed array
             order = torch.sort(dist.flip(0), stable=True).indices[:k_eff]
             rows = (n - 1) - order
-            out_ids[j, :k_eff] = (rows + self.row_lo).to(torch.int32)
-            out_d[j, :k_eff] = dist[rows]
+            d = dist[rows]
+            out_ids[j, :k_eff] = torch.where(torch.isinf(d), -1, rows + self.row_lo).to(torch.int32)
+            out_d[j, :k_eff] = d
         return out_ids, out_d
 
     # ------------------------------------------------------------------ batched search (tensor cores)
@@ -420,9 +455,10 @@ class MornaSearch(object):
         self._bws = {}
         self.last_stats = None
 
-    def _batched_launch(self, queries, k, stream=None, phase_events=None):
+    def _batched_launch(self, queries, k, stream=None, phase_events=None, qg=None):
         """Enqueues morna_knn_batched for every row block; no host synchronisation.  Returns the
-        per-block (b0, b1, ids, dists, overflow, stats) device tensors."""
+        per-block (b0, b1, ids, dists, overflow, stats) device tensors.  With query labels `qg`: the scoring half with
+        the exclusion (each block given its slice of row_group), then the usual re-rank."""
         nq, dev = queries.shape[0], self.device
         n = self.row_hi - self.row_lo
         sid = (stream if stream is not None else torch.cuda.current_stream(dev)).cuda_stream
@@ -438,19 +474,32 @@ class MornaSearch(object):
                 ws = self._bws.get(sid)                # one workspace per stream: batches in flight do not share
                 if ws is None or ws.numel() < need:
                     ws = self._bws[sid] = _lib.workspace(need, dev)
-                _lib.check(self.lib.morna_knn_batched(
-                    _lib.dev_ptr(self.vectors[b0:b1]), _lib.dev_ptr(self.pp[b0:b1]), _lib.dev_ptr(self.hs[b0:b1]),
-                    self.ld_h, _lib.dev_ptr(self.rho_max), b1 - b0, self.dim, self.ld, self.row_lo + b0,
-                    _lib.ptr(queries), nq, self.dim, k, _lib.dev_ptr(out_ids), _lib.dev_ptr(out_d),
-                    _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws), ws.numel(),
-                    phase_events, _lib.stream_ptr(stream)), "morna_knn_batched")
+                if qg is None:
+                    _lib.check(self.lib.morna_knn_batched(
+                        _lib.dev_ptr(self.vectors[b0:b1]), _lib.dev_ptr(self.pp[b0:b1]), _lib.dev_ptr(self.hs[b0:b1]),
+                        self.ld_h, _lib.dev_ptr(self.rho_max), b1 - b0, self.dim, self.ld, self.row_lo + b0,
+                        _lib.ptr(queries), nq, self.dim, k, _lib.dev_ptr(out_ids), _lib.dev_ptr(out_d),
+                        _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws), ws.numel(),
+                        phase_events, _lib.stream_ptr(stream)), "morna_knn_batched")
+                else:
+                    _lib.check(self.lib.morna_knn_batched_score_excl(
+                        _lib.dev_ptr(self.hs[b0:b1]), self.ld_h, _lib.dev_ptr(self.rho_max), b1 - b0, self.dim, self.row_lo + b0,
+                        _lib.ptr(queries), nq, self.dim, k, _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws),
+                        ws.numel(), phase_events, None, None, *self._excl_args(qg, slice(b0, b1)), _lib.stream_ptr(stream)),
+                        "morna_knn_batched_score_excl")
+                    _lib.check(self.lib.morna_knn_batched_rerank(
+                        _lib.dev_ptr(self.vectors[b0:b1]), _lib.dev_ptr(self.pp[b0:b1]), b1 - b0, self.dim, self.ld,
+                        self.row_lo + b0, _lib.ptr(queries), nq, self.dim, k, _lib.dev_ptr(out_ids), _lib.dev_ptr(out_d),
+                        _lib.dev_ptr(overflow), _lib.dev_ptr(ws), ws.numel(), 0, _lib.stream_ptr(stream)),
+                        "morna_knn_batched_rerank")
                 parts.append((b0, b1, out_ids, out_d, overflow, stats))
         return parts
 
-    def _batched_finish(self, parts, queries, k, stream=None, host_stats=None):
+    def _batched_finish(self, parts, queries, k, stream=None, host_stats=None, qg=None):
         """Host half: queries whose candidate lists overflowed (ties wider than the lists) are answered
         by the exact scan, then the row blocks' lists are merged.  `host_stats`: stats already copied
-        to the host, one [4] int tensor per block; otherwise they are read here (synchronises)."""
+        to the host, one [4] int tensor per block; otherwise they are read here (synchronises).  `qg`: the
+        query labels of an excluded search (the scan then masks the same rows)."""
         from . import dist as mdist
         stats_total = torch.zeros(4, dtype=torch.int64)
         for i, (b0, b1, out_ids, out_d, overflow, stats) in enumerate(parts):
@@ -464,7 +513,10 @@ class MornaSearch(object):
                 sub.row_lo, sub.row_hi, sub._ws_pool = self.row_lo + b0, self.row_lo + b1, {}
                 if (b0, b1) != (0, self.row_hi - self.row_lo):
                     sub.csr = None                          # (the CSR form covers the whole resident block)
-                e_ids, e_d = sub.exact_search_device(queries[idx], k, stream, allow_single=False)
+                if qg is not None:
+                    sub.row_group = self.row_group[b0:b1]
+                e_ids, e_d = sub.exact_search_device(queries[idx], k, stream, allow_single=False,
+                                                     query_groups=None if qg is None else qg[idx])
                 out_ids[idx] = e_ids
                 out_d[idx] = e_d
         self.last_stats = stats_total.tolist()
@@ -472,11 +524,11 @@ class MornaSearch(object):
             return parts[0][2], parts[0][3]
         return mdist.merge_topk(torch.cat([p[2] for p in parts], 1), torch.cat([p[3] for p in parts], 1), k, stream)
 
-    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None):
+    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None):
         """Same contract and same results as exact_search_device, with the N x D
         contraction on the tensor cores (fp16 first pass with a rigorous error bound,
         FP64 re-rank).  Queries whose candidate lists overflow (massive ties) are
-        answered by the exact scan."""
+        answered by the exact scan.  ``query_groups``: per-query exclusion, as in exact_search_device."""
         from . import dist as mdist
         self.enable_tensor_path()
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2
@@ -484,11 +536,12 @@ class MornaSearch(object):
         nq = queries.shape[0]
         n = self.row_hi - self.row_lo
         assert queries.shape[1] == self.dim
+        qg = self._query_groups(query_groups, nq)
         if n == 0 or nq == 0 or k > 512 or k <= 0 or k > n or (self.csr is not None and self.sparse_exact):
-            return self.exact_search_device(queries, k, stream)     # (a sparse index: its ties would overflow every list)
-        parts = self._batched_launch(queries, k, stream, phase_events)
+            return self.exact_search_device(queries, k, stream, query_groups=qg)   # (a sparse index: its ties would overflow every list)
+        parts = self._batched_launch(queries, k, stream, phase_events, qg)
         if check_overflow:
-            return self._batched_finish(parts, queries, k, stream)
+            return self._batched_finish(parts, queries, k, stream, qg=qg)
         if len(parts) == 1:
             return parts[0][2], parts[0][3]
         return mdist.merge_topk(torch.cat([p[2] for p in parts], 1), torch.cat([p[3] for p in parts], 1), k, stream)
@@ -566,23 +619,31 @@ class MornaSearch(object):
             return self._batched_finish(parts, queries, k)
         return out_ids, out_d
 
-    def search_batches(self, batches, k, depth=2, side_job=False):
+    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None):
         """Streams query batches through the GPU: generator over ``batches`` (each a numpy or torch
         [nq x dim] float32/float64 array, or a 1-D integer array of INTERNAL IDS whose stored rows are the queries, as
         ``search -q``) yielding ``(ids, dists)`` numpy arrays in order -- the same
         results as ``exact_search_batch`` per batch.  ``depth`` batches are in flight, each on its own
         CUDA stream with its own pinned staging buffers and workspace, so batch i+1's host->device
-        copy and batch i-1's device->host copy overlap batch i's kernels."""
+        copy and batch i-1's device->host copy overlap batch i's kernels.
+        ``query_groups`` (per-query exclusion, see set_row_groups): True -- every batch is internal ids and takes its
+        labels from row_group[ids] (a stored row then never finds itself); or an iterable of int32 label arrays, one per
+        batch, in step with ``batches``.  Not with ``side_job``."""
+        if query_groups is not None and side_job:
+            raise ValueError("side_job cannot be combined with query_groups")
+        if query_groups is not None and self.row_group is None:
+            raise ValueError("query_groups need row labels: call set_row_groups first")
         pipes = self.__dict__.setdefault("_pipes", {})
         pipe = pipes.get((k, depth))           # slots (streams, pinned buffers, workspaces) are kept between calls
         if pipe is None or pipe.head != pipe.tail or pipe.side_job != (bool(side_job) and depth > 1):
             pipe = pipes[(k, depth)] = BatchPipeline(self, k, depth, side_job)
+        labels = iter(query_groups) if query_groups is not None and query_groups is not True else None
         pending = 0
         for q in batches:
             if pending == depth:
                 yield pipe.collect()
                 pending -= 1
-            pipe.submit(q)
+            pipe.submit(q, query_groups=next(labels) if labels is not None else query_groups)
             pending += 1
         while pending:
             yield pipe.collect()
@@ -623,14 +684,15 @@ class MornaSearch(object):
             return None
         return out[8 * k:12 * k].view(np.int32).reshape(1, k).copy(), out[:8 * k].view(np.float64).reshape(1, k).copy()
 
-    def exact_search_batch(self, queries, k, tensor_cores=None):
+    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None):
         """Host entry: queries numpy [nq x dim] (float32 or float64) -> numpy (ids, dists).
         float32 queries cross PCIe as float32 and are widened (exactly) on the device.  Batches of 64+
-        queries use the tensor-core path, which returns the same bits as the scan."""
+        queries use the tensor-core path, which returns the same bits as the scan.  ``query_groups``: per-query
+        exclusion, as in exact_search_device."""
         queries = np.ascontiguousarray(queries)
         if queries.dtype != np.float32:
             queries = queries.astype(np.float64, copy=False)
-        if queries.shape[0] == 1 and not tensor_cores:
+        if queries.shape[0] == 1 and not tensor_cores and query_groups is None:
             got = self._single_query_host(queries[0], k)
             if got is not None:
                 return got
@@ -640,12 +702,13 @@ class MornaSearch(object):
         qd = q.to(self.device, non_blocking=True).to(torch.float64)
         if tensor_cores is None:
             tensor_cores = qd.shape[0] >= 64
-        ids, d = (self.batched_search_device if tensor_cores else self.exact_search_device)(qd, k)
+        ids, d = (self.batched_search_device if tensor_cores else self.exact_search_device)(qd, k, query_groups=query_groups)
         return ids.cpu().numpy(), d.cpu().numpy()
 
-    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False):
-        """morna.py:681-730 for the current ``query_sample``."""
-        ids, d = self.exact_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], num_neighbors)
+    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None):
+        """morna.py:681-730 for the current ``query_sample``; ``query_groups``: its label ([1]), as in exact_search_device."""
+        ids, d = self.exact_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], num_neighbors,
+                                         query_groups=query_groups)
         keep = ids[0] >= 0
         results = (ids[0][keep].tolist(),)
         if include_distances:
@@ -655,10 +718,13 @@ class MornaSearch(object):
         return results
 
     # ------------------------------------------------------------------ approximate mode
-    def approx_search_device(self, queries, k):
+    def approx_search_device(self, queries, k, query_groups=None):
         """The k best rows by fp16 tensor-core score, no exact re-rank (morna_knn_batched_approx): the approximate mode
         that stands where the reference asks Annoy (morna.py:632-678).  Same contract as batched_search_device; queries
-        whose lists overflow, tiny shards and sparse indexes are answered exactly."""
+        whose lists overflow, tiny shards and sparse indexes are answered exactly.  There is no per-query exclusion in
+        this mode: ``query_groups`` raises ValueError."""
+        if query_groups is not None:
+            raise ValueError("the approximate mode has no per-query exclusion; use an exact search")
         self.enable_tensor_path()
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2 and queries.shape[1] == self.dim
         queries = queries.contiguous()
@@ -698,17 +764,23 @@ class MornaSearch(object):
         return results
 
     def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
-                        meta_db=False, out=None, max_distance=None):
+                        meta_db=False, out=None, max_distance=None, exclude=False):
         """morna.py:733-787 with the stored row as the query (float32 values), run
         through the exact scan.  With ``max_distance``: every sample within it (range_search_nn), the first
-        ``num_neighbors`` of them when that is not None."""
+        ``num_neighbors`` of them when that is not None.  ``exclude``: the query takes its row's label (set_row_groups),
+        so its own sample and every sample of its group are left out."""
         internal_id = _member_internal_id(self.internal_id_map, query_id, out)
         if not (self.row_lo <= internal_id < self.row_hi):
             raise ValueError("internal id %d is not resident on this shard" % internal_id)
         self.query_sample = self.vectors[internal_id - self.row_lo, :self.dim].to(torch.float64).cpu().tolist()
+        qg = None
+        if exclude:
+            if self.row_group is None:
+                raise ValueError("exclude needs row labels: call set_row_groups first")
+            qg = self.row_group[internal_id - self.row_lo:internal_id - self.row_lo + 1]
         if max_distance is not None:
-            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors)
-        return self.exact_search_nn(num_neighbors, include_distances, meta_db)
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg)
+        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg)
 
     def _metadata(self, internal_ids):
         """morna.py:666-676: keywords of every result's sample id from basename.meta.mor."""
@@ -725,26 +797,27 @@ class MornaSearch(object):
     RANGE_BATCH_QUERIES = 4096        # queries per morna_range_batched call (its candidate lists: 4096 x 4096 entries)
     RANGE_TENSOR_MIN_QUERIES = 64     # smaller batches go to the FP64 scan, as top-k batches do
 
-    def range_search_device(self, queries, max_distance):
+    def range_search_device(self, queries, max_distance, query_groups=None):
         """Every row within ``max_distance`` of each query: queries CUDA float64 [nq x dim] -> device CSR (offsets int64
         [nq+1], ids int32 [total], dists float64 [total]); query j's list is ids/dists[offsets[j]:offsets[j+1]], ordered as
         the reference orders results (distance ascending, equal distances id descending), ids global.  The distance is
         exactly exact_search_device's and the comparison inclusive; a query with nothing in range has an empty list.
         Sets ``last_stats`` = [overflowed queries, first-pass survivors, matches] and ``last_range_route`` ("tensor":
-        the tensor-core filter with an FP64 check, overflowed queries answered by the scan; "exact": the FP64 scan)."""
-        return concat_range_groups(list(self.range_search_groups(queries, max_distance)), self.device)
+        the tensor-core filter with an FP64 check, overflowed queries answered by the scan; "exact": the FP64 scan).
+        ``query_groups``: per-query exclusion, as in exact_search_device."""
+        return concat_range_groups(list(self.range_search_groups(queries, max_distance, query_groups=query_groups)), self.device)
 
-    def range_search_groups(self, queries, max_distance, byte_cap=None):
+    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None):
         """Generator over (lo, hi, offsets, ids, dists): the range_search_device CSR of queries [lo, hi), in query order.
         Batches of RANGE_BATCH_QUERIES are counted first (one small read back); with ``byte_cap``, a batch whose lists
         would take more than that many bytes (12 per match) is emitted in groups of consecutive queries that fit it (one
         query per group at least), so no more than that is allocated at once."""
-        for b0, st in self.range_count_batches(queries, max_distance):
+        for b0, st in self.range_count_batches(queries, max_distance, query_groups):
             for lo, hi in _range_groups(st["counts"], byte_cap):
                 off, ids, d = self.range_emit(st, lo, hi)
                 yield b0 + lo, b0 + hi, off, ids, d
 
-    def range_count_batches(self, queries, max_distance):
+    def range_count_batches(self, queries, max_distance, query_groups=None):
         """The counting half of range_search_groups: generator over (b0, st), one per batch of RANGE_BATCH_QUERIES
         queries starting at query b0, where st["counts"] (host int64) holds the batch's matches per query and st is what
         range_emit needs to write any run of its lists.  Updates last_range_route and last_stats as the batches go."""
@@ -752,16 +825,18 @@ class MornaSearch(object):
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2 and queries.shape[1] == self.dim
         queries = queries.contiguous()
         nq = queries.shape[0]
+        qg = self._query_groups(query_groups, nq)
         route = self._range_route(nq)
         stats = [0, 0, 0]
         self.last_range_route, self.last_stats = route, list(stats)
         for b0 in range(0, nq, self.RANGE_BATCH_QUERIES):
-            st = self._range_counts(queries[b0:b0 + self.RANGE_BATCH_QUERIES], r, route)
+            st = self._range_counts(queries[b0:b0 + self.RANGE_BATCH_QUERIES], r, route,
+                                    None if qg is None else qg[b0:b0 + self.RANGE_BATCH_QUERIES])
             stats = [a + b for a, b in zip(stats, st["stats"])]
             self.last_stats = list(stats)
             yield b0, st
 
-    def range_search_batch(self, queries, max_distance):
+    def range_search_batch(self, queries, max_distance, query_groups=None):
         """Host entry: queries numpy [nq x dim] -> numpy CSR (offsets, ids, dists) of range_search_device."""
         queries = np.ascontiguousarray(queries)
         if queries.dtype != np.float32:
@@ -770,12 +845,13 @@ class MornaSearch(object):
         if q.numel():
             q = q.pin_memory()
         qd = q.to(self.device, non_blocking=True).to(torch.float64)
-        return tuple(t.cpu().numpy() for t in self.range_search_device(qd, max_distance))
+        return tuple(t.cpu().numpy() for t in self.range_search_device(qd, max_distance, query_groups))
 
-    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None):
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None):
         """Every indexed sample within ``max_distance`` of the current ``query_sample``, as exact_search_nn returns its
         results; ``num_neighbors``: keep only the first that many."""
-        _, ids, d = self.range_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], max_distance)
+        _, ids, d = self.range_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], max_distance,
+                                            query_groups)
         if num_neighbors is not None:
             ids, d = ids[:max(int(num_neighbors), 0)], d[:max(int(num_neighbors), 0)]
         results = (ids.tolist(),)
@@ -791,47 +867,50 @@ class MornaSearch(object):
         tensor = 0 < n <= self.BATCH_BLOCK_ROWS and nq >= self.RANGE_TENSOR_MIN_QUERIES and not sparse_ties
         return "tensor" if tensor else "exact"
 
-    def _range_counts(self, queries, r, route):
+    def _range_counts(self, queries, r, route, qg=None):
         """Matches per query of one batch (host int64) and what range_emit needs; on the tensor route the counts,
         overflow flags and stats come back in one copy, and overflowed queries are counted again by the scan."""
         nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
         st = {"queries": queries, "r": r, "route": route, "over": np.zeros(0, np.int64), "stats": [0, 0, 0],
-              "counts": np.zeros(nq, np.int64)}
+              "counts": np.zeros(nq, np.int64), "qg": qg}
         if n == 0 or nq == 0:
             return st
+        excl = () if qg is None else self._excl_args(qg)
         with torch.cuda.device(dev):
             if route == "exact":
-                st["counts"] = self._range_exact_counts(queries, r)
+                st["counts"] = self._range_exact_counts(queries, r, qg)
             else:
                 self.enable_tensor_path()
                 counts = torch.empty(nq, dtype=torch.int32, device=dev)
                 overflow = torch.empty(nq, dtype=torch.uint8, device=dev)
                 stats = torch.empty(4, dtype=torch.int64, device=dev)
                 ws = self._workspace(self.lib.morna_range_batched_workspace_bytes(n, nq, self.dim), "range")
-                _lib.check(self.lib.morna_range_batched(
+                _lib.check((self.lib.morna_range_batched_excl if excl else self.lib.morna_range_batched)(
                     _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), _lib.dev_ptr(self.hs), self.ld_h, _lib.dev_ptr(self.rho_max),
                     n, self.dim, self.ld, self.row_lo, _lib.ptr(queries), nq, self.dim, r, _lib.dev_ptr(counts),
-                    _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()),
+                    _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws), ws.numel(), *excl, _lib.stream_ptr()),
                     "morna_range_batched")
                 host = torch.cat([counts.to(torch.int64), overflow.to(torch.int64), stats]).cpu().numpy()
                 c, over = host[:nq].copy(), np.nonzero(host[nq:2 * nq])[0]
                 if len(over):
-                    c[over] = self._range_exact_counts(queries[torch.from_numpy(over).to(dev)], r)
+                    over_dev = torch.from_numpy(over).to(dev)
+                    c[over] = self._range_exact_counts(queries[over_dev], r, None if qg is None else qg[over_dev])
                 st.update(counts=c, over=over, ws=ws, overflow=overflow)
                 st["stats"] = [int(host[2 * nq]), int(host[2 * nq + 1]), 0]
         st["stats"][2] = int(st["counts"].sum())
         return st
 
-    def _range_exact_counts(self, queries, r):
+    def _range_exact_counts(self, queries, r, qg=None):
         nq, n = queries.shape[0], self.row_hi - self.row_lo
         counts = torch.empty(nq, dtype=torch.int32, device=self.device)
         ws = self._workspace(self.lib.morna_range_exact_workspace_bytes(n, nq, 0), "range_exact")
-        _lib.check(self.lib.morna_range_exact_count(
+        excl = () if qg is None else self._excl_args(qg)
+        _lib.check((self.lib.morna_range_exact_count_excl if excl else self.lib.morna_range_exact_count)(
             _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.ptr(queries), nq, self.dim, r,
-            _lib.dev_ptr(counts), _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_range_exact_count")
+            _lib.dev_ptr(counts), _lib.dev_ptr(ws), ws.numel(), *excl, _lib.stream_ptr()), "morna_range_exact_count")
         return counts.cpu().numpy().astype(np.int64)
 
-    def _range_exact_fill(self, queries, r, counts):
+    def _range_exact_fill(self, queries, r, counts, qg=None):
         """FP64 route's lists of `queries` given their counts: device (offsets, ids, dists)."""
         nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
         off = np.zeros(nq + 1, dtype=np.int64)
@@ -842,10 +921,11 @@ class MornaSearch(object):
         d = torch.empty(total, dtype=torch.float64, device=dev)
         if total:
             ws = self._workspace(self.lib.morna_range_exact_workspace_bytes(n, nq, total), "range_exact")
-            _lib.check(self.lib.morna_range_exact_fill(
+            excl = () if qg is None else self._excl_args(qg)
+            _lib.check((self.lib.morna_range_exact_fill_excl if excl else self.lib.morna_range_exact_fill)(
                 _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, self.row_lo, _lib.ptr(queries), nq,
                 self.dim, r, _lib.dev_ptr(offsets), total, _lib.dev_ptr(ids), _lib.dev_ptr(d), _lib.dev_ptr(ws), ws.numel(),
-                _lib.stream_ptr()), "morna_range_exact_fill")
+                *excl, _lib.stream_ptr()), "morna_range_exact_fill")
         return offsets, ids, d
 
     def range_emit(self, st, lo, hi):
@@ -853,8 +933,9 @@ class MornaSearch(object):
         counted."""
         dev, n = self.device, self.row_hi - self.row_lo
         with torch.cuda.device(dev):
+            qg = st["qg"]
             if st["route"] == "exact" or n == 0:
-                return self._range_exact_fill(st["queries"][lo:hi], st["r"], st["counts"][lo:hi])
+                return self._range_exact_fill(st["queries"][lo:hi], st["r"], st["counts"][lo:hi], None if qg is None else qg[lo:hi])
             nq = st["queries"].shape[0]
             counts = st["counts"]
             full = np.zeros(nq + 1, dtype=np.int64)              # queries outside [lo, hi) get empty ranges
@@ -871,8 +952,9 @@ class MornaSearch(object):
                     _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_range_batched_emit")
             over = st["over"][(st["over"] >= lo) & (st["over"] < hi)]
             if len(over):                                        # the scan's lists spliced into their places
-                sub_off, sub_ids, sub_d = self._range_exact_fill(st["queries"][torch.from_numpy(over).to(dev)], st["r"],
-                                                                 counts[over])
+                over_dev = torch.from_numpy(over).to(dev)
+                sub_off, sub_ids, sub_d = self._range_exact_fill(st["queries"][over_dev], st["r"], counts[over],
+                                                                 None if qg is None else qg[over_dev])
                 sub_total = sub_ids.numel()
                 if sub_total:
                     lens = torch.from_numpy(counts[over]).to(dev)
@@ -926,10 +1008,13 @@ class FilteredSearch(object):
             inner.row_lo, inner.row_hi = 0, m
             inner.vectors = parent.vectors.index_select(0, rows)
             inner.pp = parent.pp.index_select(0, rows)
+            if parent.row_group is not None:        # the subset rows keep their labels; queries keep theirs
+                inner.row_group = parent.row_group.index_select(0, rows)
             inner._build_csr()
             inner.query, inner.query_sample = defaultdict(int), [0.0] * parent.dim
         self.inner = inner
         self._parent_rows = parent.vectors if keep_parent_rows else None
+        self._parent_row_group = parent.row_group
 
     def _to_parent(self, ids):
         """Result ids of `inner` (torch on the current stream, or numpy) -> parent internal ids (int32); -1 padding stays."""
@@ -987,13 +1072,19 @@ class FilteredSearch(object):
         return self.inner.vectors[local, :self.dim].to(torch.float64).contiguous()
 
     # ------------------------------------------------------------------ top-k (MornaSearch's entry points, ids mapped)
-    def exact_search_device(self, queries, k, stream=None, allow_single=True):
-        ids, d = self.inner.exact_search_device(queries, k, stream, allow_single)
+    def row_groups_of(self, internal_ids):
+        """Exclusion labels of these parent internal ids (any resident row, in the subset or not), as the parent holds them."""
+        if self._parent_row_group is None:
+            raise ValueError("query_groups need row labels: call set_row_groups on the parent before subset()")
+        return self._parent_row_group[torch.as_tensor(internal_ids).to(self.device).long() - self.row_lo]
+
+    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None):
+        ids, d = self.inner.exact_search_device(queries, k, stream, allow_single, query_groups)
         with torch.cuda.stream(stream):
             return self._to_parent(ids), d
 
-    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None):
-        ids, d = self.inner.batched_search_device(queries, k, stream, check_overflow, phase_events)
+    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None):
+        ids, d = self.inner.batched_search_device(queries, k, stream, check_overflow, phase_events, query_groups)
         with torch.cuda.stream(stream):
             return self._to_parent(ids), d
 
@@ -1006,54 +1097,69 @@ class FilteredSearch(object):
         ids, d = self.inner.single_search_stream(queries, k)
         return self._to_parent(ids), d
 
-    def approx_search_device(self, queries, k):
-        ids, d = self.inner.approx_search_device(queries, k)
+    def approx_search_device(self, queries, k, query_groups=None):
+        ids, d = self.inner.approx_search_device(queries, k, query_groups)
         return self._to_parent(ids), d
 
-    def exact_search_batch(self, queries, k, tensor_cores=None):
-        ids, d = self.inner.exact_search_batch(queries, k, tensor_cores)
+    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None):
+        ids, d = self.inner.exact_search_batch(queries, k, tensor_cores, query_groups)
         return self._to_parent(ids), d
 
-    def search_batches(self, batches, k, depth=2, side_job=False):
+    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None):
         """MornaSearch.search_batches over the subset; a batch of internal ids becomes the stored rows of those ids
-        (stored_queries) on the device.  The distances are views of pinned buffers, as there."""
+        (stored_queries) on the device, and with ``query_groups=True`` takes the parent's labels of those ids (a query
+        outside the subset too).  The distances are views of pinned buffers, as there."""
+        by_rows = query_groups is True
+        labels = iter(query_groups) if query_groups is not None and not by_rows else None
+        pairs = []
+
         def queries():
             for q in batches:
                 t = torch.from_numpy(np.ascontiguousarray(q)) if isinstance(q, np.ndarray) else q
-                yield self.stored_queries(t) if t.dim() == 1 and t.dtype in (torch.int32, torch.int64) else t
-        for ids, d in self.inner.search_batches(queries(), k, depth, side_job):
+                by_id = t.dim() == 1 and t.dtype in (torch.int32, torch.int64)
+                if by_rows and not by_id:
+                    raise ValueError("query_groups=True needs batches of internal ids")
+                pairs.append(self.row_groups_of(t) if by_rows else next(labels) if labels is not None else None)
+                yield self.stored_queries(t) if by_id else t
+        def groups():
+            while True:
+                yield pairs.pop(0)          # the labels of the batch queries() has just yielded
+
+        for ids, d in self.inner.search_batches(queries(), k, depth, side_job, None if query_groups is None else groups()):
             yield self._to_parent(ids), d
 
-    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False):
-        return self._nn(self.inner.exact_search_nn(num_neighbors, include_distances), meta_db)
+    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None):
+        return self._nn(self.inner.exact_search_nn(num_neighbors, include_distances, query_groups=query_groups), meta_db)
 
     def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False):
         return self._nn(self.inner.search_nn(num_neighbors, search_k, include_distances), meta_db)
 
     def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
-                        meta_db=False, out=None, max_distance=None):
-        """MornaSearch.search_member_n over the subset; the queried sample may lie outside it."""
+                        meta_db=False, out=None, max_distance=None, exclude=False):
+        """MornaSearch.search_member_n over the subset; the queried sample may lie outside it (with ``exclude`` it takes
+        its label from the parent's rows)."""
         internal_id = _member_internal_id(self.internal_id_map, query_id, out)
         self.query_sample = self.stored_queries([internal_id])[0].cpu().tolist()
+        qg = self.row_groups_of([internal_id]) if exclude else None
         if max_distance is not None:
-            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors)
-        return self.exact_search_nn(num_neighbors, include_distances, meta_db)
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg)
+        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg)
 
     # ------------------------------------------------------------------ range search
-    def range_search_device(self, queries, max_distance):
-        offsets, ids, d = self.inner.range_search_device(queries, max_distance)
+    def range_search_device(self, queries, max_distance, query_groups=None):
+        offsets, ids, d = self.inner.range_search_device(queries, max_distance, query_groups)
         return offsets, self._to_parent(ids), d
 
-    def range_search_groups(self, queries, max_distance, byte_cap=None):
-        for lo, hi, offsets, ids, d in self.inner.range_search_groups(queries, max_distance, byte_cap):
+    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None):
+        for lo, hi, offsets, ids, d in self.inner.range_search_groups(queries, max_distance, byte_cap, query_groups):
             yield lo, hi, offsets, self._to_parent(ids), d
 
-    def range_search_batch(self, queries, max_distance):
-        offsets, ids, d = self.inner.range_search_batch(queries, max_distance)
+    def range_search_batch(self, queries, max_distance, query_groups=None):
+        offsets, ids, d = self.inner.range_search_batch(queries, max_distance, query_groups)
         return offsets, self._to_parent(ids), d
 
-    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None):
-        return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors), meta_db)
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None):
+        return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors, query_groups), meta_db)
 
 
 class _PipeSlot(object):
@@ -1085,7 +1191,7 @@ class BatchPipeline(object):
             sl.compute = self.compute if self.side_job else torch.cuda.Stream(device=dev)
             sl.h2d, sl.scored, sl.ranked, sl.done = (torch.cuda.Event() for _ in range(4))
             sl.nq = -1
-            sl.host_q = sl.ws = sl.job = sl.parts = None
+            sl.host_q = sl.ws = sl.job = sl.parts = sl.qg = None
             self.slots.append(sl)
         self.head = self.tail = 0           # next slot to submit into / to collect from
         self.unranked = None                # the slot whose candidate lists wait for their re-rank
@@ -1114,10 +1220,16 @@ class BatchPipeline(object):
         if sl.ws is None or sl.ws.numel() < need:
             sl.ws = _lib.workspace(need, s.device)
         job = ctypes.byref(side.job) if side is not None else None
-        _lib.check(lib.morna_knn_batched_score(
-            _lib.dev_ptr(s.hs), s.ld_h, _lib.dev_ptr(s.rho_max), n, s.dim, s.row_lo, _lib.ptr(sl.qd), sl.nq, s.dim, k,
-            _lib.dev_ptr(sl.overflow), _lib.dev_ptr(sl.stats), _lib.dev_ptr(sl.ws), sl.ws.numel(), None, job, None,
-            _lib.stream_ptr()), "morna_knn_batched_score")
+        if sl.qg is None:
+            _lib.check(lib.morna_knn_batched_score(
+                _lib.dev_ptr(s.hs), s.ld_h, _lib.dev_ptr(s.rho_max), n, s.dim, s.row_lo, _lib.ptr(sl.qd), sl.nq, s.dim, k,
+                _lib.dev_ptr(sl.overflow), _lib.dev_ptr(sl.stats), _lib.dev_ptr(sl.ws), sl.ws.numel(), None, job, None,
+                _lib.stream_ptr()), "morna_knn_batched_score")
+        else:
+            _lib.check(lib.morna_knn_batched_score_excl(
+                _lib.dev_ptr(s.hs), s.ld_h, _lib.dev_ptr(s.rho_max), n, s.dim, s.row_lo, _lib.ptr(sl.qd), sl.nq, s.dim, k,
+                _lib.dev_ptr(sl.overflow), _lib.dev_ptr(sl.stats), _lib.dev_ptr(sl.ws), sl.ws.numel(), None, job, None,
+                *s._excl_args(sl.qg), _lib.stream_ptr()), "morna_knn_batched_score_excl")
         sl.job = _lib.RerankJob(s.vectors.data_ptr(), s.pp.data_ptr(), n, s.dim, s.ld, s.row_lo, sl.qd.data_ptr(), sl.nq, s.dim, k,
                                 sl.overflow.data_ptr(), sl.ws.data_ptr(), sl.ws.numel())
 
@@ -1129,8 +1241,10 @@ class BatchPipeline(object):
         replayed from then on: one launch per batch instead of twelve (no gaps between the kernels, a tenth of the host
         time).  Any change of buffer or size falls back to plain launches."""
         def buffers():
+            # (with an exclusion the captured scoring call also reads the row labels: set_row_groups may replace them)
+            labels = (sl.qg.data_ptr(), self.search.row_group.data_ptr()) if sl.qg is not None else 0
             return (sl.nq, sl.qd.data_ptr(), sl.ws.data_ptr() if sl.ws is not None else 0, sl.ids.data_ptr(), sl.d.data_ptr(),
-                    sl.overflow.data_ptr(), sl.stats.data_ptr())
+                    sl.overflow.data_ptr(), sl.stats.data_ptr(), labels)
         key = buffers()
         if self.use_graphs and getattr(sl, "graph_key", None) == key:
             sl.graph.replay()
@@ -1210,7 +1324,19 @@ class BatchPipeline(object):
             raise ValueError("internal ids %d..%d are not all resident on this shard (rows %d..%d)"
                              % (lo, hi, s.row_lo, s.row_hi - 1))
 
-    def submit(self, queries):
+    def _stage_groups(self, sl, labels):
+        """The batch's query labels in the slot's own device buffer (a stable address for the captured step), or None."""
+        if labels is None:
+            sl.qg = None
+            return
+        if getattr(sl, "qgbuf", None) is None or sl.qgbuf.shape[0] != sl.nq:
+            sl.qgbuf = torch.empty(max(sl.nq, 1), dtype=torch.int32, device=self.search.device)
+        sl.qgbuf[:sl.nq].copy_(torch.as_tensor(labels).reshape(-1).to(device=self.search.device, dtype=torch.int32),
+                               non_blocking=True)
+        sl.qg = sl.qgbuf[:sl.nq]
+
+    def submit(self, queries, query_groups=None):
+        """``query_groups``: None, True (a batch of internal ids takes the labels row_group[ids]) or int32 labels [nq]."""
         s, k = self.search, self.k
         sl = self.slots[self.head % self.depth]
         assert self.head - self.tail < self.depth, "collect() before submitting more than `depth` batches"
@@ -1218,6 +1344,13 @@ class BatchPipeline(object):
         by_id = q.dim() == 1 and q.dtype in (torch.int32, torch.int64)      # stored rows as queries (search -q): only ids cross PCIe
         if by_id:
             self._check_resident_ids(q)      # before the slot is taken: the pipeline stays usable after the error
+        if query_groups is not None:
+            if self.side_job:
+                raise ValueError("side_job cannot be combined with query_groups")
+            if query_groups is True and not by_id:
+                raise ValueError("query_groups=True needs a batch of internal ids")
+            if len(torch.as_tensor(q if query_groups is True else query_groups).reshape(-1)) != q.shape[0]:
+                raise ValueError("query_groups must hold one label per query")
         self.head += 1
         if by_id:
             self._size(sl, q.shape[0], torch.float64, staging=False)
@@ -1225,7 +1358,17 @@ class BatchPipeline(object):
                 if q.is_cuda:
                     sl.stream.wait_stream(torch.cuda.current_stream(s.device))
                 rows = q.to(s.device, non_blocking=True).long() - s.row_lo
-                sl.qd = s.vectors[rows, :s.dim].to(torch.float64).contiguous()
+                if query_groups is None:
+                    sl.qd = s.vectors[rows, :s.dim].to(torch.float64).contiguous()
+                else:
+                    # an excluded batch by ids goes to the slot's own buffer: with its labels also in a slot buffer, the
+                    # step's addresses stay the same from batch to batch, so it is captured and replayed as a vector
+                    # batch's is (a search without an exclusion takes the line above, as it always has)
+                    if getattr(sl, "qbuf", None) is None or sl.qbuf.shape[0] != sl.nq:
+                        sl.qbuf = torch.empty((sl.nq, s.dim), dtype=torch.float64, device=s.device)
+                    sl.qbuf.copy_(s.vectors[rows, :s.dim])
+                    sl.qd = sl.qbuf
+                self._stage_groups(sl, s.row_group[rows] if query_groups is True else query_groups)
                 sl.h2d.record(sl.stream)
             self._launch(sl)
             return
@@ -1249,6 +1392,7 @@ class BatchPipeline(object):
                     sl.qbuf = torch.empty((sl.nq, s.dim), dtype=torch.float64, device=s.device)
                 sl.qbuf.copy_(src.to(s.device, non_blocking=True))
                 sl.qd = sl.qbuf
+            self._stage_groups(sl, query_groups)
             sl.h2d.record(sl.stream)
         self._launch(sl)
 
@@ -1264,7 +1408,7 @@ class BatchPipeline(object):
             if n == 0 or sl.nq == 0 or k > 512 or k <= 0 or k > n or (s.csr is not None and s.sparse_exact):
                 if prev is not None:
                     self._rerank(prev, resume=False)
-                ids, d = s.exact_search_device(sl.qd, k)
+                ids, d = s.exact_search_device(sl.qd, k, query_groups=sl.qg)
                 sl.keep = (ids, d)
                 sl.ranked.record()
                 self._copy_back(sl, ids, d, [])
@@ -1272,7 +1416,7 @@ class BatchPipeline(object):
                 if prev is not None:
                     self._rerank(prev, resume=False)
                 sl.mode = "blocks"
-                sl.parts = s._batched_launch(sl.qd, k)
+                sl.parts = s._batched_launch(sl.qd, k, qg=sl.qg)
                 sl.ranked.record()
                 self._copy_back(sl, None, None, [part[5] for part in sl.parts])
             elif not self.side_job:
@@ -1303,7 +1447,7 @@ class BatchPipeline(object):
         overflowed = int(sl.host_stats[:nparts, 0].sum()) > 0
         if overflowed or nparts > 1:         # rare: exact-scan fix-up and/or merge of row blocks, then copy again
             with torch.cuda.stream(sl.compute):
-                ids, d = s._batched_finish(sl.parts, sl.qd, k, host_stats=[sl.host_stats[i] for i in range(nparts)])
+                ids, d = s._batched_finish(sl.parts, sl.qd, k, host_stats=[sl.host_stats[i] for i in range(nparts)], qg=sl.qg)
                 sl.host_ids.copy_(ids, non_blocking=True)
                 sl.host_d.copy_(d, non_blocking=True)
             sl.compute.synchronize()
