@@ -852,8 +852,10 @@ extern "C" int morna_index_accumulate(const int64_t *row_off, const uint8_t *pas
     AccWs w = acc_ws_layout(n_rows, nnz, dim);
     if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
     cudaStream_t s = (cudaStream_t)stream;
-    if (n_rows == 0 || id_hi == id_lo) {
-        MORNA_CUDA_TRY(cudaMemsetAsync(acc, 0, (size_t)dim * (size_t)acc_ld * sizeof(double), s));
+    if (n_rows == 0 || id_hi == id_lo) {     // nothing to add: cells [0, id_hi - id_lo) are zero, the rest stays untouched
+        if (id_hi > id_lo)
+            MORNA_CUDA_TRY(cudaMemset2DAsync(acc, (size_t)acc_ld * sizeof(double), 0, (size_t)(id_hi - id_lo) * sizeof(double),
+                                             (size_t)dim, s));
         return MORNA_OK;
     }
     // (no zero-fill of acc: the kernels below write every cell [0, id_hi - id_lo) of every bucket column -- the sums of a
