@@ -458,6 +458,47 @@ int morna_range_exact_fill_excl(const float *vectors, const double *pp, int64_t 
 int morna_merge_sorted_csr(const void *gathered, int32_t n_lists, int64_t nq, int64_t cap, const int64_t *rank_offsets,
                            const int64_t *out_offsets, int64_t total, int32_t *out_ids, double *out_dist, void *stream);
 
+/* Group-capped search: per query, the nearest rows with at most max_per_group (N >= 1) rows of any one group.  Every row
+ * carries a cap label (int32; < 0: ungrouped, a group of its own).  The answer is the walk over the brute-force list of
+ * the allowed rows in the reference order (distance ascending, equal distances id descending): a row is kept iff fewer
+ * than N rows of its group were kept before it, and the walk stops after k kept rows.
+ *
+ * The walk as a primitive, on lists already in the reference order:
+ *   offsets   [dev] int64[n_lists + 1]: list j is entries [offsets[j], offsets[j + 1]) of ids / dists (total entries)
+ *   cap_group [dev] int32[n_rows]: the label of id i is cap_group[i - id_base]; an id outside the rows is ungrouped;
+ *             an id < 0 is padding and skipped
+ *   limit     at most this many entries kept per list (< 0: no limit)
+ *   out_ld > 0: list j written to out_ids / out_dists [n_lists x out_ld], padded with id -1 / +inf (0 <= limit <= out_ld;
+ *             out_offsets unused)
+ *   out_ld == 0: a CSR -- out_offsets [dev] int64[n_lists + 1] from 0, list j's kept entries at [out_offsets[j],
+ *             out_offsets[j + 1]) of out_ids / out_dists (room for `total` entries)
+ * Ids and distance bits are copied unchanged; no host synchronisation; any list length. */
+size_t morna_cap_sorted_lists_workspace_bytes(int64_t n_lists, int64_t total);
+int morna_cap_sorted_lists(const int64_t *offsets, int64_t n_lists, const int32_t *ids, const double *dists, int64_t total,
+                           const int32_t *cap_group, int32_t id_base, int64_t n_rows, int32_t max_per_group, int64_t limit,
+                           int64_t *out_offsets, int32_t *out_ids, double *out_dists, int64_t out_ld, void *workspace,
+                           size_t workspace_bytes, void *stream);
+/* The capped top-k on the tensor cores (arguments as morna_knn_batched; cap_group covers this call's n rows; row_group /
+ * query_group: an optional exclusion as in morna_knn_batched_score_excl, both NULL or both set).  The selection passes
+ * use capped k-th scores (the k-th best score among every group's best N) for their thresholds and drop an entry once N
+ * rows of its group score more than 2 eps above it; the final lists are re-ranked in FP64 as usual, sorted whole and
+ * walked.  out_ids / out_dist [nq x k] are the exact capped answer, bit for bit, padded with id -1 / +inf, for every
+ * query not flagged in overflow (its lists overflowed: answer it with the walk over its full FP64 list).  1 <= k <= 512,
+ * n <= 2^24.  stats as morna_knn_batched.
+ *   block_ends [host] n_block_ends ascending row counts: after the pilot, blocks of rows end at these (ends at or below
+ *              the pilot's rows are skipped), then the usual blocks follow, with a capped refinement between blocks.
+ *              While the rows scored so far hold few capped entries the thresholds are weak (absent below k) and the
+ *              filter appends most rows of a block, so a block must be small for the lists to stay below 4096 entries.
+ *              Any schedule gives the same results (a list that overflows goes to the FP64 route); MornaSearch sizes the
+ *              blocks from the labels alone. */
+size_t morna_knn_batched_capped_workspace_bytes(int64_t n, int64_t nq, int32_t dim, int32_t k);
+int morna_knn_batched_capped(const float *vectors, const double *pp, const void *hs, int64_t ld_h, const float *rho_max,
+                             int64_t n, int32_t dim, int64_t ld, int32_t id_base, const double *queries, int64_t nq,
+                             int64_t q_ld, int32_t k, const int32_t *cap_group, int32_t max_per_group,
+                             const int64_t *block_ends, int32_t n_block_ends, const int32_t *row_group,
+                             const int32_t *query_group, int32_t *out_ids, double *out_dist,
+                             uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes, void *stream);
+
 /* Test hook: raw fp16 tensor-core scores [nq x n] (n <= 8192) and the per-query bound eps. */
 int morna_debug_tensor_scores(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
                               const double *queries, int64_t nq, int64_t q_ld, float *scores,

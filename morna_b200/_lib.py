@@ -112,6 +112,13 @@ _SIGNATURES = {
     "morna_range_exact_fill_excl": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64,
                                                    ctypes.c_double, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_sz, _c_vp, _c_vp, _c_vp]),
     "morna_merge_sorted_csr": (ctypes.c_int, [_c_vp, _c_i32, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp]),
+    "morna_cap_sorted_lists_workspace_bytes": (_c_sz, [_c_i64, _c_i64]),
+    "morna_cap_sorted_lists": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp, _c_i32, _c_i64, _c_i32, _c_i64,
+                                              _c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_sz, _c_vp]),
+    "morna_knn_batched_capped_workspace_bytes": (_c_sz, [_c_i64, _c_i64, _c_i32, _c_i32]),
+    "morna_knn_batched_capped": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp,
+                                                _c_i64, _c_i64, _c_i32, _c_vp, _c_i32, _c_vp, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp,
+                                                _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_tensor_scores": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_vp,
                                                  _c_i64, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_set_tuning": (ctypes.c_int, [_c_i32, _c_i32]),

@@ -221,10 +221,11 @@ class QueryFile(object):
         return out
 
 
-def search_query_file(search, path, k, exact=True, cap=None, query_labels=None):
+def search_query_file(search, path, k, exact=True, cap=None, query_labels=None, max_per_group=None):
     """Generator of (sample ids [b], ids [b x k], dists [b x k]) numpy arrays, batch by batch in query order.  The arrays
     are the caller's (search_batches' own are views of pinned buffers that the pipeline reuses two batches later).
-    `query_labels(sample_ids)` -> int32 labels: per-query exclusion (exact only; the search's rows carry labels)."""
+    `query_labels(sample_ids)` -> int32 labels: per-query exclusion (exact only; the search's rows carry labels).
+    `max_per_group`: at most that many results per cap label (exact only; the search's rows carry cap labels)."""
     qf = QueryFile(search, path)
     for lo, hi in qf.slices(cap):
         vecs = qf.query_vectors(lo, hi)
@@ -232,7 +233,8 @@ def search_query_file(search, path, k, exact=True, cap=None, query_labels=None):
         if exact:
             groups = None if query_labels is None else \
                 (query_labels(qf.sample_ids[lo + b:min(hi, lo + b + BATCH_QUERIES)]) for b in starts)
-            results = search.search_batches((vecs[b:b + BATCH_QUERIES] for b in starts), k, query_groups=groups)
+            results = search.search_batches((vecs[b:b + BATCH_QUERIES] for b in starts), k, query_groups=groups,
+                                            max_per_group=max_per_group)
         else:
             results = (tuple(t.cpu().numpy() for t in search.approx_search_device(vecs[b:b + BATCH_QUERIES], k)) for b in starts)
         for b, (ids, d) in zip(starts, results):
@@ -247,18 +249,19 @@ def all_sample_ids(search):
     return np.arange(search.index_size, dtype=np.int64)
 
 
-def search_all_samples(search, k, inverse, exclude=False):
+def search_all_samples(search, k, inverse, exclude=False, max_per_group=None):
     """Every indexed sample by internal id (the stored rows as queries, as `search -q`), exactly; only ids cross PCIe.
     Yields (sample ids, ids, dists) numpy arrays as search_query_file does.  `exclude`: each query takes its row's label
     (the search's rows carry labels), so it leaves out its own sample and its group."""
     members = all_sample_ids(search)
     starts = range(0, len(members), BATCH_QUERIES)
     batches = (members[b:b + BATCH_QUERIES] for b in starts)
-    for b, (ids, d) in zip(starts, search.search_batches(batches, k, query_groups=True if exclude else None)):
+    for b, (ids, d) in zip(starts, search.search_batches(batches, k, query_groups=True if exclude else None,
+                                                         max_per_group=max_per_group)):
         yield inverse[members[b:b + ids.shape[0]]], ids.copy(), d.copy()
 
 
-def search_query_file_range(search, path, max_distance, cap=None, result_cap=None, query_labels=None):
+def search_query_file_range(search, path, max_distance, cap=None, result_cap=None, query_labels=None, max_per_group=None):
     """Range variant of search_query_file (always exact): every indexed sample within `max_distance` of each query.
     Yields (sample ids [b], offsets int64 [b+1], ids, dists) numpy CSR batches in query order; query j's list is
     ids/dists[offsets[j]:offsets[j+1]].  The lists of a 4096-query batch are counted first, and a batch whose lists
@@ -269,11 +272,12 @@ def search_query_file_range(search, path, max_distance, cap=None, result_cap=Non
         vecs = qf.query_vectors(lo, hi)
         for b in range(0, hi - lo, BATCH_QUERIES):
             groups = None if query_labels is None else query_labels(qf.sample_ids[lo + b:min(hi, lo + b + BATCH_QUERIES)])
-            for g0, g1, off, ids, d in search.range_search_groups(vecs[b:b + BATCH_QUERIES], max_distance, result_cap, groups):
+            for g0, g1, off, ids, d in search.range_search_groups(vecs[b:b + BATCH_QUERIES], max_distance, result_cap, groups,
+                                                                  max_per_group):
                 yield qf.sample_ids[lo + b + g0:lo + b + g1], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
 
 
-def search_all_samples_range(search, max_distance, inverse, result_cap=None, exclude=False):
+def search_all_samples_range(search, max_distance, inverse, result_cap=None, exclude=False, max_per_group=None):
     """Range variant of search_all_samples: the stored rows as queries, built on the device from their ids.  Yields
     (sample ids, offsets, ids, dists) numpy CSR batches as search_query_file_range does."""
     members = all_sample_ids(search)
@@ -290,7 +294,7 @@ def search_all_samples_range(search, max_distance, inverse, result_cap=None, exc
             q = search.vectors[rows, :search.dim].to(torch.float64).contiguous()
             if exclude:
                 groups = search.row_group[rows]
-        for g0, g1, off, ids, d in search.range_search_groups(q, max_distance, result_cap, groups):
+        for g0, g1, off, ids, d in search.range_search_groups(q, max_distance, result_cap, groups, max_per_group):
             yield inverse[batch[g0:g1]], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
 
 

@@ -126,6 +126,12 @@ def build_parser():
     search_parser.add_argument("--max-distance", metavar="<float>", type=float, required=False, default=None,
                                help="return every sample within this angular distance of the query (exact; -r N, if "
                                     "given, keeps the first N per query)")
+    search_parser.add_argument("--max-per-group", metavar="<int>", type=int, required=False, default=None,
+                               help="return at most this many samples of any one group (--groups) per query: the nearest "
+                                    "samples, skipping a sample once this many of its group are listed (exact only)")
+    search_parser.add_argument("--groups", metavar="<file>", type=str, required=False, default=None,
+                               help="the groups --max-per-group caps: a file of 'sample_id<TAB>group' lines, as for "
+                                    "--exclude-group; a sample not listed is a group of its own")
     junctions_parser = subs.add_parser("junctions", help="extracts the junctions of a query's nearest neighbors")
     add_search_parameters(junctions_parser)                      # morna.py:1023-1054
     junctions_parser.add_argument("-i", "--index", metavar="<idx>", type=str, required=True,
@@ -209,6 +215,60 @@ class Exclusion(object):
         return out
 
 
+def read_group_file(flag, path):
+    """A file of 'sample_id<TAB>group' lines -> {sample id: group number} (groups numbered densely in order of first
+    appearance; whitespace stripped, blank lines skipped).  Raises ValueError with the message for the user."""
+    group_of = {}
+    try:
+        with open(path) as fh:
+            lines = fh.read().splitlines()
+    except (OSError, UnicodeDecodeError) as exc:
+        raise ValueError("%s: cannot read %s: %s" % (flag, path, exc))
+    numbers, first_line = {}, {}
+    for number, line in enumerate(lines, 1):
+        text = line.strip()
+        if not text:
+            continue
+        fields = text.split("\t")
+        if len(fields) != 2 or not fields[1].strip():
+            raise ValueError("%s: line %d of %s is not 'sample_id<TAB>group': %r" % (flag, number, path, text))
+        try:
+            sample_id = int(fields[0].strip())
+        except ValueError:
+            raise ValueError("%s: line %d of %s does not start with an integer sample id: %r" % (flag, number, path, text))
+        g = numbers.setdefault(fields[1].strip(), len(numbers))
+        if group_of.setdefault(sample_id, g) != g:
+            raise ValueError("%s: sample id %d is listed with two different groups (lines %d and %d of %s)"
+                             % (flag, sample_id, first_line[sample_id], number, path))
+        first_line.setdefault(sample_id, number)
+    return group_of
+
+
+def cap_groups(args):
+    """--max-per-group N --groups FILE: (N, int32 cap label per internal id -- the group number of a listed sample, -1
+    for one not listed, which is never capped), or None without either flag.  Raises ValueError with the message for
+    the user when the flags, the query mode or the file are not usable (before any GPU work)."""
+    n, path = getattr(args, "max_per_group", None), getattr(args, "groups", None)
+    if n is None and path is None:
+        return None
+    if n is None:
+        raise ValueError("--groups needs --max-per-group")
+    if path is None:
+        raise ValueError("--max-per-group needs --groups")
+    if n < 1:
+        raise ValueError("--max-per-group must be at least 1")
+    if args.rawlist:
+        raise ValueError("-rl cannot be combined with --max-per-group")
+    if args.query_id is None and not args.all_samples and not args.exact and args.max_distance is None:
+        raise ValueError("--max-per-group needs -e or --max-distance: the approximate mode has no cap per group")
+    group_of = read_group_file("--groups", path)
+    from . import files
+    labels = np.full(files.read_stats(args.basename)[1], -1, dtype=np.int32)
+    for sample_id, iid in files.read_map(args.basename).items():
+        labels[iid] = group_of.get(sample_id, -1)
+    return n, labels
+
+
 def exclusion(args):
     """--exclude-self / --exclude-group: an Exclusion, or None without either flag.  Raises ValueError with the message
     for the user when the flags, the query mode or the file are not usable (before any GPU work)."""
@@ -223,42 +283,21 @@ def exclusion(args):
                          "from stdin has no sample id" % flag)
     if args.query_intropolis is not None and not args.exact:
         raise ValueError("%s with --query-intropolis needs -e: the approximate mode has no exclusion" % flag)
-    group_of = {}
-    if path is not None:
-        try:
-            with open(path) as fh:
-                lines = fh.read().splitlines()
-        except (OSError, UnicodeDecodeError) as exc:
-            raise ValueError("%s: cannot read %s: %s" % (flag, path, exc))
-        numbers, first_line = {}, {}
-        for number, line in enumerate(lines, 1):
-            text = line.strip()
-            if not text:
-                continue
-            fields = text.split("\t")
-            if len(fields) != 2 or not fields[1].strip():
-                raise ValueError("%s: line %d of %s is not 'sample_id<TAB>group': %r" % (flag, number, path, text))
-            try:
-                sample_id = int(fields[0].strip())
-            except ValueError:
-                raise ValueError("%s: line %d of %s does not start with an integer sample id: %r" % (flag, number, path, text))
-            g = numbers.setdefault(fields[1].strip(), len(numbers))
-            if group_of.setdefault(sample_id, g) != g:
-                raise ValueError("%s: sample id %d is listed with two different groups (lines %d and %d of %s)"
-                                 % (flag, sample_id, first_line[sample_id], number, path))
-            first_line.setdefault(sample_id, number)
+    group_of = read_group_file(flag, path) if path is not None else {}
     from . import files
     index_size = files.read_stats(args.basename)[1]
     return Exclusion(group_of, files.read_map(args.basename), index_size)
 
 
-def open_search(basename, keep, keep_parent_rows, excl=None):
+def open_search(basename, keep, keep_parent_rows, excl=None, cap=None):
     """The index's MornaSearch, or with `keep` (sample_filter's ids) a FilteredSearch over those samples; with `excl`
-    (an Exclusion) every row carries its label."""
+    (an Exclusion) every row carries its label, with `cap` (cap_groups' result) its cap label."""
     from .search import MornaSearch
     searcher = MornaSearch(basename=basename)
     if excl is not None:
         searcher.set_row_groups(excl.row_labels)
+    if cap is not None:
+        searcher.set_cap_groups(cap[1])
     return searcher if keep is None else searcher.subset(keep, keep_parent_rows)
 
 
@@ -293,26 +332,28 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     try:
         keep = sample_filter(args)
         excl = exclusion(args) if args.subparser_name == "search" else None
+        cap = cap_groups(args) if args.subparser_name == "search" else None
     except ValueError as exc:
         stderr.write(str(exc) + "\n")
         return 2
+    per_group = cap[0] if cap is not None else None
     if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
-        return batch_search(args, stdout, stderr, max_distance, limit, keep, excl)
+        return batch_search(args, stdout, stderr, max_distance, limit, keep, excl, cap)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
         stdin = opened = open(args.pass1_sam)
     # (a filter keeps the whole index's rows only for -q, whose sample may lie outside the subset)
-    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None, excl=excl)
+    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None, excl=excl, cap=cap)
     if args.query_id is not None:                               # morna.py:1358-1365
         if max_distance is not None:
             results = searcher.search_member_n(args.query_id, limit, include_distances=args.distances,
                                                meta_db=args.metadata, out=stdout, max_distance=max_distance,
-                                               exclude=excl is not None)
+                                               exclude=excl is not None, max_per_group=per_group)
         else:
             results = searcher.search_member_n(args.query_id, args.results, args.search_k,
                                                include_distances=args.distances, meta_db=args.metadata, out=stdout,
-                                               exclude=excl is not None)
+                                               exclude=excl is not None, max_per_group=per_group)
         results_output(results, stdout)
         return 0
     if args.format == "sam":                                    # :1367-1373
@@ -337,9 +378,10 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
         stderr.write("\n")
     if max_distance is not None:                                # always exact: -e changes nothing
         results = searcher.range_search_nn(max_distance, include_distances=args.distances, meta_db=args.metadata,
-                                           num_neighbors=limit)
+                                           num_neighbors=limit, max_per_group=per_group)
     elif args.exact:                                            # :1477-1483
-        results = searcher.exact_search_nn(args.results, include_distances=args.distances, meta_db=args.metadata)
+        results = searcher.exact_search_nn(args.results, include_distances=args.distances, meta_db=args.metadata,
+                                           max_per_group=per_group)
     else:
         results = searcher.search_nn(args.results, args.search_k, include_distances=args.distances, meta_db=args.metadata)
     results_output(results, stdout)
@@ -350,11 +392,11 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     return 0
 
 
-def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None, excl=None):
+def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None, excl=None, cap=None):
     """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches.  With
     `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given.  With
     `keep` (sample_filter's ids), the search runs over those samples only.  With `excl` (an Exclusion), each query
-    leaves out the samples of its group."""
+    leaves out the samples of its group.  With `cap` (cap_groups' result), at most N samples per group."""
     from . import batch_query
     named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
                                    ("--all-samples", args.all_samples), ("-q", args.query_id is not None),
@@ -363,25 +405,27 @@ def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None,
         stderr.write("%s cannot be combined with %s\n" % (named[0], ", ".join(named[1:])))
         return 2
     # (with an exclusion, --all-samples over a subset takes its labels from the whole index's rows)
-    searcher = open_search(args.basename, keep, keep_parent_rows=False, excl=excl)
+    searcher = open_search(args.basename, keep, keep_parent_rows=False, excl=excl, cap=cap)
+    per_group = cap[0] if cap is not None else None
     inverse = batch_query.inverse_map(searcher)
     meta = args.basename if args.metadata else None
     exclude = excl is not None
     query_labels = excl.labels_of_samples if exclude else None
     if max_distance is not None:
         if args.all_samples:
-            results = batch_query.search_all_samples_range(searcher, max_distance, inverse, exclude=exclude)
+            results = batch_query.search_all_samples_range(searcher, max_distance, inverse, exclude=exclude,
+                                                           max_per_group=per_group)
         else:
             results = batch_query.search_query_file_range(searcher, args.query_intropolis, max_distance,
-                                                          query_labels=query_labels)
+                                                          query_labels=query_labels, max_per_group=per_group)
         for sample_ids, offsets, ids, dists in results:
             batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse, offsets=offsets, limit=limit)
         return 0
     if args.all_samples:                       # the stored rows as queries: exact, as -q is
-        results = batch_query.search_all_samples(searcher, args.results, inverse, exclude=exclude)
+        results = batch_query.search_all_samples(searcher, args.results, inverse, exclude=exclude, max_per_group=per_group)
     else:
         results = batch_query.search_query_file(searcher, args.query_intropolis, args.results, exact=args.exact,
-                                                query_labels=query_labels)
+                                                query_labels=query_labels, max_per_group=per_group)
     for sample_ids, ids, dists in results:
         batch_query.write_results(stdout, sample_ids, ids, dists, args.distances, meta, inverse)
     return 0

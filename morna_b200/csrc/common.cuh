@@ -95,4 +95,34 @@ int launch_mask_excluded(double *dist, int64_t n, int64_t dist_ld, int64_t nq, c
                          const int32_t *query_group, cudaStream_t s);
 int launch_pad_masked(int32_t *ids, const double *dist, int64_t total, cudaStream_t s);
 
+// Parameters of the selection passes between the GEMM launches of the batched path (kth_warp_kernel, search_batched.cu,
+// and its group-capped counterpart cap_select_kernel, search_capped.cu)
+struct KthParams {
+    int32_t k, n0, n_begin, id_base, cap, fcap;
+    const float *pilot; int64_t pilot_ld;
+    const float *eps;
+    float *thr;
+    float *cand_score; int32_t *cand_id; int32_t *cand_cnt;
+    float *cand2_score; int32_t *cand2_id;        // refine mode: the compacted list goes here
+    int32_t *fin_id; int32_t *fin_cnt;
+    uint8_t *overflow; int32_t *stats;
+    float *kth_bound;                             // modes 3 / 4: per-query lower bound of the k-th best true cosine
+    // modes 0-2, per-query exclusion (nullptr = off): the row behind entry idx (pilot: row n_begin + idx; lists:
+    // cand_id[idx] - id_base) is absent for query q iff query_group[q] >= 0 && row_group[row] == query_group[q]
+    const int32_t *row_group; const int32_t *query_group;
+};
+
+// Group-capped search (search_capped.cu): the passes that take the place of kth_warp_kernel modes 1 (pilot), 2 (refine)
+// and 0 (final) when every row of the call carries a cap label (cap_group; < 0: ungrouped) and at most max_per_group rows
+// of a label may be returned
+int launch_cap_select(int mode, const KthParams &p, const int32_t *cap_group, int32_t max_per_group, int64_t nq,
+                      cudaStream_t s);
+
+// The walk of morna_cap_sorted_lists on fixed-stride lists (list j = entries [j * in_ld, (j + 1) * in_ld), at most
+// kCapWalkChunk long), written padded to [n_lists x out_ld]: the last step of the capped tensor-core route.
+constexpr int kCapWalkChunk = 1024;
+int launch_cap_walk_strided(const int32_t *ids, const double *dists, int64_t n_lists, int64_t in_ld, const int32_t *cap_group,
+                            int32_t id_base, int64_t n_rows, int32_t max_per_group, int64_t limit, int32_t *out_ids,
+                            double *out_dists, int64_t out_ld, cudaStream_t s);
+
 }  // namespace morna

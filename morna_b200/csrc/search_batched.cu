@@ -997,20 +997,6 @@ __device__ __forceinline__ float key_float(uint32_t k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
-struct KthParams {
-    int32_t k, n0, n_begin, id_base, cap, fcap;
-    const float *pilot; int64_t pilot_ld;
-    const float *eps;
-    float *thr;
-    float *cand_score; int32_t *cand_id; int32_t *cand_cnt;
-    float *cand2_score; int32_t *cand2_id;        // refine mode: the compacted list goes here
-    int32_t *fin_id; int32_t *fin_cnt;
-    uint8_t *overflow; int32_t *stats;
-    float *kth_bound;                             // modes 3 / 4: per-query lower bound of the k-th best true cosine
-    // modes 0-2, per-query exclusion (nullptr = off): the row behind entry idx (pilot: row n_begin + idx; lists:
-    // cand_id[idx] - id_base) is absent for query q iff query_group[q] >= 0 && row_group[row] == query_group[q]
-    const int32_t *row_group; const int32_t *query_group;
-};
 
 // key of the kk-th largest of the keys one warp holds in registers (kItems per lane; 0 = padding)
 template <int kItems>
@@ -1452,7 +1438,9 @@ struct BatchWs {
     size_t hq, qq, eps, pilot, thr, cand_score, cand_id, cand2_score, cand2_id, cand_cnt, fin_id, fin_cnt, fin_dist, queue, total;
     int64_t nq_pad, n0, pilot_ld;
 };
-static BatchWs batch_ws_layout(int64_t n, int64_t nq, int64_t ld_h) {
+// refine_lists: the second list buffers even when one row block is scored (a capped search refines between its lead
+// blocks); they then go last, so every other offset is the same as without
+static BatchWs batch_ws_layout(int64_t n, int64_t nq, int64_t ld_h, bool refine_lists = false) {
     BatchWs w{};
     w.nq_pad = (nq + 2 * gemm::BM - 1) / (2 * gemm::BM) * (2 * gemm::BM);      // CTA pairs own 256 query rows
     w.n0 = n < g_pilot_rows ? n : g_pilot_rows;
@@ -1476,6 +1464,10 @@ static BatchWs batch_ws_layout(int64_t n, int64_t nq, int64_t ld_h) {
     w.fin_cnt = take((size_t)nq * sizeof(int32_t));
     w.fin_dist = take((size_t)nq * kFinCap * sizeof(double));
     w.queue = take(sizeof(unsigned long long));
+    if (refine_lists && !w.cand2_score) {
+        w.cand2_score = take((size_t)nq * kCandCap * sizeof(float));
+        w.cand2_id = take((size_t)nq * kCandCap * sizeof(int32_t));
+    }
     w.total = off + 1024;
     return w;
 }
@@ -1515,16 +1507,21 @@ extern "C" size_t morna_knn_batched_workspace_bytes(int64_t n, int64_t nq, int32
 // Scoring half of morna_knn_batched: fp16 tensor-core scores, thresholds and the final candidate
 // lists of every query, left in the workspace (tensor-core bound; touches HBM lightly).
 // final_mode: 0 = final candidate lists, 1 = this rank's score bounds only (kth_bound), 2 = leave the first-pass lists
+// cap_group (with max_per_group >= 1, final_mode 0 only): a group-capped search -- the selection passes are
+// cap_select_kernel's (search_capped.cu) in place of kth_warp_kernel's, and the blocks after the pilot end at the
+// host-given cap_ends (ascending; ends at or below the pilot are skipped) before the usual blocks take over
 static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
                       int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
                       uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes,
                       void *const *phase_events, const morna_rerank_job *side_job, float *kth_bound, int final_mode,
-                      const int32_t *row_group, const int32_t *query_group, void *stream) {
+                      const int32_t *row_group, const int32_t *query_group, void *stream,
+                      const int32_t *cap_group = nullptr, int32_t max_per_group = 0, const int64_t *cap_ends = nullptr,
+                      int32_t n_cap_ends = 0) {
     if (!hs || !rho_max || !queries || !overflow || !stats || n <= 0 || n > kBatchedMaxRows || nq <= 0 || dim <= 0 ||
         q_ld < dim || k <= 0 || k > kFinCap / 2 || ld_h != morna_tensor_operand_ld(dim) || !row_group != !query_group ||
-        (row_group && final_mode == 1))
+        (row_group && final_mode == 1) || (cap_group && (final_mode != 0 || max_per_group < 1)))
         return MORNA_ERR_INVALID_ARGUMENT;
-    BatchWs w = batch_ws_layout(n, nq, ld_h);
+    BatchWs w = batch_ws_layout(n, nq, ld_h, cap_group != nullptr);
     if (!workspace || workspace_bytes < w.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
     RerankParams side{};
     const RerankParams *side_ptr = nullptr;
@@ -1594,22 +1591,36 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
     if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<0>, kKwSmem)) != MORNA_OK) return rc;
     if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<2>, kKwSmem)) != MORNA_OK) return rc;
     const unsigned kth_grid = (unsigned)((nq + kKwWarps - 1) / kKwWarps);
+    auto capped_select = [&](int mode) -> int { return launch_cap_select(mode, kp, cap_group, max_per_group, nq, s); };
 
     rc = launch_gemm(0, (int32_t)w.n0, 0);                       // pilot block: dump scores
     if (rc != MORNA_OK) return rc;
     mark();                                                      // 2: pilot GEMM
-    kth_warp_kernel<1><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
-    MORNA_LAUNCH_CHECK();
+    if (cap_group) {
+        if ((rc = capped_select(1)) != MORNA_OK) return rc;
+    } else {
+        kth_warp_kernel<1><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
+        MORNA_LAUNCH_CHECK();
+    }
     mark();                                                      // 3: thresholds
     // the rest in blocks of g_block_rows rows: keep scores above thr; between blocks thr is tightened to the
     // k-th best seen so far and the lists are compacted, so a later block adds ~k entries per query, not ~N/n0 * k
     // (key 36 lets the blocks grow geometrically: after the first refinement a query's threshold passes ~k/rows_seen of the
     // rows, so a block as large as everything seen so far adds about k entries to its list; off by default)
     int64_t step = g_block_rows;
+    // (a capped search: while the rows scored so far hold few capped entries its thresholds are weak or absent and the
+    // filter appends most rows it scores, so the host sizes the blocks from the labels; see morna_knn_batched_capped)
+    int ci = 0;
+    if (cap_group) while (ci < n_cap_ends && cap_ends[ci] <= w.n0) ++ci;
     for (int64_t b0 = w.n0; b0 < n;) {
-        int64_t b1 = b0 == w.n0 ? (int64_t)(g_first_block > 0 ? g_first_block : g_block_rows) : b0 + step;
-        if (b0 != w.n0 && g_block_growth > 1) step *= g_block_growth;
-        if (b1 <= b0) b1 = b0 + step;      // key 11 (or key 9) at or below the pilot rows: the first block is `step` rows, not the rest
+        int64_t b1;
+        if (cap_group && ci < n_cap_ends) {
+            b1 = cap_ends[ci++];
+        } else {
+            b1 = b0 == w.n0 ? (int64_t)(g_first_block > 0 ? g_first_block : g_block_rows) : b0 + step;
+            if (b0 != w.n0 && g_block_growth > 1) step *= g_block_growth;
+            if (b1 <= b0) b1 = b0 + step;  // key 11 (or key 9) at or below the pilot rows: the first block is `step` rows, not the rest
+        }
         if (b1 > n) b1 = n;
         rc = launch_gemm((int32_t)b0, (int32_t)b1, 1);
         if (rc != MORNA_OK) return rc;
@@ -1617,8 +1628,12 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
         if (b0 < n) {
             kp.cand2_score = (float *)(ws + w.cand2_score);
             kp.cand2_id = (int32_t *)(ws + w.cand2_id);
-            kth_warp_kernel<2><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
-            MORNA_LAUNCH_CHECK();
+            if (cap_group) {
+                if ((rc = capped_select(2)) != MORNA_OK) return rc;
+            } else {
+                kth_warp_kernel<2><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
+                MORNA_LAUNCH_CHECK();
+            }
             // the compacted lists are now the current ones
             float *ts = kp.cand_score; kp.cand_score = kp.cand2_score; kp.cand2_score = ts;
             int32_t *ti = kp.cand_id; kp.cand_id = kp.cand2_id; kp.cand2_id = ti;
@@ -1633,10 +1648,13 @@ static int score_impl(const void *hs, int64_t ld_h, const float *rho_max, int64_
         kp.kth_bound = kth_bound;
         if ((rc = ensure_dynamic_smem((const void *)kth_warp_kernel<3>, kKwSmem)) != MORNA_OK) return rc;
         kth_warp_kernel<3><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
+        MORNA_LAUNCH_CHECK();
+    } else if (cap_group) {
+        if ((rc = capped_select(0)) != MORNA_OK) return rc;
     } else {
         kth_warp_kernel<0><<<kth_grid, kKwWarps * 32, kKwSmem, s>>>(kp, (int)nq);
+        MORNA_LAUNCH_CHECK();
     }
-    MORNA_LAUNCH_CHECK();
     mark();                                                      // 5: final candidate lists
     return MORNA_OK;
 }
@@ -1872,10 +1890,12 @@ static int make_rerank_params(RerankParams &rp, bool &warp_kernel, const float *
 // in the same workspace, ordered under the reference rule (HBM/L2-gather bound; no tensor cores).
 // resume != 0: a later morna_knn_batched_score call carried this batch as its side job -- only what its
 // helper warps left in the queue is re-ranked here.
-extern "C" int morna_knn_batched_rerank(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
-                                        int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
-                                        int32_t *out_ids, double *out_dist, const uint8_t *overflow, void *workspace,
-                                        size_t workspace_bytes, int32_t resume, void *stream) {
+namespace morna {
+// out_k: entries of each sorted list written out ([nq x out_k]): k for a top-k search, kFinCap for the capped route's walk
+static int rerank_impl(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                       const double *queries, int64_t nq, int64_t q_ld, int32_t k, int32_t out_k, int32_t *out_ids,
+                       double *out_dist, const uint8_t *overflow, void *workspace, size_t workspace_bytes, int32_t resume,
+                       void *stream) {
     if (!out_ids || !out_dist) return MORNA_ERR_INVALID_ARGUMENT;
     RerankParams rp;
     bool warp_kernel = true;
@@ -1931,10 +1951,19 @@ extern "C" int morna_knn_batched_rerank(const float *vectors, const double *pp, 
         MORNA_LAUNCH_CHECK();
     }
     const size_t or_smem = (size_t)kFinCap * (sizeof(double) + sizeof(int));
-    rerank_order_kernel<<<(unsigned)nq, kOrderThreads, or_smem, s>>>(rp.fin_id, rp.fin_cnt, rp.fin_dist, overflow, kFinCap, k,
+    rerank_order_kernel<<<(unsigned)nq, kOrderThreads, or_smem, s>>>(rp.fin_id, rp.fin_cnt, rp.fin_dist, overflow, kFinCap, out_k,
                                                                     out_ids, out_dist);
     MORNA_LAUNCH_CHECK();
     return MORNA_OK;
+}
+}  // namespace morna
+
+extern "C" int morna_knn_batched_rerank(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                                        int32_t id_base, const double *queries, int64_t nq, int64_t q_ld, int32_t k,
+                                        int32_t *out_ids, double *out_dist, const uint8_t *overflow, void *workspace,
+                                        size_t workspace_bytes, int32_t resume, void *stream) {
+    return rerank_impl(vectors, pp, n, dim, ld, id_base, queries, nq, q_ld, k, k, out_ids, out_dist, overflow, workspace,
+                       workspace_bytes, resume, stream);
 }
 
 extern "C" int morna_knn_batched(const float *vectors, const double *pp, const void *hs, int64_t ld_h,
@@ -1950,6 +1979,55 @@ extern "C" int morna_knn_batched(const float *vectors, const double *pp, const v
                                   workspace, workspace_bytes, 0, stream);
     if (rc == MORNA_OK && phase_events) cudaEventRecord((cudaEvent_t)phase_events[6], (cudaStream_t)stream);
     return rc;
+}
+
+// Group-capped search on the tensor cores: the scoring half with cap_select_kernel's passes, the usual FP64 re-rank of
+// the final lists sorted whole (kFinCap entries per query, into the workspace after the batched layout), then the walk.
+namespace morna {
+struct CappedWs { size_t sorted_ids, sorted_dist, total; };
+static CappedWs capped_ws_layout(int64_t n, int64_t nq, int32_t dim) {
+    CappedWs c{};
+    size_t off = align_up(batch_ws_layout(n, nq, morna_tensor_operand_ld(dim), true).total, 256);
+    c.sorted_ids = off; off += align_up((size_t)nq * kFinCap * sizeof(int32_t), 256);
+    c.sorted_dist = off; off += (size_t)nq * kFinCap * sizeof(double);
+    c.total = off;
+    return c;
+}
+}  // namespace morna
+
+extern "C" size_t morna_knn_batched_capped_workspace_bytes(int64_t n, int64_t nq, int32_t dim, int32_t k) {
+    (void)k;
+    if (n <= 0 || nq <= 0 || dim <= 0) return 1024;
+    return capped_ws_layout(n, nq, dim).total;
+}
+
+extern "C" int morna_knn_batched_capped(const float *vectors, const double *pp, const void *hs, int64_t ld_h,
+                                        const float *rho_max, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                                        const double *queries, int64_t nq, int64_t q_ld, int32_t k, const int32_t *cap_group,
+                                        int32_t max_per_group, const int64_t *block_ends, int32_t n_block_ends,
+                                        const int32_t *row_group, const int32_t *query_group,
+                                        int32_t *out_ids, double *out_dist, uint8_t *overflow, int32_t *stats,
+                                        void *workspace, size_t workspace_bytes, void *stream) {
+    if (!vectors || !pp || !out_ids || !out_dist || !cap_group || max_per_group < 1 || n_block_ends < 0 ||
+        (n_block_ends > 0 && !block_ends) || ld < dim || (ld & 3) || nq <= 0 ||
+        dim <= 0)
+        return MORNA_ERR_INVALID_ARGUMENT;
+    for (int32_t i = 0; i < n_block_ends; ++i)
+        if (block_ends[i] <= (i ? block_ends[i - 1] : 0)) return MORNA_ERR_INVALID_ARGUMENT;
+    const CappedWs c = capped_ws_layout(n, nq, dim);
+    if (!workspace || workspace_bytes < c.total) return MORNA_ERR_WORKSPACE_TOO_SMALL;
+    int rc = score_impl(hs, ld_h, rho_max, n, dim, id_base, queries, nq, q_ld, k, overflow, stats, workspace, workspace_bytes,
+                        nullptr, nullptr, nullptr, 0, row_group, query_group, stream, cap_group, max_per_group, block_ends,
+                        n_block_ends);
+    if (rc != MORNA_OK) return rc;
+    unsigned char *ws = (unsigned char *)workspace;
+    int32_t *sorted_ids = (int32_t *)(ws + c.sorted_ids);
+    double *sorted_dist = (double *)(ws + c.sorted_dist);
+    rc = rerank_impl(vectors, pp, n, dim, ld, id_base, queries, nq, q_ld, k, kFinCap, sorted_ids, sorted_dist, overflow,
+                     workspace, workspace_bytes, 0, stream);
+    if (rc != MORNA_OK) return rc;
+    return launch_cap_walk_strided(sorted_ids, sorted_dist, nq, kFinCap, cap_group, id_base, n, max_per_group, k, out_ids,
+                                   out_dist, k, (cudaStream_t)stream);
 }
 
 // Raw fp16 tensor-core scores of a query block against the first n0 samples, plus the

@@ -359,20 +359,175 @@ class MornaSearch(object):
         """The (row_group, query_group) pointers an *_excl entry point takes."""
         return (_lib.dev_ptr(self.row_group[rows]), _lib.dev_ptr(qg))
 
+    cap_group = None                 # device int32 [n]: cap label of every resident row (set_cap_groups), or None
+
+    def set_cap_groups(self, labels):
+        """Labels for group-capped search: int32 [n], one per resident row (None clears them); a label < 0 leaves the row
+        ungrouped (a group of its own, never capped).  A search given ``max_per_group=N`` then returns, per query, the
+        nearest rows with at most N rows of any one label.  Independent of set_row_groups: "leave out my own study, at
+        most N per other study" takes both."""
+        self._cap_prefix = {}
+        if labels is None:
+            self.cap_group = None
+            return
+        t = torch.as_tensor(labels).to(device=self.device, dtype=torch.int32).contiguous()
+        if t.shape != (self.row_hi - self.row_lo,):
+            raise ValueError("cap labels must be one per resident row (%d), got shape %r" % (self.row_hi - self.row_lo, tuple(t.shape)))
+        self.cap_group = t
+
+    CAP_BLOCK = 2048                 # rows a capped block may add to a candidate list (of 4096) above a weak threshold
+
+    def _cap_blocks(self, m, k):
+        """Block ends (host int64) for the capped tensor route (morna_knn_batched_capped's block_ends), from the labels
+        alone.  c(b), the capped entries the first b rows hold (a label counted at most m times, an ungrouped row once),
+        bounds how selective a threshold after b rows can be: below k + m there may be none (the extra m covers a query
+        that excludes one group), and above it about k + m of c(b) representatives pass, so a block of
+        CAP_BLOCK * c(b) / (k + m) rows adds about CAP_BLOCK entries.  Ends are multiples of CAP_BLOCK while below that,
+        so that any pilot size that is a multiple of it lands on one; the usual blocks take over at BATCH_BLOCK_ROWS ...
+        131072 rows per block.  Cached per (m, k)."""
+        cache = self.__dict__.setdefault("_cap_prefix", {})
+        if (m, k) in cache:
+            return cache[(m, k)]
+        counts = cache.get(m)
+        if counts is None:
+            g = self.cap_group.long()
+            n = g.numel()
+            order = torch.sort(g, stable=True).indices
+            sg = g[order]
+            head = torch.ones(n, dtype=torch.bool, device=g.device)
+            head[1:] = sg[1:] != sg[:-1]
+            pos = torch.arange(n, device=g.device)
+            rank = torch.empty_like(pos)
+            rank[order] = pos - torch.cummax(torch.where(head, pos, torch.zeros_like(pos)), 0).values
+            counts = cache[m] = ((g < 0) | (rank < m)).to(torch.int64).cumsum(0).cpu().numpy()
+        n, need, ends, b = counts.size, k + m, [], 0
+        while b < n:
+            c = int(counts[b - 1]) if b else 0
+            step = self.CAP_BLOCK if c < need else min(131072, max(self.CAP_BLOCK, self.CAP_BLOCK * c // need))
+            b = min(n, b + step)
+            ends.append(b)
+            if step == 131072:
+                break
+        cache[(m, k)] = out = np.array(ends, dtype=np.int64)
+        return out
+
+    def _cap(self, max_per_group):
+        """max_per_group as an int >= 1, or None for an uncapped search."""
+        if max_per_group is None:
+            return None
+        if isinstance(max_per_group, bool) or int(max_per_group) != max_per_group or max_per_group < 1:
+            raise ValueError("max_per_group must be an integer >= 1, got %r" % (max_per_group,))
+        if self.cap_group is None:
+            raise ValueError("max_per_group needs cap labels: call set_cap_groups first")
+        return int(max_per_group)
+
+    def cap_sorted_lists(self, offsets, ids, dists, max_per_group, limit=None, out=None):
+        """The walk of a capped search (morna_cap_sorted_lists) over device lists already in the reference order: offsets
+        int64 [L+1], ids int32 (global; -1 is padding), dists float64.  Each entry is kept iff fewer than max_per_group
+        entries of its cap label were kept before it in its list, and at most ``limit`` per list (None: no limit).  Returns
+        the capped CSR (offsets, ids, dists), or with ``out`` = (ids [L x w], dists [L x w]) fills those, padded."""
+        L, total = offsets.numel() - 1, ids.numel()
+        dev = self.device
+        lim = -1 if limit is None else max(int(limit), 0)
+        with torch.cuda.device(dev):
+            ws = self._workspace(self.lib.morna_cap_sorted_lists_workspace_bytes(L, total), "cap_walk")
+            args = (_lib.dev_ptr(offsets), L, _lib.ptr(ids), _lib.ptr(dists), total, _lib.dev_ptr(self.cap_group),
+                    self.row_lo, self.row_hi - self.row_lo, max_per_group, lim)
+            if out is not None:
+                _lib.check(self.lib.morna_cap_sorted_lists(*args, None, _lib.ptr(out[0]), _lib.ptr(out[1]), out[0].shape[1],
+                                                           _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_cap_sorted_lists")
+                return out
+            out_off = torch.empty(L + 1, dtype=torch.int64, device=dev)
+            out_ids = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+            out_d = torch.empty(max(total, 1), dtype=torch.float64, device=dev)
+            _lib.check(self.lib.morna_cap_sorted_lists(*args, _lib.dev_ptr(out_off), _lib.dev_ptr(out_ids), _lib.dev_ptr(out_d), 0,
+                                                       _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_cap_sorted_lists")
+            kept = int(out_off[-1].item())
+            return out_off, out_ids[:kept], out_d[:kept]
+
+    CAPPED_SORT_ENTRIES = 1 << 24    # distances sorted at once by the capped FP64 route (queries x rows)
+
+    def _capped_search(self, queries, k, qg, m):
+        """Top-k with at most m rows per cap label (see set_cap_groups): the tensor-core route (morna_knn_batched_capped)
+        for a dense index of one row block and k <= 512, its overflowed queries and everything else by the FP64 route."""
+        nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
+        k = max(int(k), 0)
+        if n == 0 or nq == 0 or k == 0:
+            return (torch.full((nq, k), -1, dtype=torch.int32, device=dev),
+                    torch.full((nq, k), float("inf"), dtype=torch.float64, device=dev))
+        if k > 512 or n > self.BATCH_BLOCK_ROWS or (self.csr is not None and self.sparse_exact):
+            return self._capped_full_sort(queries, k, qg, m)
+        self.enable_tensor_path()
+        with torch.cuda.device(dev):
+            out_ids = torch.empty((nq, k), dtype=torch.int32, device=dev)
+            out_d = torch.empty((nq, k), dtype=torch.float64, device=dev)
+            overflow = torch.empty(nq, dtype=torch.uint8, device=dev)
+            stats = torch.empty(4, dtype=torch.int32, device=dev)
+            ws = self._workspace(self.lib.morna_knn_batched_capped_workspace_bytes(n, nq, self.dim, k), "capped")
+            excl = (None, None) if qg is None else self._excl_args(qg)
+            blocks = self._cap_blocks(m, k)
+            _lib.check(self.lib.morna_knn_batched_capped(
+                _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), _lib.dev_ptr(self.hs), self.ld_h, _lib.dev_ptr(self.rho_max),
+                n, self.dim, self.ld, self.row_lo, _lib.ptr(queries), nq, self.dim, k, _lib.dev_ptr(self.cap_group), m,
+                blocks.ctypes.data_as(ctypes.c_void_p), blocks.size, *excl,
+                _lib.dev_ptr(out_ids), _lib.dev_ptr(out_d), _lib.dev_ptr(overflow), _lib.dev_ptr(stats), _lib.dev_ptr(ws),
+                ws.numel(), _lib.stream_ptr()), "morna_knn_batched_capped")
+            st = stats.cpu()
+            self.last_stats = st.to(torch.int64).tolist()
+            if int(st[0]) > 0:
+                idx = overflow.nonzero().flatten()
+                e_ids, e_d = self._capped_full_sort(queries[idx], k, None if qg is None else qg[idx], m)
+                out_ids[idx] = e_ids
+                out_d[idx] = e_d
+        return out_ids, out_d
+
+    def _capped_full_sort(self, queries, k, qg, m):
+        """The capped FP64 route: every row's canonical FP64 distance (morna_angular_distances), excluded pairs at +inf, a
+        full sort per query under the reference order (torch's; rare), then the walk.  Any k, any number of rows."""
+        nq, n, dev = queries.shape[0], self.row_hi - self.row_lo, self.device
+        out_ids = torch.full((nq, k), -1, dtype=torch.int32, device=dev)
+        out_d = torch.full((nq, k), float("inf"), dtype=torch.float64, device=dev)
+        if n == 0 or nq == 0 or k == 0:
+            return out_ids, out_d
+        per = max(1, self.CAPPED_SORT_ENTRIES // n)
+        with torch.cuda.device(dev):
+            for j0 in range(0, nq, per):
+                q = queries[j0:j0 + per].contiguous()
+                b = q.shape[0]
+                dist = torch.empty((b, n), dtype=torch.float64, device=dev)
+                _lib.check(self.lib.morna_angular_distances(
+                    _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.ptr(q), b, self.dim,
+                    _lib.dev_ptr(dist), n, _lib.stream_ptr()), "morna_angular_distances")
+                if qg is not None:
+                    g = qg[j0:j0 + b, None]
+                    dist.masked_fill_((self.row_group[None, :] == g) & (g >= 0), float("inf"))
+                # distance ascending, equal distances id descending: stable sort of the id-reversed rows
+                rows = (n - 1) - torch.sort(dist.flip(1), dim=1, stable=True).indices
+                d = dist.gather(1, rows)
+                del dist
+                ids = torch.where(torch.isinf(d), -1, rows + self.row_lo).to(torch.int32)
+                del rows
+                offsets = torch.arange(b + 1, dtype=torch.int64, device=dev) * n
+                self.cap_sorted_lists(offsets, ids, d, m, k, out=(out_ids[j0:j0 + b], out_d[j0:j0 + b]))
+        return out_ids, out_d
+
     MAX_SELECT_K = 2048              # kSelMaxK of morna_select_topk
     sparse_exact = False             # set at load for a sparse index whose tie groups would overflow the tensor path's lists
     TIE_GROUP_FOR_SPARSE_PATH = 512  # (the final candidate lists hold 1024 rows; a query usually sees two or more such groups)
 
-    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None):
+    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None, max_per_group=None):
         """queries: CUDA float64 [nq x dim].  Returns device (ids int32 [nq x k], dists float64 [nq x k]); ids are
         global internal ids (row_lo + local row); short lists are padded with id -1 / +inf.  Like the reference's
         exact_search_nn (morna.py:681-712) any k is served: k above the number of rows returns every row, k <= 0
         an empty list.  ``query_groups`` (int32 [nq], see set_row_groups): query q leaves out the rows labelled
-        query_groups[q]; the lists are the brute-force lists of the remaining rows."""
+        query_groups[q]; the lists are the brute-force lists of the remaining rows.  ``max_per_group`` (see
+        set_cap_groups): the brute-force list walked in order, a row kept iff fewer than that many rows of its cap label
+        were kept before it, until k are kept."""
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2
         if stream is not None and stream != torch.cuda.current_stream(self.device):
             with torch.cuda.stream(stream):
-                return self.exact_search_device(queries, k, allow_single=allow_single, query_groups=query_groups)
+                return self.exact_search_device(queries, k, allow_single=allow_single, query_groups=query_groups,
+                                                max_per_group=max_per_group)
         queries = queries.contiguous()
         nq = queries.shape[0]
         q_ld = queries.shape[1]            # (a size-1 leading dimension may report stride 0)
@@ -384,8 +539,11 @@ class MornaSearch(object):
         out_d = torch.full((nq, k), float("inf"), dtype=torch.float64, device=dev)
         k_eff = min(k, n)
         qg = self._query_groups(query_groups, nq)
+        m = self._cap(max_per_group)
         if n == 0 or nq == 0 or k_eff == 0:
             return out_ids, out_d
+        if m is not None:
+            return self._capped_search(queries, k, qg, m)
         if nq == 1 and allow_single and k_eff <= 512 and self.csr is None and qg is None:
             return self.single_search_device(queries[0], k)
         excl = () if qg is None else self._excl_args(qg)
@@ -524,11 +682,13 @@ class MornaSearch(object):
             return parts[0][2], parts[0][3]
         return mdist.merge_topk(torch.cat([p[2] for p in parts], 1), torch.cat([p[3] for p in parts], 1), k, stream)
 
-    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None):
+    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None,
+                              max_per_group=None):
         """Same contract and same results as exact_search_device, with the N x D
         contraction on the tensor cores (fp16 first pass with a rigorous error bound,
         FP64 re-rank).  Queries whose candidate lists overflow (massive ties) are
-        answered by the exact scan.  ``query_groups``: per-query exclusion, as in exact_search_device."""
+        answered by the exact scan.  ``query_groups``: per-query exclusion, as in exact_search_device.
+        ``max_per_group``: a group-capped search, as in exact_search_device (one call at a time, no phase events)."""
         from . import dist as mdist
         self.enable_tensor_path()
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2
@@ -537,6 +697,10 @@ class MornaSearch(object):
         n = self.row_hi - self.row_lo
         assert queries.shape[1] == self.dim
         qg = self._query_groups(query_groups, nq)
+        m = self._cap(max_per_group)
+        if m is not None:
+            with torch.cuda.stream(stream if stream is not None else torch.cuda.current_stream(self.device)):
+                return self._capped_search(queries, k, qg, m)
         if n == 0 or nq == 0 or k > 512 or k <= 0 or k > n or (self.csr is not None and self.sparse_exact):
             return self.exact_search_device(queries, k, stream, query_groups=qg)   # (a sparse index: its ties would overflow every list)
         parts = self._batched_launch(queries, k, stream, phase_events, qg)
@@ -619,7 +783,7 @@ class MornaSearch(object):
             return self._batched_finish(parts, queries, k)
         return out_ids, out_d
 
-    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None):
+    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None, max_per_group=None):
         """Streams query batches through the GPU: generator over ``batches`` (each a numpy or torch
         [nq x dim] float32/float64 array, or a 1-D integer array of INTERNAL IDS whose stored rows are the queries, as
         ``search -q``) yielding ``(ids, dists)`` numpy arrays in order -- the same
@@ -628,7 +792,13 @@ class MornaSearch(object):
         copy and batch i-1's device->host copy overlap batch i's kernels.
         ``query_groups`` (per-query exclusion, see set_row_groups): True -- every batch is internal ids and takes its
         labels from row_group[ids] (a stored row then never finds itself); or an iterable of int32 label arrays, one per
-        batch, in step with ``batches``.  Not with ``side_job``."""
+        batch, in step with ``batches``.  Not with ``side_job``.  ``max_per_group`` (see set_cap_groups): each batch is a
+        capped batched_search_device call, one at a time (no pipelining, no graph replay)."""
+        if max_per_group is not None:
+            if side_job:
+                raise ValueError("side_job cannot be combined with max_per_group")
+            yield from self._capped_batches(batches, k, query_groups, self._cap(max_per_group))
+            return
         if query_groups is not None and side_job:
             raise ValueError("side_job cannot be combined with query_groups")
         if query_groups is not None and self.row_group is None:
@@ -648,6 +818,29 @@ class MornaSearch(object):
         while pending:
             yield pipe.collect()
             pending -= 1
+
+    def _capped_batches(self, batches, k, query_groups, m):
+        if query_groups is not None and self.row_group is None:
+            raise ValueError("query_groups need row labels: call set_row_groups first")
+        labels = iter(query_groups) if query_groups is not None and query_groups is not True else None
+        for q in batches:
+            t = torch.from_numpy(np.ascontiguousarray(q)) if isinstance(q, np.ndarray) else q
+            by_id = t.dim() == 1 and t.dtype in (torch.int32, torch.int64)
+            if query_groups is True and not by_id:
+                raise ValueError("query_groups=True needs a batch of internal ids")
+            if by_id:
+                if t.numel():
+                    lo, hi = (int(v) for v in (t.min(), t.max()))
+                    if lo < self.row_lo or hi >= self.row_hi:
+                        raise ValueError("internal ids %d..%d are not all resident on this shard (rows %d..%d)"
+                                         % (lo, hi, self.row_lo, self.row_hi - 1))
+                rows = t.to(self.device).long() - self.row_lo
+                qd = self.vectors[rows, :self.dim].to(torch.float64).contiguous()
+            else:
+                qd = t.to(self.device).to(torch.float64).contiguous()
+            qg = self.row_group[rows] if query_groups is True else next(labels) if labels is not None else None
+            ids, d = self.batched_search_device(qd, k, query_groups=qg, max_per_group=m)
+            yield ids.cpu().numpy(), d.cpu().numpy()
 
     def _single_query_host(self, query, k):
         """One host query through the single-query kernel with persistent pinned staging: one host->device copy (the
@@ -684,15 +877,17 @@ class MornaSearch(object):
             return None
         return out[8 * k:12 * k].view(np.int32).reshape(1, k).copy(), out[:8 * k].view(np.float64).reshape(1, k).copy()
 
-    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None):
+    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None, max_per_group=None):
         """Host entry: queries numpy [nq x dim] (float32 or float64) -> numpy (ids, dists).
         float32 queries cross PCIe as float32 and are widened (exactly) on the device.  Batches of 64+
         queries use the tensor-core path, which returns the same bits as the scan.  ``query_groups``: per-query
-        exclusion, as in exact_search_device."""
+        exclusion, ``max_per_group``: a group-capped search, as in exact_search_device."""
         queries = np.ascontiguousarray(queries)
         if queries.dtype != np.float32:
             queries = queries.astype(np.float64, copy=False)
-        if queries.shape[0] == 1 and not tensor_cores and query_groups is None:
+        if max_per_group is not None:
+            self._cap(max_per_group)
+        if queries.shape[0] == 1 and not tensor_cores and query_groups is None and max_per_group is None:
             got = self._single_query_host(queries[0], k)
             if got is not None:
                 return got
@@ -702,13 +897,15 @@ class MornaSearch(object):
         qd = q.to(self.device, non_blocking=True).to(torch.float64)
         if tensor_cores is None:
             tensor_cores = qd.shape[0] >= 64
-        ids, d = (self.batched_search_device if tensor_cores else self.exact_search_device)(qd, k, query_groups=query_groups)
+        ids, d = (self.batched_search_device if tensor_cores else self.exact_search_device)(qd, k, query_groups=query_groups,
+                                                                                            max_per_group=max_per_group)
         return ids.cpu().numpy(), d.cpu().numpy()
 
-    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None):
-        """morna.py:681-730 for the current ``query_sample``; ``query_groups``: its label ([1]), as in exact_search_device."""
+    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None, max_per_group=None):
+        """morna.py:681-730 for the current ``query_sample``; ``query_groups``: its label ([1]), ``max_per_group``: a
+        group-capped search, as in exact_search_device."""
         ids, d = self.exact_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], num_neighbors,
-                                         query_groups=query_groups)
+                                         query_groups=query_groups, max_per_group=max_per_group)
         keep = ids[0] >= 0
         results = (ids[0][keep].tolist(),)
         if include_distances:
@@ -718,13 +915,15 @@ class MornaSearch(object):
         return results
 
     # ------------------------------------------------------------------ approximate mode
-    def approx_search_device(self, queries, k, query_groups=None):
+    def approx_search_device(self, queries, k, query_groups=None, max_per_group=None):
         """The k best rows by fp16 tensor-core score, no exact re-rank (morna_knn_batched_approx): the approximate mode
         that stands where the reference asks Annoy (morna.py:632-678).  Same contract as batched_search_device; queries
         whose lists overflow, tiny shards and sparse indexes are answered exactly.  There is no per-query exclusion in
-        this mode: ``query_groups`` raises ValueError."""
+        this mode, nor a cap: ``query_groups`` and ``max_per_group`` raise ValueError."""
         if query_groups is not None:
             raise ValueError("the approximate mode has no per-query exclusion; use an exact search")
+        if max_per_group is not None:
+            raise ValueError("the approximate mode has no cap per group; use an exact search")
         self.enable_tensor_path()
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.dim() == 2 and queries.shape[1] == self.dim
         queries = queries.contiguous()
@@ -748,10 +947,13 @@ class MornaSearch(object):
                 _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_knn_batched_approx")
         return self._batched_finish([(0, n, out_ids, out_d, overflow, stats)], queries, k)
 
-    def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False):
+    def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False, max_per_group=None):
         """morna.py:632-678 for the current ``query_sample``: the reference's default (approximate) mode.  Annoy's
         forest is not rebuilt here; the approximate answer is the tensor-core pass without the exact re-rank
-        (``search_k`` has no counterpart and is ignored).  ``exact_search_nn`` (-e) is the exact mode."""
+        (``search_k`` has no counterpart and is ignored).  ``exact_search_nn`` (-e) is the exact mode.  There is no cap
+        per group in this mode: ``max_per_group`` raises ValueError."""
+        if max_per_group is not None:
+            raise ValueError("the approximate mode has no cap per group; use an exact search")
         q = torch.tensor(self.query_sample, dtype=torch.float64)[None, :].to(self.device)
         ids, d = self.approx_search_device(q, num_neighbors)
         ids, d = ids.cpu().numpy(), d.cpu().numpy()
@@ -764,11 +966,12 @@ class MornaSearch(object):
         return results
 
     def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
-                        meta_db=False, out=None, max_distance=None, exclude=False):
+                        meta_db=False, out=None, max_distance=None, exclude=False, max_per_group=None):
         """morna.py:733-787 with the stored row as the query (float32 values), run
         through the exact scan.  With ``max_distance``: every sample within it (range_search_nn), the first
         ``num_neighbors`` of them when that is not None.  ``exclude``: the query takes its row's label (set_row_groups),
-        so its own sample and every sample of its group are left out."""
+        so its own sample and every sample of its group are left out.  ``max_per_group``: at most that many results per
+        cap label (set_cap_groups)."""
         internal_id = _member_internal_id(self.internal_id_map, query_id, out)
         if not (self.row_lo <= internal_id < self.row_hi):
             raise ValueError("internal id %d is not resident on this shard" % internal_id)
@@ -779,8 +982,9 @@ class MornaSearch(object):
                 raise ValueError("exclude needs row labels: call set_row_groups first")
             qg = self.row_group[internal_id - self.row_lo:internal_id - self.row_lo + 1]
         if max_distance is not None:
-            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg)
-        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg)
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg,
+                                        max_per_group=max_per_group)
+        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg, max_per_group=max_per_group)
 
     def _metadata(self, internal_ids):
         """morna.py:666-676: keywords of every result's sample id from basename.meta.mor."""
@@ -797,24 +1001,30 @@ class MornaSearch(object):
     RANGE_BATCH_QUERIES = 4096        # queries per morna_range_batched call (its candidate lists: 4096 x 4096 entries)
     RANGE_TENSOR_MIN_QUERIES = 64     # smaller batches go to the FP64 scan, as top-k batches do
 
-    def range_search_device(self, queries, max_distance, query_groups=None):
+    def range_search_device(self, queries, max_distance, query_groups=None, max_per_group=None):
         """Every row within ``max_distance`` of each query: queries CUDA float64 [nq x dim] -> device CSR (offsets int64
         [nq+1], ids int32 [total], dists float64 [total]); query j's list is ids/dists[offsets[j]:offsets[j+1]], ordered as
         the reference orders results (distance ascending, equal distances id descending), ids global.  The distance is
         exactly exact_search_device's and the comparison inclusive; a query with nothing in range has an empty list.
         Sets ``last_stats`` = [overflowed queries, first-pass survivors, matches] and ``last_range_route`` ("tensor":
         the tensor-core filter with an FP64 check, overflowed queries answered by the scan; "exact": the FP64 scan).
-        ``query_groups``: per-query exclusion, as in exact_search_device."""
-        return concat_range_groups(list(self.range_search_groups(queries, max_distance, query_groups=query_groups)), self.device)
+        ``query_groups``: per-query exclusion, as in exact_search_device.  ``max_per_group`` (see set_cap_groups): each
+        list walked in its order, an entry kept iff fewer than that many entries of its cap label were kept before it."""
+        return concat_range_groups(list(self.range_search_groups(queries, max_distance, query_groups=query_groups,
+                                                                 max_per_group=max_per_group)), self.device)
 
-    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None):
+    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None, max_per_group=None):
         """Generator over (lo, hi, offsets, ids, dists): the range_search_device CSR of queries [lo, hi), in query order.
         Batches of RANGE_BATCH_QUERIES are counted first (one small read back); with ``byte_cap``, a batch whose lists
         would take more than that many bytes (12 per match) is emitted in groups of consecutive queries that fit it (one
-        query per group at least), so no more than that is allocated at once."""
+        query per group at least), so no more than that is allocated at once.  With ``max_per_group`` each group's lists are then walked
+        (cap_sorted_lists); the byte cap applies to the lists before the walk."""
+        m = self._cap(max_per_group)
         for b0, st in self.range_count_batches(queries, max_distance, query_groups):
             for lo, hi in _range_groups(st["counts"], byte_cap):
                 off, ids, d = self.range_emit(st, lo, hi)
+                if m is not None:
+                    off, ids, d = self.cap_sorted_lists(off, ids, d, m)
                 yield b0 + lo, b0 + hi, off, ids, d
 
     def range_count_batches(self, queries, max_distance, query_groups=None):
@@ -836,7 +1046,7 @@ class MornaSearch(object):
             self.last_stats = list(stats)
             yield b0, st
 
-    def range_search_batch(self, queries, max_distance, query_groups=None):
+    def range_search_batch(self, queries, max_distance, query_groups=None, max_per_group=None):
         """Host entry: queries numpy [nq x dim] -> numpy CSR (offsets, ids, dists) of range_search_device."""
         queries = np.ascontiguousarray(queries)
         if queries.dtype != np.float32:
@@ -845,13 +1055,14 @@ class MornaSearch(object):
         if q.numel():
             q = q.pin_memory()
         qd = q.to(self.device, non_blocking=True).to(torch.float64)
-        return tuple(t.cpu().numpy() for t in self.range_search_device(qd, max_distance, query_groups))
+        return tuple(t.cpu().numpy() for t in self.range_search_device(qd, max_distance, query_groups, max_per_group))
 
-    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None):
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None,
+                        max_per_group=None):
         """Every indexed sample within ``max_distance`` of the current ``query_sample``, as exact_search_nn returns its
-        results; ``num_neighbors``: keep only the first that many."""
+        results; ``num_neighbors``: keep only the first that many (after the cap, with ``max_per_group``)."""
         _, ids, d = self.range_search_batch(np.asarray(self.query_sample, dtype=np.float64)[None, :], max_distance,
-                                            query_groups)
+                                            query_groups, max_per_group)
         if num_neighbors is not None:
             ids, d = ids[:max(int(num_neighbors), 0)], d[:max(int(num_neighbors), 0)]
         results = (ids.tolist(),)
@@ -1010,6 +1221,8 @@ class FilteredSearch(object):
             inner.pp = parent.pp.index_select(0, rows)
             if parent.row_group is not None:        # the subset rows keep their labels; queries keep theirs
                 inner.row_group = parent.row_group.index_select(0, rows)
+            if parent.cap_group is not None:        # and their cap labels
+                inner.set_cap_groups(parent.cap_group.index_select(0, rows))
             inner._build_csr()
             inner.query, inner.query_sample = defaultdict(int), [0.0] * parent.dim
         self.inner = inner
@@ -1078,13 +1291,14 @@ class FilteredSearch(object):
             raise ValueError("query_groups need row labels: call set_row_groups on the parent before subset()")
         return self._parent_row_group[torch.as_tensor(internal_ids).to(self.device).long() - self.row_lo]
 
-    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None):
-        ids, d = self.inner.exact_search_device(queries, k, stream, allow_single, query_groups)
+    def exact_search_device(self, queries, k, stream=None, allow_single=True, query_groups=None, max_per_group=None):
+        ids, d = self.inner.exact_search_device(queries, k, stream, allow_single, query_groups, max_per_group)
         with torch.cuda.stream(stream):
             return self._to_parent(ids), d
 
-    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None):
-        ids, d = self.inner.batched_search_device(queries, k, stream, check_overflow, phase_events, query_groups)
+    def batched_search_device(self, queries, k, stream=None, check_overflow=True, phase_events=None, query_groups=None,
+                              max_per_group=None):
+        ids, d = self.inner.batched_search_device(queries, k, stream, check_overflow, phase_events, query_groups, max_per_group)
         with torch.cuda.stream(stream):
             return self._to_parent(ids), d
 
@@ -1097,15 +1311,15 @@ class FilteredSearch(object):
         ids, d = self.inner.single_search_stream(queries, k)
         return self._to_parent(ids), d
 
-    def approx_search_device(self, queries, k, query_groups=None):
-        ids, d = self.inner.approx_search_device(queries, k, query_groups)
+    def approx_search_device(self, queries, k, query_groups=None, max_per_group=None):
+        ids, d = self.inner.approx_search_device(queries, k, query_groups, max_per_group)
         return self._to_parent(ids), d
 
-    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None):
-        ids, d = self.inner.exact_search_batch(queries, k, tensor_cores, query_groups)
+    def exact_search_batch(self, queries, k, tensor_cores=None, query_groups=None, max_per_group=None):
+        ids, d = self.inner.exact_search_batch(queries, k, tensor_cores, query_groups, max_per_group)
         return self._to_parent(ids), d
 
-    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None):
+    def search_batches(self, batches, k, depth=2, side_job=False, query_groups=None, max_per_group=None):
         """MornaSearch.search_batches over the subset; a batch of internal ids becomes the stored rows of those ids
         (stored_queries) on the device, and with ``query_groups=True`` takes the parent's labels of those ids (a query
         outside the subset too).  The distances are views of pinned buffers, as there."""
@@ -1125,41 +1339,47 @@ class FilteredSearch(object):
             while True:
                 yield pairs.pop(0)          # the labels of the batch queries() has just yielded
 
-        for ids, d in self.inner.search_batches(queries(), k, depth, side_job, None if query_groups is None else groups()):
+        for ids, d in self.inner.search_batches(queries(), k, depth, side_job, None if query_groups is None else groups(),
+                                                max_per_group):
             yield self._to_parent(ids), d
 
-    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None):
-        return self._nn(self.inner.exact_search_nn(num_neighbors, include_distances, query_groups=query_groups), meta_db)
+    def exact_search_nn(self, num_neighbors, include_distances=True, meta_db=False, query_groups=None, max_per_group=None):
+        return self._nn(self.inner.exact_search_nn(num_neighbors, include_distances, query_groups=query_groups,
+                                                   max_per_group=max_per_group), meta_db)
 
-    def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False):
-        return self._nn(self.inner.search_nn(num_neighbors, search_k, include_distances), meta_db)
+    def search_nn(self, num_neighbors, search_k=None, include_distances=True, meta_db=False, max_per_group=None):
+        return self._nn(self.inner.search_nn(num_neighbors, search_k, include_distances, max_per_group=max_per_group), meta_db)
 
     def search_member_n(self, query_id, num_neighbors, search_k=None, include_distances=True,
-                        meta_db=False, out=None, max_distance=None, exclude=False):
+                        meta_db=False, out=None, max_distance=None, exclude=False, max_per_group=None):
         """MornaSearch.search_member_n over the subset; the queried sample may lie outside it (with ``exclude`` it takes
         its label from the parent's rows)."""
         internal_id = _member_internal_id(self.internal_id_map, query_id, out)
         self.query_sample = self.stored_queries([internal_id])[0].cpu().tolist()
         qg = self.row_groups_of([internal_id]) if exclude else None
         if max_distance is not None:
-            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg)
-        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg)
+            return self.range_search_nn(max_distance, include_distances, meta_db, num_neighbors, query_groups=qg,
+                                        max_per_group=max_per_group)
+        return self.exact_search_nn(num_neighbors, include_distances, meta_db, query_groups=qg, max_per_group=max_per_group)
 
     # ------------------------------------------------------------------ range search
-    def range_search_device(self, queries, max_distance, query_groups=None):
-        offsets, ids, d = self.inner.range_search_device(queries, max_distance, query_groups)
+    def range_search_device(self, queries, max_distance, query_groups=None, max_per_group=None):
+        offsets, ids, d = self.inner.range_search_device(queries, max_distance, query_groups, max_per_group)
         return offsets, self._to_parent(ids), d
 
-    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None):
-        for lo, hi, offsets, ids, d in self.inner.range_search_groups(queries, max_distance, byte_cap, query_groups):
+    def range_search_groups(self, queries, max_distance, byte_cap=None, query_groups=None, max_per_group=None):
+        for lo, hi, offsets, ids, d in self.inner.range_search_groups(queries, max_distance, byte_cap, query_groups,
+                                                                      max_per_group):
             yield lo, hi, offsets, self._to_parent(ids), d
 
-    def range_search_batch(self, queries, max_distance, query_groups=None):
-        offsets, ids, d = self.inner.range_search_batch(queries, max_distance, query_groups)
+    def range_search_batch(self, queries, max_distance, query_groups=None, max_per_group=None):
+        offsets, ids, d = self.inner.range_search_batch(queries, max_distance, query_groups, max_per_group)
         return offsets, self._to_parent(ids), d
 
-    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None):
-        return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors, query_groups), meta_db)
+    def range_search_nn(self, max_distance, include_distances=True, meta_db=False, num_neighbors=None, query_groups=None,
+                        max_per_group=None):
+        return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors, query_groups,
+                                                   max_per_group), meta_db)
 
 
 class _PipeSlot(object):
