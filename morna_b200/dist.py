@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .search import _range_groups, check_radius, concat_range_groups
+from .search import _range_groups, check_max_per_group, check_radius, concat_range_groups
 
 
 def shard_bounds(n_rows, rank, world):
@@ -113,9 +113,11 @@ def sharded_exact_search(local_search, queries, k, group=None, merge=None, query
     return (merge or merge_topk)(ids, dists, k)
 
 
-def sharded_batched_search(search, queries, k, group=None, check_overflow=True, query_groups=None):
+def sharded_batched_search(search, queries, k, group=None, check_overflow=True, query_groups=None, max_per_group=None,
+                           merge=None, walk=None):
     """Rows-sharded exact search of a query batch on the tensor-core path, one process per GPU.  `search` holds this
     rank's row block (MornaSearch(..., shard=(rank, world))), `queries` (CUDA float64 [nq x dim]) are replicated.
+    ``max_per_group``: a group-capped search (sharded_capped_search below; `merge` and `walk` are its hooks).
 
       1. every rank scores the queries against its rows and writes, per query, lower bounds of the true cosines of
          its k best rows (fp16 score minus the rank's rigorous error bound);
@@ -128,6 +130,8 @@ def sharded_batched_search(search, queries, k, group=None, check_overflow=True, 
     Returns (ids, dists), identical on every rank and identical to one process scanning all rows.  ``query_groups``
     (per-query exclusion) is not supported here: ValueError."""
     _no_exclusion(query_groups)
+    if max_per_group is not None:
+        return sharded_capped_search(search, queries, k, max_per_group, group, merge, walk)
     import torch.distributed as td
     world = td.get_world_size(group) if (td.is_available() and td.is_initialized()) else 1
     if world == 1:
@@ -149,25 +153,145 @@ def gather_merge_packed(ids, dists, k, group=None, packed=None):
     import torch.distributed as td
     world = td.get_world_size(group)
     nq, k_in = ids.shape
-    nd, ni = nq * k_in * 8, nq * k_in * 4
-    mine = packed
-    if mine is None:
-        mine = torch.empty(nd + ni, dtype=torch.uint8, device=ids.device)
-        mine[:nd].view(torch.float64).copy_(dists.reshape(-1))
-        mine[nd:].view(torch.int32).copy_(ids.reshape(-1))
-    every = torch.empty((world, nd + ni), dtype=torch.uint8, device=ids.device)
+    mine = packed if packed is not None else pack_topk_lists(ids, dists)
+    every = torch.empty((world, mine.numel()), dtype=torch.uint8, device=ids.device)
     td.all_gather_into_tensor(every, mine, group=group)
+    return merge_packed_lists(every, nq, k_in, k)
+
+
+def pack_topk_lists(ids, dists):
+    """One rank's send buffer of the packed list all-gather: nq * k doubles (distances), then nq * k int32 (ids)."""
+    nd = ids.numel() * 8
+    mine = torch.empty(nd + ids.numel() * 4, dtype=torch.uint8, device=ids.device)
+    mine[:nd].view(torch.float64).copy_(dists.reshape(-1))
+    mine[nd:].view(torch.int32).copy_(ids.reshape(-1))
+    return mine
+
+
+def merge_packed_lists(every, nq, k_in, k):
+    """The rank-counting merge of an all-gather of packed lists: `every` uint8 [world x nq * k_in * 12], one
+    pack_topk_lists buffer per rank -> the top-k (ids, dists) [nq x k]."""
+    world = every.shape[0]
+    nd = nq * k_in * 8
     if (nq * k_in) % 2:                       # odd element count: the packed ids would not be 8-byte aligned per rank
         gd = every[:, :nd].contiguous().view(torch.float64).view(world, nq, k_in)
         gi = every[:, nd:].contiguous().view(torch.int32).view(world, nq, k_in)
         return merge_sorted_lists(gi, gd, k)
     lib = _lib.load()
-    out_i = torch.empty((nq, k), dtype=torch.int32, device=ids.device)
-    out_d = torch.empty((nq, k), dtype=torch.float64, device=ids.device)
-    with torch.cuda.device(ids.device):
+    out_i = torch.empty((nq, k), dtype=torch.int32, device=every.device)
+    out_d = torch.empty((nq, k), dtype=torch.float64, device=every.device)
+    with torch.cuda.device(every.device):
         _lib.check(lib.morna_merge_packed_topk(_lib.dev_ptr(every), world, nq, k_in, k, _lib.dev_ptr(out_i), _lib.dev_ptr(out_d),
                                                _lib.stream_ptr()), "morna_merge_packed_topk")
     return out_i, out_d
+
+
+# ------------------------------------------------------------------ group-capped search over a rows-sharded index
+# A group can have rows on several ranks, so a row one rank's walk kept can lose its place to another rank's rows of the
+# same group: the per-rank lists are merged and the merged order is walked again, with every row's cap label.  Exact
+# because every row of the global capped top-k is in its own rank's capped top-k (DESIGN.md section 6).
+
+MERGE_MAX_ENTRIES = 200 * 1024 // 12      # world * k entries per query morna_merge_packed_topk stages in shared memory
+
+
+def _cap_fields(search, max_per_group, group, world):
+    """The capped header's fields: (N or -1 if malformed, index size, 1 if this rank has cap labels, 1 if its row block is
+    shard_bounds' block of its rank).  Nothing here raises: a rank that raised on its own before a collective would
+    leave the others waiting in it."""
+    import torch.distributed as td
+    try:
+        m = check_max_per_group(max_per_group)
+    except (TypeError, ValueError):
+        m = -1
+    block = (search.row_lo, search.row_hi) == shard_bounds(search.index_size, td.get_rank(group), world)
+    return [m, int(search.index_size), int(search.cap_group is not None), int(block)]
+
+
+def _agree(fields, names, dev, group, world, what):
+    """One all-gather of an int64 header; ValueError on every rank unless every rank sent the same fields."""
+    import torch.distributed as td
+    head = torch.tensor(fields, dtype=torch.int64, device=dev)
+    every = torch.empty(world * head.numel(), dtype=torch.int64, device=dev)
+    td.all_gather_into_tensor(every, head, group=group)
+    rows = every.view(world, -1).cpu()
+    if not bool((rows == rows[0]).all()):
+        raise ValueError("%s: the ranks' (%s) differ: %s" % (what, ", ".join(names), rows.tolist()))
+
+
+def _check_cap_fields(max_per_group, fields):
+    """After the header agreed: the cap as an int, or the same ValueError on every rank."""
+    m = check_max_per_group(max_per_group)
+    if not fields[2]:
+        raise ValueError("max_per_group needs cap labels on every rank: call set_cap_groups first")
+    if not fields[3]:
+        raise ValueError("group-capped sharded search: the row blocks are not shard_bounds(%d, rank, world)" % fields[1])
+    return m
+
+
+CAP_FIELD_NAMES = ("max_per_group", "index size", "has cap labels", "row block of its rank")
+
+
+def cap_label_block(search, world):
+    """This rank's send buffer of the cap-label all-gather: its block's labels (set_cap_groups) padded with -1 to
+    ceil(index_size / world) rows, so that the gathered blocks sit at their rows (shard_bounds blocks are contiguous)."""
+    per = -(-search.index_size // world)
+    mine = torch.full((per,), -1, dtype=torch.int32, device=search.cap_group.device)
+    mine[:search.row_hi - search.row_lo] = search.cap_group
+    return mine
+
+
+def all_gather_cap_labels(search, group=None):
+    """Every row's cap label, int32 [index_size] on this rank's device, in ONE all-gather of cap_label_block."""
+    import torch.distributed as td
+    world = td.get_world_size(group)
+    mine = cap_label_block(search, world)
+    every = torch.empty(world * mine.numel(), dtype=torch.int32, device=mine.device)
+    td.all_gather_into_tensor(every, mine, group=group)
+    return every[:search.index_size]
+
+
+def merge_capped_topk(search, every, labels, nq, k, max_per_group, merge=None, walk=None):
+    """The step after the list all-gather of a capped top-k: `every` (uint8 [world x nq * k * 12], each rank's capped
+    [nq x k] lists as pack_topk_lists) merged whole, world * k entries per query (merge_packed_lists, or `merge` with its
+    arguments), then the merged order walked with every row's label `labels` (int32 [index_size]) and cut to k
+    (search.cap_sorted_lists, or `walk` with its arguments).  Returns (ids, dists) [nq x k], padded with -1 / +inf."""
+    world = every.shape[0]
+    ids, dists = (merge or merge_packed_lists)(every, nq, k, world * k)
+    offsets = torch.arange(nq + 1, dtype=torch.int64, device=ids.device) * (world * k)
+    out = (torch.empty((nq, k), dtype=torch.int32, device=ids.device), torch.empty((nq, k), dtype=torch.float64, device=ids.device))
+    return (walk or search.cap_sorted_lists)(offsets, ids, dists, max_per_group, k, out=out, cap_group=labels)
+
+
+def sharded_capped_search(search, queries, k, max_per_group, group=None, merge=None, walk=None):
+    """Group-capped top-k over a rows-sharded index (sharded_batched_search(..., max_per_group=N)): per query the nearest
+    rows with at most N of any one cap label, identical on every rank and to one process holding all rows.  Every rank
+    labels its block (set_cap_groups(global_labels[lo:hi])) and passes the same arguments, max_per_group included.
+
+      1. one all-gather of a header (nq, dim, k, N, index size, has cap labels, row block): ValueError on every rank if
+         the ranks differ, or if N is malformed or no rank has labels;
+      2. one all-gather of every row's cap label (all_gather_cap_labels; every call, 4 bytes per row);
+      3. every rank's capped top-k of its rows (batched_search_device(..., max_per_group=N): the tensor cores, or the FP64
+         route), ONE all-gather of the packed lists, the merge of all world * k entries and the walk over the merged
+         order, cut to k (merge_capped_topk)."""
+    world = _world_size(group)
+    if world == 1:
+        return search.batched_search_device(queries, k, max_per_group=max_per_group)
+    nq, k = int(queries.shape[0]), int(k)
+    fields = _cap_fields(search, max_per_group, group, world)
+    _agree([nq, int(queries.shape[1]), k] + fields, ("queries", "dim", "k") + CAP_FIELD_NAMES, queries.device, group, world,
+           "group-capped sharded search")
+    m = _check_cap_fields(max_per_group, fields)
+    if world * k > MERGE_MAX_ENTRIES:
+        raise ValueError("group-capped sharded search: world size x k = %d exceeds %d" % (world * k, MERGE_MAX_ENTRIES))
+    labels = all_gather_cap_labels(search, group)
+    ids, dists = search.batched_search_device(queries, k, max_per_group=m)
+    if nq == 0 or k <= 0:                 # the same on every rank: no list collective
+        return ids, dists
+    import torch.distributed as td
+    mine = pack_topk_lists(ids, dists)
+    every = torch.empty(world * mine.numel(), dtype=torch.uint8, device=mine.device)     # (flat: gloo takes 1-D only)
+    td.all_gather_into_tensor(every, mine, group=group)
+    return merge_capped_topk(search, every.view(world, -1), labels, nq, k, m, merge, walk)
 
 
 # ------------------------------------------------------------------ range search over a rows-sharded index
@@ -238,7 +362,8 @@ def _range_group_exchange(search, st, lo, hi, counts, group, merge):
     return merge_gathered_csr(every, counts, cap, merge)
 
 
-def sharded_range_search_groups(search, queries, max_distance, group=None, byte_cap=None, merge=None, query_groups=None):
+def sharded_range_search_groups(search, queries, max_distance, group=None, byte_cap=None, merge=None, query_groups=None,
+                                max_per_group=None, walk=None):
     """Range search over a rows-sharded index, one process per GPU: generator over (lo, hi, offsets, ids, dists), the
     device CSR of queries [lo, hi) in query order, as MornaSearch.range_search_groups.  `search` holds this rank's row
     block (MornaSearch(..., shard=(rank, world))); `queries` (CUDA float64 [nq x dim]) and every argument are the same
@@ -251,39 +376,55 @@ def sharded_range_search_groups(search, queries, max_distance, group=None, byte_
       3. per group every rank writes its lists, ONE all-gather of the packed lists (skipped when no rank has a
          match), and morna_merge_sorted_csr (or `merge`) puts every entry in its place.
     Collectives use flat 1-D tensors on the queries' device (NCCL with CUDA tensors, gloo with CPU tensors).
-    ``query_groups`` (per-query exclusion) is not supported here: ValueError."""
+    ``max_per_group`` (every rank labelled as for sharded_capped_search): the header also carries N, the index size and
+    the label checks, every row's cap label is all-gathered once, and each group's merged lists (the union of the ranks'
+    uncapped lists: the global in-range lists) are walked (search.cap_sorted_lists, or `walk` with its arguments);
+    byte_cap bounds the lists before the walk.  ``query_groups`` (per-query exclusion) is not supported here: ValueError."""
     _no_exclusion(query_groups)
     import torch.distributed as td
     world = _world_size(group)
     if world == 1:
-        yield from search.range_search_groups(queries, max_distance, byte_cap)
+        yield from search.range_search_groups(queries, max_distance, byte_cap, max_per_group=max_per_group)
         return
     dev = queries.device
     nq = int(queries.shape[0])
     r = float(max_distance)
-    head = torch.tensor([nq, int(queries.shape[1]), struct.unpack("<q", struct.pack("<d", r))[0],
-                         -1 if byte_cap is None else int(byte_cap)], dtype=torch.int64, device=dev)
-    every = torch.empty(world * head.numel(), dtype=torch.int64, device=dev)
-    td.all_gather_into_tensor(every, head, group=group)
-    rows = every.view(world, -1).cpu()
-    if not bool((rows == rows[0]).all()):
-        raise ValueError("sharded range search: the ranks' (queries, dim, radius bits, byte cap) differ: %s" % rows.tolist())
+    fields = [nq, int(queries.shape[1]), struct.unpack("<q", struct.pack("<d", r))[0], -1 if byte_cap is None else int(byte_cap)]
+    if max_per_group is None:
+        head = torch.tensor(fields, dtype=torch.int64, device=dev)
+        every = torch.empty(world * head.numel(), dtype=torch.int64, device=dev)
+        td.all_gather_into_tensor(every, head, group=group)
+        rows = every.view(world, -1).cpu()
+        if not bool((rows == rows[0]).all()):
+            raise ValueError("sharded range search: the ranks' (queries, dim, radius bits, byte cap) differ: %s" % rows.tolist())
+        m = labels = None
+    else:
+        cap_fields = _cap_fields(search, max_per_group, group, world)
+        _agree(fields + cap_fields, ("queries", "dim", "radius bits", "byte cap") + CAP_FIELD_NAMES, dev, group, world,
+               "sharded range search")
+        m = _check_cap_fields(max_per_group, cap_fields)
     if nq == 0:
         check_radius(r)
         return
+    if m is not None:
+        labels = all_gather_cap_labels(search, group)
     for b0, st in search.range_count_batches(queries, r):
         counts = torch.from_numpy(np.ascontiguousarray(st["counts"], dtype=np.int64)).to(dev)
         every = torch.empty(world * counts.numel(), dtype=torch.int64, device=dev)
         td.all_gather_into_tensor(every, counts, group=group)
         rank_counts = every.cpu().numpy().reshape(world, -1)
         for lo, hi in _range_groups(rank_counts.sum(axis=0) * (world + 1), byte_cap):
-            yield (b0 + lo, b0 + hi) + tuple(_range_group_exchange(search, st, lo, hi, rank_counts[:, lo:hi], group, merge))
+            csr = _range_group_exchange(search, st, lo, hi, rank_counts[:, lo:hi], group, merge)
+            if m is not None:
+                csr = (walk or search.cap_sorted_lists)(*csr, m, cap_group=labels)
+            yield (b0 + lo, b0 + hi) + tuple(csr)
 
 
-def sharded_range_search(search, queries, max_distance, group=None, merge=None, query_groups=None):
+def sharded_range_search(search, queries, max_distance, group=None, merge=None, query_groups=None, max_per_group=None,
+                         walk=None):
     """The whole device CSR (offsets, ids, dists) of sharded_range_search_groups, as MornaSearch.range_search_device."""
     _no_exclusion(query_groups)
     if _world_size(group) == 1:
-        return search.range_search_device(queries, max_distance)
-    return concat_range_groups(list(sharded_range_search_groups(search, queries, max_distance, group, merge=merge)),
-                               queries.device)
+        return search.range_search_device(queries, max_distance, max_per_group=max_per_group)
+    return concat_range_groups(list(sharded_range_search_groups(search, queries, max_distance, group, merge=merge,
+                                                                max_per_group=max_per_group, walk=walk)), queries.device)

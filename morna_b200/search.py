@@ -27,6 +27,13 @@ def check_radius(max_distance):
     return r
 
 
+def check_max_per_group(max_per_group):
+    """A group cap as an int: an integer >= 1, else ValueError."""
+    if isinstance(max_per_group, bool) or int(max_per_group) != max_per_group or max_per_group < 1:
+        raise ValueError("max_per_group must be an integer >= 1, got %r" % (max_per_group,))
+    return int(max_per_group)
+
+
 def _range_groups(counts, byte_cap):
     """[lo, hi) runs of consecutive queries whose lists (12 bytes per match) fit byte_cap; one run without a cap."""
     nq = len(counts)
@@ -129,8 +136,9 @@ class MornaSearch(object):
             self.vectors[:, :self.dim].copy_(block, non_blocking=False)
         self.pp = torch.empty(max(n, 1), dtype=torch.float64, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(self.lib.morna_row_norms(_lib.dev_ptr(self.vectors), n, self.dim, self.ld,
-                                                _lib.dev_ptr(self.pp), _lib.stream_ptr()), "morna_row_norms")
+            if n:                                          # (a rank of a rows-sharded index may hold no rows)
+                _lib.check(self.lib.morna_row_norms(_lib.dev_ptr(self.vectors), n, self.dim, self.ld,
+                                                    _lib.dev_ptr(self.pp), _lib.stream_ptr()), "morna_row_norms")
         self._build_csr()
 
     def _summation_plans(self, counts, row_off, cols):
@@ -415,24 +423,29 @@ class MornaSearch(object):
         """max_per_group as an int >= 1, or None for an uncapped search."""
         if max_per_group is None:
             return None
-        if isinstance(max_per_group, bool) or int(max_per_group) != max_per_group or max_per_group < 1:
-            raise ValueError("max_per_group must be an integer >= 1, got %r" % (max_per_group,))
+        m = check_max_per_group(max_per_group)
         if self.cap_group is None:
             raise ValueError("max_per_group needs cap labels: call set_cap_groups first")
-        return int(max_per_group)
+        return m
 
-    def cap_sorted_lists(self, offsets, ids, dists, max_per_group, limit=None, out=None):
+    def cap_sorted_lists(self, offsets, ids, dists, max_per_group, limit=None, out=None, cap_group=None):
         """The walk of a capped search (morna_cap_sorted_lists) over device lists already in the reference order: offsets
         int64 [L+1], ids int32 (global; -1 is padding), dists float64.  Each entry is kept iff fewer than max_per_group
         entries of its cap label were kept before it in its list, and at most ``limit`` per list (None: no limit).  Returns
-        the capped CSR (offsets, ids, dists), or with ``out`` = (ids [L x w], dists [L x w]) fills those, padded."""
+        the capped CSR (offsets, ids, dists), or with ``out`` = (ids [L x w], dists [L x w]) fills those, padded.
+        ``cap_group``: device int32 labels indexed from id 0 (every row of a rows-sharded index) in place of this
+        block's own."""
         L, total = offsets.numel() - 1, ids.numel()
         dev = self.device
         lim = -1 if limit is None else max(int(limit), 0)
+        if cap_group is None:
+            labels = (self.cap_group, self.row_lo, self.row_hi - self.row_lo)
+        else:
+            labels = (cap_group, 0, cap_group.numel())
         with torch.cuda.device(dev):
             ws = self._workspace(self.lib.morna_cap_sorted_lists_workspace_bytes(L, total), "cap_walk")
-            args = (_lib.dev_ptr(offsets), L, _lib.ptr(ids), _lib.ptr(dists), total, _lib.dev_ptr(self.cap_group),
-                    self.row_lo, self.row_hi - self.row_lo, max_per_group, lim)
+            args = (_lib.dev_ptr(offsets), L, _lib.ptr(ids), _lib.ptr(dists), total, _lib.dev_ptr(labels[0]), labels[1],
+                    labels[2], max_per_group, lim)
             if out is not None:
                 _lib.check(self.lib.morna_cap_sorted_lists(*args, None, _lib.ptr(out[0]), _lib.ptr(out[1]), out[0].shape[1],
                                                            _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_cap_sorted_lists")
@@ -607,9 +620,10 @@ class MornaSearch(object):
         self.hs = torch.empty((max(n, 1), self.ld_h), dtype=torch.float16, device=dev)
         self.rho_max = torch.zeros(1, dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(self.lib.morna_prepare_tensor_operand(
-                _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.dev_ptr(self.hs),
-                self.ld_h, _lib.dev_ptr(self.rho_max), _lib.stream_ptr()), "morna_prepare_tensor_operand")
+            if n:                                          # (no rows: nothing to prepare, and no row pointer to pass)
+                _lib.check(self.lib.morna_prepare_tensor_operand(
+                    _lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), n, self.dim, self.ld, _lib.dev_ptr(self.hs),
+                    self.ld_h, _lib.dev_ptr(self.rho_max), _lib.stream_ptr()), "morna_prepare_tensor_operand")
         self._bws = {}
         self.last_stats = None
 
