@@ -499,6 +499,44 @@ int morna_knn_batched_capped(const float *vectors, const double *pp, const void 
                              const int32_t *query_group, int32_t *out_ids, double *out_dist,
                              uint8_t *overflow, int32_t *stats, void *workspace, size_t workspace_bytes, void *stream);
 
+/* Within-group search, grouped FP64 route: each query against the rows of its own group only (at most 8192 rows),
+ * many groups in one call.  The caller lists the rows grouped and the queries sorted by group:
+ *   group_rows  [dev] int32 local row ids (0 .. n-1); the rows of one group are contiguous and ascending
+ *   queries     [dev] float64 [nq x q_ld], every query's group a run of consecutive queries
+ *   row_begin   [dev] int32[nq]: where query j's group starts in group_rows
+ *   seg_off     [dev] int64[nq + 1] from 0: query j's segment of the distance scratch (the workspace) is
+ *               [seg_off[j], seg_off[j + 1]), one entry per row of its group, at most max_segment (<= 8192) entries;
+ *               total = seg_off[nq]
+ *   items       [dev] int32[n_items x 4], 16-byte aligned: {first query, query count 1..8, first row (index into
+ *               group_rows), row count}; the queries of an item share one group, the rows are part of it, and together
+ *               the items cover every (query, row of its group) pair once.  An item's queries are staged once and every
+ *               row it names is read once for all of them; items of one group should be adjacent (their rows stay in L2)
+ *   exclude_rows [dev] int32[nq] or NULL: a local row left out of query j's list (-1: none)
+ *   out_slot    [dev] int32[nq]: the output row of query j
+ * Distances are the canonical sums of morna_angular_distances, bit for bit.  No host synchronisation.
+ * Top-k: out_ids / out_dist [.. x k], row out_slot[j] = the first k of query j's segment under the reference order (ids
+ * id_base + row), padded with id -1 / +inf (an excluded row is padding too). */
+size_t morna_within_group_workspace_bytes(int64_t total);
+int morna_within_group_topk(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld, int32_t id_base,
+                            const int32_t *group_rows, const double *queries, int64_t nq, int64_t q_ld, const int32_t *items,
+                            int64_t n_items, const int64_t *seg_off, int64_t total, const int32_t *row_begin,
+                            int32_t max_segment, const int32_t *exclude_rows, const int32_t *out_slot, int32_t k,
+                            int32_t *out_ids, double *out_dist, void *workspace, size_t workspace_bytes, void *stream);
+/* Range, in two calls: the count writes counts [dev] int64[out_slot[j]] = the entries of query j's segment with
+ * d <= max_distance (finite, >= 0) and leaves the distances in the workspace; the fill, given the unchanged workspace and
+ * out_offsets [dev] int64 (query j's list at [out_offsets[out_slot[j]], out_offsets[out_slot[j] + 1]), its length the
+ * count), writes each list in the reference order. */
+int morna_within_group_range_count(const float *vectors, const double *pp, int64_t n, int32_t dim, int64_t ld,
+                                   const int32_t *group_rows, const double *queries, int64_t nq, int64_t q_ld,
+                                   const int32_t *items, int64_t n_items, const int64_t *seg_off, int64_t total,
+                                   const int32_t *row_begin, int32_t max_segment, const int32_t *exclude_rows,
+                                   const int32_t *out_slot, double max_distance, int64_t *counts, void *workspace,
+                                   size_t workspace_bytes, void *stream);
+int morna_within_group_range_fill(int64_t nq, const int32_t *group_rows, int32_t id_base, const int64_t *seg_off,
+                                  int64_t total, const int32_t *row_begin, int32_t max_segment, const int32_t *out_slot,
+                                  const int64_t *out_offsets, int32_t *out_ids, double *out_dist, const void *workspace,
+                                  size_t workspace_bytes, void *stream);
+
 /* Test hook: raw fp16 tensor-core scores [nq x n] (n <= 8192) and the per-query bound eps. */
 int morna_debug_tensor_scores(const void *hs, int64_t ld_h, const float *rho_max, int64_t n, int32_t dim,
                               const double *queries, int64_t nq, int64_t q_ld, float *scores,

@@ -119,6 +119,15 @@ _SIGNATURES = {
     "morna_knn_batched_capped": (ctypes.c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp,
                                                 _c_i64, _c_i64, _c_i32, _c_vp, _c_i32, _c_vp, _c_i32, _c_vp, _c_vp, _c_vp, _c_vp,
                                                 _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_within_group_workspace_bytes": (_c_sz, [_c_i64]),
+    "morna_within_group_topk": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_i32, _c_vp, _c_vp, _c_i64, _c_i64,
+                                               _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_i32, _c_vp, _c_vp, _c_i32, _c_vp, _c_vp,
+                                               _c_vp, _c_sz, _c_vp]),
+    "morna_within_group_range_count": (ctypes.c_int, [_c_vp, _c_vp, _c_i64, _c_i32, _c_i64, _c_vp, _c_vp, _c_i64, _c_i64,
+                                                      _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_i32, _c_vp, _c_vp,
+                                                      ctypes.c_double, _c_vp, _c_vp, _c_sz, _c_vp]),
+    "morna_within_group_range_fill": (ctypes.c_int, [_c_i64, _c_vp, _c_i32, _c_vp, _c_i64, _c_vp, _c_i32, _c_vp, _c_vp,
+                                                     _c_vp, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_tensor_scores": (ctypes.c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i32, _c_vp, _c_i64, _c_i64, _c_vp,
                                                  _c_i64, _c_vp, _c_vp, _c_sz, _c_vp]),
     "morna_debug_set_tuning": (ctypes.c_int, [_c_i32, _c_i32]),

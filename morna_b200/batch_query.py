@@ -298,6 +298,38 @@ def search_all_samples_range(search, max_distance, inverse, result_cap=None, exc
             yield inverse[batch[g0:g1]], off.cpu().numpy(), ids.cpu().numpy(), d.cpu().numpy()
 
 
+def _within_batch(search, queries, groups, exclude, k, max_distance):
+    """One batch of a within-group search as numpy: (ids, dists) top-k, or with max_distance (offsets, ids, dists)."""
+    if max_distance is None:
+        return tuple(t.cpu().numpy() for t in search.within_group_search(queries, k, groups, exclude))
+    return tuple(t.cpu().numpy() for t in search.within_group_range(queries, max_distance, groups, exclude))
+
+
+def search_all_samples_within(search, inverse, labels, k=None, max_distance=None, exclude_self=False):
+    """--all-samples --within-group: every sample (of the subset) by internal id, against the samples of its own group
+    only (`labels`: the group label of every internal id; the search's rows carry the same labels).  Yields (sample ids,
+    ids, dists) numpy batches in query order, or with `max_distance` (sample ids, offsets, ids, dists) CSR batches.
+    `exclude_self`: a query's own sample is left out of its list."""
+    members = all_sample_ids(search)
+    for b in range(0, len(members), BATCH_QUERIES):
+        batch = members[b:b + BATCH_QUERIES]
+        yield (inverse[batch],) + _within_batch(search, torch.from_numpy(batch), labels[batch],
+                                                batch.astype(np.int32) if exclude_self else None, k, max_distance)
+
+
+def search_query_file_within(search, path, query_labels, exclude_ids=None, k=None, max_distance=None, cap=None):
+    """--query-intropolis -e --within-group: every sample of the file against the samples of its own group
+    (`query_labels(sample_ids)` -> int32 labels; < 0: no group, an empty list).  `exclude_ids(sample_ids)` -> the internal
+    id each query leaves out (-1: none).  Yields batches as search_all_samples_within does."""
+    qf = QueryFile(search, path)
+    for lo, hi in qf.slices(cap):
+        vecs = qf.query_vectors(lo, hi)
+        for b in range(0, hi - lo, BATCH_QUERIES):
+            sids = qf.sample_ids[lo + b:min(hi, lo + b + BATCH_QUERIES)]
+            yield (sids,) + _within_batch(search, vecs[b:b + BATCH_QUERIES], query_labels(sids),
+                                          None if exclude_ids is None else exclude_ids(sids), k, max_distance)
+
+
 def cut_lists(offsets, ids, dists, limit):
     """CSR lists cut to their first `limit` entries (numpy; None: unchanged)."""
     if limit is None:

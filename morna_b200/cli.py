@@ -132,6 +132,10 @@ def build_parser():
     search_parser.add_argument("--groups", metavar="<file>", type=str, required=False, default=None,
                                help="the groups --max-per-group caps: a file of 'sample_id<TAB>group' lines, as for "
                                     "--exclude-group; a sample not listed is a group of its own")
+    search_parser.add_argument("--within-group", metavar="<file>", type=str, required=False, default=None,
+                               help="a file of 'sample_id<TAB>group' lines, as for --exclude-group: each query searches "
+                                    "only the samples of its own group (-q, --all-samples, --query-intropolis -e); a "
+                                    "sample not listed is a group of its own")
     junctions_parser = subs.add_parser("junctions", help="extracts the junctions of a query's nearest neighbors")
     add_search_parameters(junctions_parser)                      # morna.py:1023-1054
     junctions_parser.add_argument("-i", "--index", metavar="<idx>", type=str, required=True,
@@ -289,6 +293,51 @@ def exclusion(args):
     return Exclusion(group_of, files.read_map(args.basename), index_size)
 
 
+def within_group(args):
+    """--within-group FILE: an Exclusion whose labels are the groups each query searches within, or None without the
+    flag.  Raises ValueError with the message for the user when the flags, the query mode or the file are not usable
+    (before any GPU work)."""
+    path = getattr(args, "within_group", None)
+    if path is None:
+        return None
+    for other, flag in (("exclude_group", "--exclude-group"), ("max_per_group", "--max-per-group")):
+        if getattr(args, other, None) is not None:
+            raise ValueError("--within-group cannot be combined with %s" % flag)
+    if args.query_id is None and not args.all_samples and args.query_intropolis is None:
+        raise ValueError("--within-group needs queries that are samples (-q, --all-samples or --query-intropolis): a "
+                         "query read from stdin has no sample id")
+    if args.query_intropolis is not None and not args.exact:
+        raise ValueError("--within-group with --query-intropolis needs -e: the approximate mode has no within-group "
+                         "search")
+    group_of = read_group_file("--within-group", path)
+    from . import files
+    return Exclusion(group_of, files.read_map(args.basename), files.read_stats(args.basename)[1])
+
+
+def within_member(searcher, args, within, exclude_self, max_distance, limit, out):
+    """-q --within-group: the result columns of the queried sample against the samples of its own group."""
+    from .batch_query import inverse_map
+    from .search import _member_internal_id
+    from . import files
+    internal_id = _member_internal_id(searcher.internal_id_map, args.query_id, out)
+    ids = np.array([internal_id], dtype=np.int64)
+    groups = within.labels_of_samples([args.query_id])
+    exclude = ids.astype(np.int32) if exclude_self else None
+    if max_distance is None:
+        r_ids, r_d = (t.cpu().numpy()[0] for t in searcher.within_group_search(ids, args.results, groups, exclude))
+        r_ids, r_d = r_ids[r_ids >= 0], r_d[r_ids >= 0]
+    else:
+        _, r_ids, r_d = (t.cpu().numpy() for t in searcher.within_group_range(ids, max_distance, groups, exclude))
+        if limit is not None:
+            r_ids, r_d = r_ids[:max(limit, 0)], r_d[:max(limit, 0)]
+    results = (r_ids.tolist(),)
+    if args.distances:
+        results += (r_d.tolist(),)
+    if args.metadata:
+        results += (files.read_meta(args.basename, inverse_map(searcher)[r_ids].tolist()),)
+    return results
+
+
 def open_search(basename, keep, keep_parent_rows, excl=None, cap=None):
     """The index's MornaSearch, or with `keep` (sample_filter's ids) a FilteredSearch over those samples; with `excl`
     (an Exclusion) every row carries its label, with `cap` (cap_groups' result) its cap label."""
@@ -331,6 +380,7 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     limit = args.results if max_distance is not None and "results" in getattr(args, "given", ()) else None
     try:
         keep = sample_filter(args)
+        within = within_group(args) if args.subparser_name == "search" else None
         excl = exclusion(args) if args.subparser_name == "search" else None
         cap = cap_groups(args) if args.subparser_name == "search" else None
     except ValueError as exc:
@@ -338,15 +388,18 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
         return 2
     per_group = cap[0] if cap is not None else None
     if getattr(args, "query_intropolis", None) is not None or getattr(args, "all_samples", False):
-        return batch_search(args, stdout, stderr, max_distance, limit, keep, excl, cap)
+        return batch_search(args, stdout, stderr, max_distance, limit, keep, excl, cap, within)
     opened = None
     if args.subparser_name == "junctions":                      # morna.py:1351-1353
         args.format = "sam"
         stdin = opened = open(args.pass1_sam)
     # (a filter keeps the whole index's rows only for -q, whose sample may lie outside the subset)
-    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None, excl=excl, cap=cap)
+    # (with --within-group the rows carry its labels; --exclude-self then leaves out the query's own row only)
+    searcher = open_search(args.basename, keep, keep_parent_rows=args.query_id is not None, excl=within or excl, cap=cap)
     if args.query_id is not None:                               # morna.py:1358-1365
-        if max_distance is not None:
+        if within is not None:
+            results = within_member(searcher, args, within, excl is not None, max_distance, limit, stdout)
+        elif max_distance is not None:
             results = searcher.search_member_n(args.query_id, limit, include_distances=args.distances,
                                                meta_db=args.metadata, out=stdout, max_distance=max_distance,
                                                exclude=excl is not None, max_per_group=per_group)
@@ -392,11 +445,13 @@ def main(argv=None, stdin=None, stdout=None, stderr=None):
     return 0
 
 
-def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None, excl=None, cap=None):
+def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None, excl=None, cap=None, within=None):
     """--query-intropolis / --all-samples: many queries in one run, results streamed in 4096-query batches.  With
     `max_distance`, every sample within it per query (CSR batches), each list cut to `limit` entries if given.  With
     `keep` (sample_filter's ids), the search runs over those samples only.  With `excl` (an Exclusion), each query
-    leaves out the samples of its group.  With `cap` (cap_groups' result), at most N samples per group."""
+    leaves out the samples of its group.  With `cap` (cap_groups' result), at most N samples per group.  With `within`
+    (within_group's Exclusion), each query searches the samples of its own group only, and `excl` (--exclude-self) leaves
+    out its own sample."""
     from . import batch_query
     named = [name for name, on in (("--query-intropolis", args.query_intropolis is not None),
                                    ("--all-samples", args.all_samples), ("-q", args.query_id is not None),
@@ -405,10 +460,25 @@ def batch_search(args, stdout, stderr, max_distance=None, limit=None, keep=None,
         stderr.write("%s cannot be combined with %s\n" % (named[0], ", ".join(named[1:])))
         return 2
     # (with an exclusion, --all-samples over a subset takes its labels from the whole index's rows)
-    searcher = open_search(args.basename, keep, keep_parent_rows=False, excl=excl, cap=cap)
+    searcher = open_search(args.basename, keep, keep_parent_rows=False, excl=within or excl, cap=cap)
     per_group = cap[0] if cap is not None else None
     inverse = batch_query.inverse_map(searcher)
     meta = args.basename if args.metadata else None
+    if within is not None:
+        k = None if max_distance is not None else args.results
+        if args.all_samples:
+            results = batch_query.search_all_samples_within(searcher, inverse, within.row_labels, k, max_distance,
+                                                            exclude_self=excl is not None)
+        else:
+            own = (lambda sids: np.array([within.id_map.get(s, -1) for s in sids.tolist()], dtype=np.int32)) \
+                if excl is not None else None
+            results = batch_query.search_query_file_within(searcher, args.query_intropolis, within.labels_of_samples, own,
+                                                           k, max_distance)
+        for batch in results:
+            offsets = batch[1] if max_distance is not None else None
+            batch_query.write_results(stdout, batch[0], batch[-2], batch[-1], args.distances, meta, inverse,
+                                      offsets=offsets, limit=limit)
+        return 0
     exclude = excl is not None
     query_labels = excl.labels_of_samples if exclude else None
     if max_distance is not None:

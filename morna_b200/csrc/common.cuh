@@ -87,6 +87,31 @@ __device__ __forceinline__ bool before(double da, int ia, double db, int ib) {
     return da < db || (da == db && ia > ib);
 }
 
+// bitonic sort of P (power of two) (key,id) pairs in shared memory under `before`
+template <bool kWithIds>
+__device__ inline void bitonic_sort_smem(double *sd, int *si, int P) {
+    for (int size = 2; size <= P; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < (P >> 1); i += blockDim.x) {
+                int lo = 2 * i - (i & (stride - 1));
+                int hi = lo + stride;
+                bool asc = (lo & size) == 0;
+                double dl = sd[lo], dh = sd[hi];
+                int il = kWithIds ? si[lo] : 0, ih = kWithIds ? si[hi] : 0;
+                bool hi_first = kWithIds ? before(dh, ih, dl, il) : (dh < dl);
+                bool lo_first = kWithIds ? before(dl, il, dh, ih) : (dl < dh);
+                bool swap = asc ? hi_first : lo_first;
+                if (swap) {
+                    sd[lo] = dh; sd[hi] = dl;
+                    if (kWithIds) { si[lo] = ih; si[hi] = il; }
+                }
+            }
+        }
+    }
+    __syncthreads();
+}
+
 // Per-query exclusion on the FP64 routes (search_exact.cu).  Row i is excluded for query q iff
 // query_group[q] >= 0 && row_group[i] == query_group[q]; the mask writes +inf into the distance scratch
 // [nq x dist_ld] of every excluded pair, so a selection after it never prefers an excluded row to a real

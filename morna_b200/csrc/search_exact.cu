@@ -120,31 +120,6 @@ constexpr int kSelChunk = kSelThreads * kSelItems;   // 8192 keys per CTA
 constexpr int kSelCap = 1024;                         // survivors the fast path sorts
 constexpr int kSelMaxK = 2048;
 
-// bitonic sort of P (power of two) (key,id) pairs in shared memory under `before`
-template <bool kWithIds>
-__device__ void bitonic_sort_smem(double *sd, int *si, int P) {
-    for (int size = 2; size <= P; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < (P >> 1); i += blockDim.x) {
-                int lo = 2 * i - (i & (stride - 1));
-                int hi = lo + stride;
-                bool asc = (lo & size) == 0;
-                double dl = sd[lo], dh = sd[hi];
-                int il = kWithIds ? si[lo] : 0, ih = kWithIds ? si[hi] : 0;
-                bool hi_first = kWithIds ? before(dh, ih, dl, il) : (dh < dl);
-                bool lo_first = kWithIds ? before(dl, il, dh, ih) : (dl < dh);
-                bool swap = asc ? hi_first : lo_first;
-                if (swap) {
-                    sd[lo] = dh; sd[hi] = dl;
-                    if (kWithIds) { si[lo] = ih; si[hi] = il; }
-                }
-            }
-        }
-    }
-    __syncthreads();
-}
-
 __global__ void __launch_bounds__(kSelThreads)
 select_topk_kernel(const double *__restrict__ keys, const int32_t *__restrict__ ids, int64_t n,
                    int64_t key_ld, int32_t id_base, int32_t k, int32_t *__restrict__ out_ids,

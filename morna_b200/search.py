@@ -344,6 +344,7 @@ class MornaSearch(object):
         """Labels for per-query exclusion: int32 [n], one per resident row (None clears them).  A search given
         ``query_groups`` then leaves out, for query q, every row whose label equals query_groups[q] (a label < 0 excludes
         nothing): with every row its own label and a query's label its row's, a stored row no longer finds itself."""
+        self._within = None                                # (the within-group layout of the old labels)
         if labels is None:
             self.row_group = None
             return
@@ -1189,6 +1190,262 @@ class MornaSearch(object):
                     d[dst] = sub_d
             return offsets[lo:hi + 1], ids, d
 
+    # ------------------------------------------------------------------ within-group search
+    # The queries of one group in one call take the grouped FP64 route (morna_within_group_*) when the group has at most
+    # WITHIN_SEGMENT_ROWS rows (the selection's shared-memory sort) and (queries x rows) is at most WITHIN_GROUPED_MAX_PAIRS;
+    # otherwise the tensor-core path searches the group as a row range of the grouped copy (_within_copy).  The grouped
+    # route costs about the same per (query, row) pair whatever the group, the tensor-core route a fixed cost per group
+    # and call and far less per pair, so the crossing is a pair count.  The sweep of profiles/r10_within_group.log (B200,
+    # top-20) puts it near 250,000 pairs for contiguous and scattered groups alike: grouped faster at 65,000 / 85,000
+    # pairs (2.6 vs 7.5, 17.4 vs 44.3 ms per 4096 queries), slower at 262,000 / 341,000 (4.5 vs 4.1, 32.5 vs 23.2).
+    WITHIN_SEGMENT_ROWS = 8192
+    WITHIN_GROUPED_MAX_PAIRS = 250000
+    WITHIN_QB = 8                    # queries per work item (kWithinQB of search_within.cu)
+    WITHIN_CHUNK_ROWS = 128          # rows per work item
+    WITHIN_SCRATCH_ENTRIES = 1 << 25 # distances of one grouped call (256 MB)
+
+    def _within_layout(self):
+        """The rows sorted by (label, id), labels < 0 left out: (device int32 local rows, host labels ascending, host
+        starts, host counts, {"copy": _within_copy's index once built}).  Cached until set_row_groups."""
+        st = self.__dict__.get("_within")
+        if st is not None:
+            return st
+        if self.row_group is None:
+            raise ValueError("a within-group search needs row labels: call set_row_groups first")
+        g = self.row_group.long()
+        order = torch.sort(g, stable=True).indices
+        keep = g[order] >= 0
+        rows = order[keep].to(torch.int32).contiguous()
+        labels, counts = torch.unique(g[order][keep], return_counts=True)
+        labels, counts = labels.cpu().numpy(), counts.cpu().numpy().astype(np.int64)
+        starts = np.zeros(len(counts), np.int64)
+        np.cumsum(counts[:-1], out=starts[1:])
+        if rows.numel() == 0:
+            rows = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._within = st = (rows, labels, starts, counts, {})
+        return st
+
+    def _within_queries(self, queries):
+        """(device float64 [nq x dim] or None, device int64 local rows or None): the queries as vectors or stored rows."""
+        t = torch.from_numpy(np.ascontiguousarray(queries)) if isinstance(queries, np.ndarray) else torch.as_tensor(queries)
+        if t.dim() == 1 and t.dtype in (torch.int32, torch.int64):
+            if t.numel():
+                lo, hi = (int(v) for v in (torch.aminmax(t) if t.is_cuda else (t.min(), t.max())))
+                if lo < self.row_lo or hi >= self.row_hi:
+                    raise ValueError("internal ids %d..%d are not all resident (rows %d..%d)"
+                                     % (lo, hi, self.row_lo, self.row_hi - 1))
+            return None, t.to(self.device).long() - self.row_lo
+        assert t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape[1] == self.dim, \
+            "queries must be CUDA float64 [nq x dim] or 1-D internal ids"
+        return t, None
+
+    def _within_plan(self, queries, query_groups, exclude_rows):
+        """Per query (host): group index, row count of its group and local excluded row (-1: none)."""
+        rows, labels, starts, counts, _ = self._within_layout()
+        vecs, qrows = self._within_queries(queries)
+        nq = qrows.numel() if qrows is not None else vecs.shape[0]
+        qg = torch.as_tensor(query_groups).cpu().numpy().astype(np.int64).reshape(-1)
+        if qg.shape != (nq,):
+            raise ValueError("query_groups must hold one label per query (%d), got %d" % (nq, qg.size))
+        gi = np.minimum(np.searchsorted(labels, qg), max(len(labels) - 1, 0))
+        present = (qg >= 0) & (labels[gi] == qg) if len(labels) else np.zeros(nq, bool)
+        size = np.where(present, counts[gi] if len(labels) else 0, 0)
+        in_call = np.bincount(gi[present], minlength=len(labels))[gi] if len(labels) else size
+        grouped = present & (size <= self.WITHIN_SEGMENT_ROWS) & (size * in_call <= self.WITHIN_GROUPED_MAX_PAIRS)
+        excl = np.full(nq, -1, np.int64)
+        if exclude_rows is not None:
+            e = torch.as_tensor(exclude_rows).cpu().numpy().astype(np.int64).reshape(-1)
+            if e.shape != (nq,):
+                raise ValueError("exclude_rows must hold one internal id per query (%d), got %d" % (nq, e.size))
+            inside = (e >= self.row_lo) & (e < self.row_hi)
+            excl[inside] = e[inside] - self.row_lo
+        self.last_within_routes = (int(grouped.sum()), int((present & ~grouped).sum()))
+        return {"vecs": vecs, "qrows": qrows, "nq": nq, "gi": gi, "size": size, "excl": excl,
+                "grouped": np.nonzero(grouped)[0], "large": np.nonzero(present & ~grouped)[0]}
+
+    def _within_rows(self, plan, idx):
+        """Float64 device query vectors of queries idx (host int64), in that order."""
+        if plan["qrows"] is not None:
+            return self.vectors[plan["qrows"][torch.from_numpy(idx).to(self.device)], :self.dim].to(torch.float64).contiguous()
+        return plan["vecs"][torch.from_numpy(idx).to(self.device)].contiguous()
+
+    def _within_grouped_calls(self, plan, slots):
+        """Generator over the grouped route's calls: (kwargs of morna_within_group_*, original query indices).  The
+        grouped queries are sorted stably by group and cut where the summed segment lengths would pass the scratch
+        budget; each call's work items are tiles of up to WITHIN_QB queries of one group x chunks of its rows.  `slots`:
+        "query" -- out_slot is the query's index in the whole call, "local" -- its index in this grouped call."""
+        rows, labels, starts, counts, _ = self._within_layout()
+        idx = plan["grouped"]
+        idx = idx[np.argsort(plan["gi"][idx], kind="stable")]
+        lens = plan["size"][idx]
+        cum = np.cumsum(lens)
+        a, dev, QB, CH = 0, self.device, self.WITHIN_QB, self.WITHIN_CHUNK_ROWS
+        while a < len(idx):
+            b = max(a + 1, int(np.searchsorted(cum, (cum[a - 1] if a else 0) + self.WITHIN_SCRATCH_ENTRIES, side="right")))
+            o, g, ln = idx[a:b], plan["gi"][idx[a:b]], lens[a:b]
+            n = b - a
+            seg_off = np.zeros(n + 1, np.int64)
+            np.cumsum(ln, out=seg_off[1:])
+            pos = np.arange(n)
+            head_run = np.r_[True, g[1:] != g[:-1]]
+            run_start = np.maximum.accumulate(np.where(head_run, pos, 0))
+            run_end = np.r_[np.nonzero(head_run)[0][1:], n][np.cumsum(head_run) - 1]
+            t0 = np.nonzero((pos - run_start) % QB == 0)[0]
+            qn = np.minimum(QB, run_end[t0] - t0)
+            nch = (ln[t0] + CH - 1) // CH
+            rep = np.repeat(np.arange(len(t0)), nch)
+            c = np.arange(rep.size) - np.repeat(np.cumsum(nch) - nch, nch)
+            items = np.stack([t0[rep], qn[rep], starts[g[t0]][rep] + c * CH, np.minimum(CH, ln[t0][rep] - c * CH)], 1)
+            up = lambda x, dt: torch.from_numpy(np.ascontiguousarray(x, dtype=dt)).to(dev)
+            excl = plan["excl"][o]
+            yield {"queries": self._within_rows(plan, o), "items": up(items, np.int32), "seg_off": up(seg_off, np.int64),
+                   "total": int(seg_off[-1]), "row_begin": up(starts[g], np.int32), "max_segment": int(ln.max()),
+                   "exclude": up(excl, np.int32) if (excl >= 0).any() else None,
+                   "out_slot": up(o if slots == "query" else pos, np.int32)}, o
+            a = b
+
+    def _within_call_args(self, c):
+        rows = self._within_layout()[0]
+        return (_lib.dev_ptr(self.vectors), _lib.dev_ptr(self.pp), self.row_hi - self.row_lo, self.dim, self.ld), \
+               (_lib.dev_ptr(rows), _lib.ptr(c["queries"]), c["queries"].shape[0], self.dim, _lib.dev_ptr(c["items"]),
+                c["items"].shape[0], _lib.dev_ptr(c["seg_off"]), c["total"], _lib.dev_ptr(c["row_begin"]), c["max_segment"],
+                _lib.dev_ptr(c["exclude"]), _lib.dev_ptr(c["out_slot"]))
+
+    def _within_copy(self):
+        """Every labelled row copied once in the layout's order, so that each group is a contiguous row range, with its
+        norms and fp16 tensor-core operand; row i carries as exclusion label its position within its group.  Built on
+        the first call that sends a group to the tensor-core route and kept until set_row_groups: one more copy of the
+        labelled rows (and their fp16 operand) instead of a sub-index per group and call."""
+        rows, labels, starts, counts, cache = self._within_layout()
+        cp = cache.get("copy")
+        if cp is None:
+            m = int(counts.sum())
+            r = rows[:m].long()
+            cp = MornaSearch.__new__(MornaSearch)
+            cp.lib, cp.device, cp.basename, cp.dim, cp.ld = self.lib, self.device, self.basename, self.dim, self.ld
+            cp.sample_count, cp.index_size = self.sample_count, m
+            cp.sample_frequencies, cp.internal_id_map = self.sample_frequencies, self.internal_id_map
+            cp.row_lo, cp.row_hi = 0, m
+            cp.vectors, cp.pp = self.vectors.index_select(0, r), self.pp.index_select(0, r)
+            cp.csr = None                      # (a sparse index's tie groups only overflow to the exact scan here)
+            first = torch.from_numpy(np.repeat(starts, counts)).to(self.device)
+            cp.row_group = (torch.arange(m, device=self.device) - first).to(torch.int32)
+            cp.query, cp.query_sample = defaultdict(int), [0.0] * self.dim
+            cp.enable_tensor_path()
+            cache["copy"] = cp
+        return cp
+
+    def _within_large(self, plan):
+        """Generator over the tensor-core route, one group at a time: (search, queries idx (host), their float64 queries,
+        exclusion labels or None, local -> internal id map).  The search is the group's row range of _within_copy (a view:
+        its rows, norms and fp16 operand sliced, ids local to the range and ascending with the internal ids); an excluded
+        row is the existing per-query exclusion on it, the query labelled with that row's position in the group."""
+        rows, labels, starts, counts, _ = self._within_layout()
+        idx = plan["large"]
+        if not len(idx):
+            return
+        cp = self._within_copy()
+        for gval in np.unique(plan["gi"][idx]).tolist():
+            sel = idx[plan["gi"][idx] == gval]
+            a, L = int(starts[gval]), int(counts[gval])
+            view = MornaSearch.__new__(MornaSearch)
+            view.__dict__.update(cp.__dict__)
+            view.vectors, view.pp, view.hs = cp.vectors[a:a + L], cp.pp[a:a + L], cp.hs[a:a + L]
+            view.row_group, view.row_lo, view.row_hi = cp.row_group[a:a + L], 0, L
+            view._ws_pool = {}                 # (the single-query workspace is laid out for one row count)
+            member = rows[a:a + L]
+            excl = plan["excl"][sel]
+            qlab = None
+            if (excl >= 0).any():
+                m = member.cpu().numpy()
+                at = np.minimum(np.searchsorted(m, excl), L - 1)
+                qlab = torch.from_numpy(np.where((excl >= 0) & (m[at] == excl), at, -1).astype(np.int32)).to(self.device)
+            yield view, sel, self._within_rows(plan, sel), qlab, member
+
+    def _within_ids(self, ids, member):
+        """Ids local to a group's row range -> internal ids; -1 padding stays."""
+        return torch.where(ids >= 0, member[ids.long().clamp(min=0)] + self.row_lo, ids).to(torch.int32)
+
+    def within_group_search(self, queries, k, query_groups, exclude_rows=None):
+        """Top-k within each query's own group: the brute-force answer over the rows labelled query_groups[q] (labels of
+        set_row_groups; a row labelled < 0 is in no group), without the row exclude_rows[q] (an internal id; -1: none).
+        ``queries``: CUDA float64 [nq x dim], or 1-D internal ids whose stored rows are the queries (as ``search -q``).
+        ``query_groups``: int32 [nq]; a label < 0 or one no row carries gives an empty list.  Returns device (ids int32
+        [nq x k], dists float64 [nq x k]) in the reference order, ids global, padded with -1 / +inf.  A group's queries
+        take the grouped FP64 route or the tensor-core route over the group's rows (see WITHIN_GROUPED_MAX_PAIRS); both
+        give the brute-force bits.  Sets ``last_within_routes`` = (queries on the grouped route, on the tensor-core
+        route)."""
+        plan = self._within_plan(queries, query_groups, exclude_rows)
+        nq, dev, k = plan["nq"], self.device, max(int(k), 0)
+        out_ids = torch.full((nq, k), -1, dtype=torch.int32, device=dev)
+        out_d = torch.full((nq, k), float("inf"), dtype=torch.float64, device=dev)
+        if nq == 0 or k == 0:
+            return out_ids, out_d
+        with torch.cuda.device(dev):
+            for c, _ in self._within_grouped_calls(plan, "query"):
+                ws = self._workspace(self.lib.morna_within_group_workspace_bytes(c["total"]), "within")
+                head, tail = self._within_call_args(c)
+                _lib.check(self.lib.morna_within_group_topk(*head, self.row_lo, *tail, k, _lib.dev_ptr(out_ids),
+                                                            _lib.dev_ptr(out_d), _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()),
+                           "morna_within_group_topk")
+            for view, sel, q, qlab, member in self._within_large(plan):
+                ids, d = view.batched_search_device(q, k, query_groups=qlab)
+                at = torch.from_numpy(sel).to(dev)
+                out_ids[at] = self._within_ids(ids, member)
+                out_d[at] = d
+        return out_ids, out_d
+
+    def within_group_range(self, queries, max_distance, query_groups, exclude_rows=None):
+        """Every row of each query's own group within ``max_distance``: the within_group_search rows (same arguments),
+        as the device CSR (offsets int64 [nq+1], ids int32, dists float64) that range_search_device returns."""
+        r = check_radius(max_distance)
+        plan = self._within_plan(queries, query_groups, exclude_rows)
+        nq, dev = plan["nq"], self.device
+        pieces = []
+        with torch.cuda.device(dev):
+            for c, o in self._within_grouped_calls(plan, "local"):
+                ws = self._workspace(self.lib.morna_within_group_workspace_bytes(c["total"]), "within")
+                head, tail = self._within_call_args(c)
+                n = len(o)
+                counts = torch.empty(n, dtype=torch.int64, device=dev)
+                _lib.check(self.lib.morna_within_group_range_count(*head, *tail, r, _lib.dev_ptr(counts), _lib.dev_ptr(ws),
+                                                                   ws.numel(), _lib.stream_ptr()), "morna_within_group_range_count")
+                off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+                torch.cumsum(counts, 0, out=off[1:])
+                total = int(off[-1].item())
+                ids = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+                d = torch.empty(max(total, 1), dtype=torch.float64, device=dev)
+                _lib.check(self.lib.morna_within_group_range_fill(
+                    n, tail[0], self.row_lo, _lib.dev_ptr(c["seg_off"]), c["total"], _lib.dev_ptr(c["row_begin"]),
+                    c["max_segment"], _lib.dev_ptr(c["out_slot"]), _lib.dev_ptr(off), _lib.dev_ptr(ids), _lib.dev_ptr(d),
+                    _lib.dev_ptr(ws), ws.numel(), _lib.stream_ptr()), "morna_within_group_range_fill")
+                pieces.append((o, off, ids[:total], d[:total]))
+            for view, sel, q, qlab, member in self._within_large(plan):
+                off, ids, d = view.range_search_device(q, r, query_groups=qlab)
+                pieces.append((sel, off - off[:1], self._within_ids(ids, member), d))
+            return splice_csr(nq, pieces, dev)
+
+
+def splice_csr(nq, pieces, device):
+    """One CSR over queries 0..nq-1 from pieces (query indices host int64 [m], offsets [m+1] from 0, ids, dists); a query
+    in no piece has an empty list."""
+    counts = torch.zeros(nq, dtype=torch.int64, device=device)
+    for idx, off, _, _ in pieces:
+        counts[torch.from_numpy(idx).to(device)] = off[1:] - off[:-1]
+    offsets = torch.zeros(nq + 1, dtype=torch.int64, device=device)
+    torch.cumsum(counts, 0, out=offsets[1:])
+    total = int(offsets[-1].item())
+    ids = torch.empty(total, dtype=torch.int32, device=device)
+    d = torch.empty(total, dtype=torch.float64, device=device)
+    for idx, off, p_ids, p_d in pieces:
+        if p_ids.numel():
+            shift = offsets[torch.from_numpy(idx).to(device)] - off[:-1]
+            dst = torch.repeat_interleave(shift, off[1:] - off[:-1], output_size=p_ids.numel()) + \
+                torch.arange(p_ids.numel(), device=device)
+            ids[dst] = p_ids
+            d[dst] = p_d
+    return offsets, ids, d
+
 
 class FilteredSearch(object):
     """The searches of a MornaSearch over a chosen subset of its rows (MornaSearch.subset), with results under the
@@ -1394,6 +1651,30 @@ class FilteredSearch(object):
                         max_per_group=None):
         return self._nn(self.inner.range_search_nn(max_distance, include_distances, False, num_neighbors, query_groups,
                                                    max_per_group), meta_db)
+
+    # ------------------------------------------------------------------ within-group search (parent ids in and out)
+    def _within_args(self, queries, exclude_rows):
+        """Queries (parent internal ids -> their stored rows) and excluded parent ids -> subset rows (-1: none)."""
+        t = torch.from_numpy(np.ascontiguousarray(queries)) if isinstance(queries, np.ndarray) else torch.as_tensor(queries)
+        if t.dim() == 1 and t.dtype in (torch.int32, torch.int64):
+            t = self.stored_queries(t)
+        if exclude_rows is None:
+            return t, None
+        e = torch.as_tensor(exclude_rows).to(self.device).long().reshape(-1)
+        inside = (e >= self.row_lo) & (e < self.row_hi)
+        return t, torch.where(inside, self._local[(e - self.row_lo).clamp(0, self.row_hi - self.row_lo - 1)], -1)
+
+    def within_group_search(self, queries, k, query_groups, exclude_rows=None):
+        """MornaSearch.within_group_search over the subset: the rows keep the parent's labels, so each list is the subset
+        rows of the query's group."""
+        q, e = self._within_args(queries, exclude_rows)
+        ids, d = self.inner.within_group_search(q, k, query_groups, e)
+        return self._to_parent(ids), d
+
+    def within_group_range(self, queries, max_distance, query_groups, exclude_rows=None):
+        q, e = self._within_args(queries, exclude_rows)
+        offsets, ids, d = self.inner.within_group_range(q, max_distance, query_groups, e)
+        return offsets, self._to_parent(ids), d
 
 
 class _PipeSlot(object):
